@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s and deals/s of the batched Tarok environment (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--mode M] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--games G] [--mode M] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: deal -> contract -> talon exchange ->
 48 x play_step (uniform-random legal-move players) -> score, for G concurrent deals per GPU
@@ -45,6 +45,7 @@ MODE_NAMES = {16: "Navadna igra (Tri/Dve/Ena forced, uniform declarer+king), tal
 CONFIG3_TOTAL = 4_194_304        # BASELINE config 3: 4M concurrent deals over the box
 CONFIG5_TOTAL = 16_777_216       # BASELINE config 5: 16M concurrent deals at 1/2/4/8 GPUs
 CONFIG4_ENVS = 65_536            # BASELINE config 4: envs per GPU
+DUMP_BYTES = 64 << 20            # --dump-outputs: at most this much over all ranks
 
 
 def workload_name(mode, games):
@@ -65,6 +66,25 @@ def hbm_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(out_dir, rank, world, scores, stats):
+    """--dump-outputs: what the timed rollout hands its caller after the last timed step -- that step's per-deal scores by
+    seat, and the statistics vector, which accumulates over the K timed steps (reset before the first) and is all-reduced over
+    the ranks -- as float .npy files, so that two builds run with the same arguments can be compared output for output.
+    Scores beyond this rank's share of DUMP_BYTES are a fixed, seeded sample of deals; `scores_rows` holds their indices in
+    the batch."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    name = "scores" if world == 1 else "scores_rank%d" % rank
+    rows = (DUMP_BYTES // world - 4096) // (4 * 4 + 8)                   # float32 x4 per deal + its float64 index
+    if len(scores) > rows:
+        idx = np.sort(np.random.default_rng(SEED).choice(len(scores), rows, replace=False))
+        scores = scores[idx]
+        np.save(os.path.join(out_dir, name + "_rows.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, name + ".npy"), scores.astype(np.float32))
+    if rank == 0:
+        np.save(os.path.join(out_dir, "stats.npy"), stats.astype(np.float64))
 
 
 def step_traffic(games, mode, kernel="k_step<random>"):
@@ -414,6 +434,8 @@ def run_ours(args, rank, world, local_rank):
     region_ms = t0.elapsed_time(t1)
     ms = max_over_ranks(sum(x.elapsed_time(y) for x, y in iter_events))
     st = stats_ring[(args.warmup + args.steps - 1) % len(stats_ring)].cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rank, world, env.scores[:n].cpu().numpy(), st)
     launches = env.launches - launches0
     # the same K steps once more as plain launches with an event pair around the 48 play_steps: the roofline's launch time
     probe_stats = env.stats_dev.clone()
@@ -740,7 +762,7 @@ def run_config4(args, local_rank):
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     ident = lambda x: x
-    rec = config4_record(local_rank, 0, 1, max(2, min(args.steps, 5)), dev, ident, ident)
+    rec = config4_record(local_rank, 0, 1, args.steps, dev, ident, ident)
     print(json.dumps({"metric": "env_steps_per_sec", "value": rec["env_steps_per_sec_incl_forwards"], "unit": "env-steps/s", "n_gpus": 1,
                       "higher_is_better": True, "dtype": "u64 env / fp32 nets", "data": "synthetic", "config4": rec}))
 
@@ -748,7 +770,10 @@ def run_config4(args, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="K, the timed steps of the headline rollout loop, of each end-to-end leg and of --config 4; the "
+                         "informational legs time min(max(K, 3), 20) forced-action replays, max(3, min(K, --sub-steps)) "
+                         "rollouts per config-3/5 sub-record and max(2, min(K, 3)) per config-4 sub-record")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--games", type=int, default=1 << 20, help="concurrent deals per GPU")
     ap.add_argument("--mode", type=int, default=16)
@@ -761,7 +786,14 @@ def main():
     ap.add_argument("--sub-steps", type=int, default=5, help="timed rollouts per sub-record")
     ap.add_argument("--no-flush", action="store_true", help="skip the L2-flush write between iterations (the 159 MB state is larger than L2)")
     ap.add_argument("--config", type=int, default=2, help="2 (default, the headline workload) or 4 (neural self-play only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="config-2 GPU rollout only (not with --impl reference or --config 4): write to DIR as .npy the "
+                         "per-deal scores of the last timed step and the statistics vector accumulated over the K timed steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == 4):
+        ap.error("--dump-outputs applies to the GPU rollout of config 2")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

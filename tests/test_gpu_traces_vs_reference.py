@@ -6,10 +6,14 @@ uniform-random legal-move players, per play the card and a digest of the legal m
   recorded cards are teacher-forced, the reference's own `mozne` at every play, its trick winners and its scores must equal
   what the GPU produced;
 * everywhere (CPU): the same replay through the C oracle;
-* GPU box (`gpu` marker): the kernels regenerate the traces from the same seed and must reproduce the committed file byte
-  for byte, which ties the CURRENT kernels to the replayed games."""
+* GPU box (`gpu` marker): the kernels regenerate the traces from the same seed and must reproduce the committed file array
+  for array, which ties the CURRENT kernels to the replayed games.
+The file stores the deals, the cards played and the per-game mask digests as one sha256 per 100 games
+(tools/export_gpu_traces.py `compact`); the C oracle's synthetic rollout regenerates the deals and the cards from the seed, and
+they must match."""
 import hashlib
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -19,9 +23,41 @@ PATH = os.path.join(HERE, "golden", "gpu_traces.npz")
 pytestmark = pytest.mark.skipif(not os.path.exists(PATH), reason="tests/golden/gpu_traces.npz not generated yet")
 
 
+def _check_digests(got, want, what):
+    """``got``: the array of all games; ``want``: its stored digests.  A mismatch names the first block of games that differs."""
+    X = _tool()
+    d = X.digests(got)
+    assert d.shape == want.shape, (what, d.shape, want.shape)
+    bad = np.flatnonzero((d != want).any(1))
+    assert not len(bad), "%s differs in games %d..%d" % (what, bad[0] * X.DIGEST_GAMES, (bad[0] + 1) * X.DIGEST_GAMES - 1)
+
+
+def _tool():
+    tools = os.path.join(os.path.dirname(HERE), "tools")
+    if tools not in sys.path:
+        sys.path.insert(0, tools)
+    import export_gpu_traces as X
+    return X
+
+
 @pytest.fixture(scope="module")
-def tr():
+def stored():
     return dict(np.load(PATH))
+
+
+@pytest.fixture(scope="module")
+def tr(stored, oracle):
+    """The committed games with their deals (`perm`) and cards (`card`) restored and checked against the stored digests."""
+    t = dict(stored)
+    assert (t["err"] == 0).all()                       # the digests cover every game: none may be an error game
+    seed = int(t["seed"][0])
+    ends = list(t["first"][1:]) + [len(t["contract"])]
+    parts = [oracle.rollout(seed, int(a), int(b - a), int(t["contract"][a])) for a, b in zip(t["first"], ends)]
+    t["perm"] = np.concatenate([p["perm"] for p in parts])
+    t["card"] = np.concatenate([p["cards"] for p in parts])
+    for k in ("perm", "card"):
+        _check_digests(t[k], t[k + "_sha256"], k)
+    return t
 
 
 def _digest(masks):
@@ -45,7 +81,7 @@ def test_gpu_traces_replay_through_the_c_oracle(tr, oracle):
         assert (rep["winner"][sel, k] == tr["winner"][sel, k]).all(), k
     masks = np.where(played, rep["mask"], 0).astype(np.uint64)
     dig = np.stack([_digest(masks[i]) for i in range(n)])
-    assert (dig[ok] == tr["mask_digest"][ok]).all()
+    _check_digests(dig, tr["mask_digest_sha256"], "legal masks")
     for c in range(10):                                                              # and the masks stored whole
         a = int(tr["first"][c])
         m = tr["mask_full"][c]
@@ -53,16 +89,16 @@ def test_gpu_traces_replay_through_the_c_oracle(tr, oracle):
 
 
 def _replay_chunk(args):
-    """Worker: replays games [a, b) through the reference; returns the list of mismatching game indices."""
-    a, b = args
+    """Worker: replays games [a, b) (`tr` = their rows) through the reference; returns the mismatching game indices and the
+    digest of the legal masks the reference showed in every game."""
+    a, b, tr = args
     from oracle import ref_harness as H
-    tr = dict(np.load(PATH))
-    bad = []
+    bad, digests = [], []
 
     class Forced(H.Policy):
         def __init__(self, i):
             super().__init__()
-            self.i, self.t = i, 0
+            self.i, self.t = i - a, 0
 
         def group(self, seat, kupcki):
             return int(tr["group"][self.i])
@@ -79,21 +115,22 @@ def _replay_chunk(args):
             return next(k for k in mozne if k.v_id() == c)          # StopIteration = the GPU played a card the reference forbids
 
     for i in range(a, b):
-        if tr["err"][i]:
-            continue
+        j = i - a
+        masks = np.zeros(48, np.uint64)
         try:
-            rec, players = H.run_forced(tr["perm"][i], int(tr["contract"][i]), int(tr["declarer"][i]), int(tr["king"][i]), Forced(i))
+            rec, players = H.run_forced(tr["perm"][j], int(tr["contract"][j]), int(tr["declarer"][j]), int(tr["king"][j]), Forced(i))
         except Exception as ex:                                     # noqa: BLE001 - any divergence is a failure of this game
             bad.append((i, repr(ex)[:80]))
+            digests.append(_digest(masks))
             continue
-        p = int(tr["plays"][i])
-        masks = np.zeros(48, np.uint64)
+        p = int(tr["plays"][j])
         masks[:p] = np.array(rec.masks, np.uint64)
-        good = (len(rec.cards) == p and list(tr["seat"][i][:p]) == rec.seats and list(tr["scores"][i]) == rec.scores
-                and list(tr["winner"][i][:p // 4]) == rec.winners and (_digest(masks) == tr["mask_digest"][i]).all())
+        digests.append(_digest(masks))
+        good = (len(rec.cards) == p and list(tr["seat"][j][:p]) == rec.seats and list(tr["scores"][j]) == rec.scores
+                and list(tr["winner"][j][:p // 4]) == rec.winners)
         if not good:
             bad.append((i, "differs"))
-    return bad
+    return bad, digests
 
 
 @pytest.mark.reference
@@ -103,18 +140,21 @@ def test_gpu_traces_replay_through_the_python_reference(tr):
     n = len(tr["contract"])
     workers = min(8, os.cpu_count() or 1)
     step = (n + 8 * workers - 1) // (8 * workers)
-    chunks = [(a, min(n, a + step)) for a in range(0, n, step)]
+    keys = ("perm", "contract", "declarer", "king", "group", "discard", "card", "seat", "scores", "winner", "plays")
+    chunks = [(a, min(n, a + step), {k: tr[k][a:a + step] for k in keys}) for a in range(0, n, step)]
     with mp.get_context("spawn").Pool(workers) as pool:
-        bad = [x for part in pool.map(_replay_chunk, chunks) for x in part]
+        parts = pool.map(_replay_chunk, chunks)
+    bad = [x for part, _ in parts for x in part]
     assert not bad, bad[:5]
+    dig = np.stack([d for _, part in parts for d in part])
+    _check_digests(dig, tr["mask_digest_sha256"], "legal masks shown by the reference")
 
 
 @pytest.mark.gpu
-def test_current_kernels_regenerate_the_committed_traces(tr, tmp_path):
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tools"))
-    import export_gpu_traces as X
+def test_current_kernels_regenerate_the_committed_traces(stored, tmp_path):
+    X = _tool()
     got = X.export(str(tmp_path / "again.npz"))
-    for k in ("perm", "contract", "declarer", "king", "group", "discard", "seat", "card", "winner", "scores", "plays", "err",
-              "mask_digest", "mask_full"):
-        assert np.array_equal(np.asarray(got[k]), tr[k]), k
+    for k in ("contract", "declarer", "king", "group", "discard", "seat", "winner", "scores", "plays", "err", "mask_full"):
+        assert np.array_equal(np.asarray(got[k]), stored[k]), k
+    for k in X.DIGESTED:
+        _check_digests(got[k], stored[k + "_sha256"], k)

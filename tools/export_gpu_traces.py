@@ -6,8 +6,9 @@ BASELINE config 1 exactly -- 10,000 Philox Klop deals, four uniform-random legal
 other contract (forced per game, uniform declarer / king, Bot-style exchange), all played by the stepwise CUDA kernels.
 Per game: the deal as the permutation Igra.razdeli would have consumed, contract / declarer / king, talon group and
 discards, the 48 cards with their seats, a digest of the 48 legal masks the device showed (full masks for the first games of
-every contract), trick winners, scores.  The committed copy is tests/golden/gpu_traces.npz; the build-container test replays
-every game through the imported Python reference, the GPU test regenerates it and compares byte for byte."""
+every contract), trick winners, scores.  The committed copy is tests/golden/gpu_traces.npz, written in the form ``compact``
+gives; the tests replay every game through the C oracle (and the imported Python reference where it is installed), the GPU
+test regenerates the file and compares it array for array."""
 import hashlib
 import os
 import sys
@@ -18,10 +19,28 @@ import numpy as np
 SEED = 0xC0FFEE2026
 PLAN = [(0, 10000)] + [(c, 2000) for c in range(1, 10)]        # (contract code, deals)
 FULL_MASKS = 64                                                # games per contract whose 48 masks are stored whole
+# stored as sha256 digests, which keeps the committed file small: the deals and the cards played are regenerated from the
+# seed by the C oracle's synthetic rollout, the per-game mask digests by its replay
+DIGESTED = ("perm", "card", "mask_digest")
+DIGEST_GAMES = 100                                             # games per digest, so that a mismatch names its games
 
 
 def mask_digest(masks_row):
     return np.frombuffer(hashlib.sha256(np.ascontiguousarray(masks_row).tobytes()).digest()[:16], np.uint8)
+
+
+def digests(a):
+    """sha256 of every DIGEST_GAMES consecutive games (rows of ``a``): uint8 [ceil(n / DIGEST_GAMES), 32]."""
+    a = np.ascontiguousarray(a)
+    return np.stack([np.frombuffer(hashlib.sha256(a[i:i + DIGEST_GAMES].tobytes()).digest(), np.uint8)
+                     for i in range(0, len(a), DIGEST_GAMES)])
+
+
+def compact(out):
+    """The stored form of ``export``'s arrays: every DIGESTED array ``k`` becomes ``k_sha256`` (``digests``)."""
+    c = {k: v for k, v in out.items() if k not in DIGESTED}
+    c.update({k + "_sha256": digests(out[k]) for k in DIGESTED})
+    return c
 
 
 def play(contract, n, gid0):
@@ -73,7 +92,7 @@ def export(path):
     out["mask_full"] = np.stack([p["mask_full"] for p in parts])          # [10, FULL_MASKS, 48]
     out["first"] = np.cumsum([0] + [n for _, n in PLAN])[:-1].astype(np.int64)
     out["seed"] = np.array([SEED], np.uint64)
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **compact(out))
     return out
 
 
