@@ -75,6 +75,24 @@ def replay(perm, contract, declarer, king, group, discard_mask, cards, want_stat
     return out
 
 
+def lists(perm, contract, declarer, king, group, discard_mask, cards):
+    """Teacher-forced replay like ``replay``, returning the reference's ordered lists: mozne uint8 [n,48,16] (0xFF
+    padded) + mozne_n [n,48], seat [n,48] (both also at the first 0xFF of a game still being played), trick_value int16 [n,12], zalozit uint8 [n,16] + zalozit_n [n] (the
+    ``mozno_zalozit()`` list after the pick-up; empty without an exchange) and groups uint8 [n,6,3] (0xFF padded)."""
+    n = len(perm)
+    args = [np.ascontiguousarray(perm, np.uint8).reshape(n, 54), np.ascontiguousarray(contract, np.uint8),
+            np.ascontiguousarray(declarer, np.uint8), np.ascontiguousarray(king, np.uint8),
+            np.ascontiguousarray(group, np.uint8), np.ascontiguousarray(discard_mask, np.uint64),
+            np.ascontiguousarray(cards, np.uint8).reshape(n, 48)]
+    out = dict(mozne=np.empty((n, 48, 16), np.uint8), mozne_n=np.empty((n, 48), np.uint8),
+               seat=np.empty((n, 48), np.uint8), trick_value=np.empty((n, 12), np.int16),
+               zalozit=np.empty((n, 16), np.uint8), zalozit_n=np.empty(n, np.uint8), groups=np.empty((n, 6, 3), np.uint8))
+    lib().orc_lists_batch(C.c_int64(n), *[_p(a) for a in args],
+                          *[_p(out[k]) for k in ("mozne", "mozne_n", "seat", "trick_value", "zalozit", "zalozit_n",
+                                                 "groups")])
+    return out
+
+
 def auction_fixed(intents):
     """intents: int8[n,4] Tip codes (-1 Naprej .. 9).  -> (declarer, contract, calls)"""
     intents = np.ascontiguousarray(intents, np.int8).reshape(-1, 4)

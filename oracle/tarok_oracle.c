@@ -526,6 +526,60 @@ void orc_replay_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, c
     }
 }
 
+/* The ordered lists the neural player decides over, with the same teacher forcing as orc_replay_batch:
+   per play (and for the first 0xFF of a game still being played: the decision pending there) the `mozne` list in the reference's order (Navadna_igra.py:158-168 / Klop.py:96-133) and the seat to move;
+   per trick the value the replay target uses (Roka.vrednost_stiha of the trick incl. Klop's talon card, Roka.py:72-95);
+   per exchange the `mozno_zalozit()` list after the pick-up (Roka.py:23-27, Igralec.py:376-380) and the talon groups
+   (Navadna_igra.py:36-44).  Unused slots are 0xFF; values of unplayed tricks are 0. */
+void orc_lists_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, const uint8_t* declarer,
+                     const uint8_t* king, const uint8_t* group, const uint64_t* discard_mask, const uint8_t* cards,
+                     uint8_t* out_mozne, uint8_t* out_mozne_n, uint8_t* out_seat, int16_t* out_trick_value,
+                     uint8_t* out_zalozit, uint8_t* out_zalozit_n, uint8_t* out_groups) {
+#pragma omp parallel for schedule(static)
+    for (int64_t i = 0; i < n; i++) {
+        orc_game g;
+        orc_razdeli(&g, perm + 54 * i);
+        orc_zacni_igro(&g, contract[i], declarer[i], king[i]);
+        memset(out_mozne + 48 * 16 * i, 0xFF, 48 * 16);
+        memset(out_mozne_n + 48 * i, 0, 48);
+        memset(out_seat + 48 * i, 0xFF, 48);
+        for (int k = 0; k < 12; k++) out_trick_value[12 * i + k] = 0;
+        memset(out_zalozit + 16 * i, 0xFF, 16);
+        out_zalozit_n[i] = 0;
+        memset(out_groups + 18 * i, 0xFF, 18);
+        if (!g.error && g.phase == 1) {
+            for (int a = 0; a < g.group_cnt; a++)
+                for (int j = 0; j < g.group_sz; j++) out_groups[18 * i + 3 * a + j] = g.group[a][j];
+            if (group[i] < g.group_cnt) {
+                orc_game tmp = g;
+                for (int j = 0; j < tmp.group_sz; j++) roka_append(&tmp, tmp.declarer, tmp.group[group[i]][j]);
+                out_zalozit_n[i] = (uint8_t)orc_mozno_zalozit(&tmp, tmp.declarer, out_zalozit + 16 * i);
+            }
+            uint8_t d[3];
+            int k = 0;
+            for (int c = 0; c < 54 && k < 3; c++) if ((discard_mask[i] >> c) & 1) d[k++] = (uint8_t)c;
+            int kk = __builtin_popcountll(discard_mask[i]);
+            orc_menjaj(&g, group[i], d, kk > 3 ? 99 : kk);
+        }
+        int t = 0;
+        while (!g.error && g.phase == 2 && t < 48) {
+            int c = cards[48 * i + t];
+            out_seat[48 * i + t] = (uint8_t)orc_na_potezi(&g);
+            out_mozne_n[48 * i + t] = (uint8_t)orc_mozne_karte(&g, out_mozne + (48 * i + t) * 16);
+            if (c == 0xFF) break;                                  /* the pending decision is written too */
+            int tr = g.tricks, before[4];
+            for (int s = 0; s < 4; s++) before[s] = g.pile_n[s];
+            orc_igraj(&g, c);
+            if (g.error) break;
+            if (g.tricks != tr) {
+                int w = g.last_winner;
+                out_trick_value[12 * i + tr] = (int16_t)orc_vrednost_stiha(g.pile[w] + before[w], g.pile_n[w] - before[w]);
+            }
+            t++;
+        }
+    }
+}
+
 typedef struct { const int8_t* v; } arr_ctx;
 static int want_fixed(void* ctx, int seat, int call) { (void)call; return ((arr_ctx*)ctx)->v[seat]; }
 static int want_scripted(void* ctx, int seat, int call) { (void)seat; return call < 16 ? ((arr_ctx*)ctx)->v[call] : ORC_NAPREJ; }

@@ -898,10 +898,8 @@ int tarok_obs_expand_buckets(tarok_t* h, const int32_t* sel_dev, const uint8_t* 
     return 0;
 }
 
-static inline u32 explore_threshold(float random_card) {
-    const double thr = (double)random_card * 4294967296.0;
-    return thr >= 4294967295.0 ? 0xFFFFFFFFu : (u32)thr;
-}
+// random.random() < random_card as "Philox word < threshold" over 64 bits: random_card = 1 gives 2^32, above every word.
+static inline u64 explore_threshold(float random_card) { return (u64)((double)random_card * 4294967296.0); }
 
 int tarok_select_action_buckets(tarok_t* h, const float* const* q_ptrs_dev, const int32_t* sel_dev, const uint8_t* selkey_dev,
                                 const uint32_t* counts_dev, uint64_t n_total, const float* random_card4, uint8_t* card_dev,
@@ -981,8 +979,7 @@ int tarok_select_action(tarok_t* h, const float* q_dev, const int32_t* sel_dev, 
     if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
     if (n_sel == 0) return 0;
     DeviceGuard dg(h->device);
-    const double thr = (double)random_card * 4294967296.0;
-    const u32 threshold = thr >= 4294967295.0 ? 0xFFFFFFFFu : (u32)thr;
+    const u64 threshold = explore_threshold(random_card);
     const u64 warps_per_cta = tk::CTA / 32;
     tk::k_select_action<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
         h->e, q_dev, (const int*)sel_dev, n_sel, threshold, card_dev, qmax_dev);
@@ -1020,8 +1017,7 @@ int tarok_select_exchange(tarok_t* h, const float* p_dev, const int32_t* sel_dev
     if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
     if (n_sel == 0) return 0;
     DeviceGuard dg(h->device);
-    const double thr = (double)random_card * 4294967296.0;
-    const u32 threshold = thr >= 4294967295.0 ? 0xFFFFFFFFu : (u32)thr;
+    const u64 threshold = explore_threshold(random_card);
     const u64 warps_per_cta = tk::CTA / 32;
     tk::k_select_exchange<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
         h->e, p_dev, (const int*)sel_dev, n_sel, threshold, group_dev, (u64*)discard_dev);

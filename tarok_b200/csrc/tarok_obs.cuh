@@ -285,11 +285,20 @@ __global__ void __launch_bounds__(CTA) k_obs_expand_all(Env e, const int* __rest
 //   legal card instead.  np.argmax returns the FIRST maximum in the order of the list `mozne`, so ties are broken
 //   by that order (A.2): when following suit / trumping it is the player's suit list -- the cards as dealt in
 //   ascending order, then the cards picked up from the talon in talon order (Roka.py:10-11,19-21); otherwise all
-//   cards sorted ascending.  One warp per game; lanes hold cards lane and lane+32.
+//   cards sorted ascending.  np.argmax also returns the first NaN, and a legal card is chosen whatever its value
+//   (-inf, -FLT_MAX), so a diverged network still plays legal cards.  One warp per game; lanes hold cards lane and lane+32.
 // ------------------------------------------------------------------------------------------------
 enum : u32 { ST_EXPLORE = 8 };
 
-__device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __restrict__ qrow, u32 explore_threshold,
+// The order np.argmax ranks values by: NaN above everything (the first NaN wins), then the usual order, so that -inf and
+// -FLT_MAX are ordinary values that any legal card can hold.  `a` ranks strictly above `b`:
+__device__ __forceinline__ bool ranks_above(float a, float b) { return a > b || (a != a && b == b); }
+
+// random.random() < random_card with random.random() = w / 2^32: `explore_threshold` = random_card * 2^32 (0 = never,
+// 2^32 = always), so random_card = 1 explores at every word, 0xFFFFFFFF included.
+__device__ __forceinline__ bool explores(u32 w, u64 explore_threshold) { return (u64)w < explore_threshold; }
+
+__device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __restrict__ qrow, u64 explore_threshold,
                                             uint8_t* __restrict__ card_out, float* __restrict__ qmax_out, u32 lane) {
     const u64 na = e.n_alloc;
     const u64 meta = e.meta[g];
@@ -301,29 +310,33 @@ __device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __
     // is `mozne` one of the player's own suit lists (list order) or the sorted union (id order)?
     bool list_order = false;
     if (pos != 0) list_order = (hand & suit_mask_of(lead)) != 0 || (hand & TAROKS) != 0;
-    const u64 dealt = e.hands0 ? e.hands0[self * na + g] : ~0ull;
+    // the cards the declarer picked up from the talon (they follow the dealt cards in its suit lists, in talon order)
     const u64 order = e.torder[g];
-    float best = -3.4e38f;
+    const u32 grp = mget(meta, M_GROUP, 3);
+    const u64 picked = grp != NO_GROUP && self == mget(meta, M_DECL, 2)
+                     ? talon_group_bits(order, talon_k(mget(meta, M_CONTRACT, 4)), grp) : 0ull;
+    // "no card yet" = (-inf, key above every real key): any legal card beats it, whatever its value
+    float best = -INFINITY;
     u32 best_key = 0xFFFFFFFFu, best_card = 0xFF;
 #pragma unroll
     for (int h = 0; h < 2; h++) {
         const u32 c = lane + 32u * h;
         if (c < 54 && ((legal >> c) & 1ull)) {
             u32 key = c;
-            if (list_order && !((dealt >> c) & 1ull)) {          // picked up from the talon: after the dealt cards
+            if (list_order && ((picked >> c) & 1ull)) {          // picked up from the talon: after the dealt cards
                 u32 tp = 0;
                 for (u32 j = 0; j < 6; j++) if (((order >> (6 * j)) & 63ull) == c) tp = j;
                 key = 64u + tp;
             }
             const float v = qrow[c];
-            if (v > best || (v == best && key < best_key)) { best = v; best_key = key; best_card = c; }
+            if (ranks_above(v, best) || (!ranks_above(best, v) && key < best_key)) { best = v; best_key = key; best_card = c; }
         }
     }
 #pragma unroll
     for (int d = 16; d >= 1; d >>= 1) {
         const float ov = __shfl_xor_sync(0xFFFFFFFFu, best, d);
         const u32 ok = __shfl_xor_sync(0xFFFFFFFFu, best_key, d), oc = __shfl_xor_sync(0xFFFFFFFFu, best_card, d);
-        if (ov > best || (ov == best && ok < best_key)) { best = ov; best_key = ok; best_card = oc; }
+        if (ranks_above(ov, best) || (!ranks_above(best, ov) && ok < best_key)) { best = ov; best_key = ok; best_card = oc; }
     }
     if (lane == 0) {
         u32 card = best_card;
@@ -331,7 +344,7 @@ __device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __
             const u64 gid = e.first_gid + g;
             const u32 plays = mget(meta, M_PLAYS, 6);
             Words4 b = philox_block(e.rng, gid, ST_EXPLORE, plays);
-            if (b.w[0] < explore_threshold) card = nth_set_bit(legal, draw_from_word(b.w[1], e.rng, gid, ST_EXPLORE, plays * 4 + 1, (u32)__popcll(legal)));
+            if (explores(b.w[0], explore_threshold)) card = nth_set_bit(legal, draw_from_word(b.w[1], e.rng, gid, ST_EXPLORE, plays * 4 + 1, (u32)__popcll(legal)));
         }
         card_out[g] = (uint8_t)card;
         if (qmax_out) qmax_out[g] = best;                         // next_Q_max = p[argmax card] (Igralec.py:351)
@@ -340,7 +353,7 @@ __device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __
 }
 
 __global__ void __launch_bounds__(CTA) k_select_action(Env e, const float* __restrict__ q, const int* __restrict__ sel,
-                                                       u64 n_sel, u32 explore_threshold, uint8_t* __restrict__ card_out,
+                                                       u64 n_sel, u64 explore_threshold, uint8_t* __restrict__ card_out,
                                                        float* __restrict__ qmax_out) {
     const u32 lane = threadIdx.x & 31u;
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
@@ -352,7 +365,7 @@ __global__ void __launch_bounds__(CTA) k_select_action(Env e, const float* __res
 
 // The action selection of EVERY bucket of a step in one launch: qptr[key] = the [bucket size, 54] output of that bucket's
 // forward pass (a table of device pointers the host fills), thr4[player] = the player's epsilon as a 32-bit threshold.
-struct Thresholds4 { u32 t[4]; };
+struct Thresholds4 { u64 t[4]; };
 // The same with the table of bucket outputs passed BY VALUE (1 KB of kernel parameters): no device table to fill and copy.
 struct QTable { const float* p[BUCKETS]; };
 __global__ void __launch_bounds__(CTA) k_select_action_all_tab(Env e, QTable qt, const int* __restrict__ sel,
@@ -366,7 +379,7 @@ __global__ void __launch_bounds__(CTA) k_select_action_all_tab(Env e, QTable qt,
     const float* q = qt.p[key & (BUCKETS - 1)];
     if (!q) return;                                               // no forward was supplied for this bucket
     const u32 p = key / 28u;
-    const u32 thr = p == 0 ? thr4.t[0] : p == 1 ? thr4.t[1] : p == 2 ? thr4.t[2] : thr4.t[3];
+    const u64 thr = p == 0 ? thr4.t[0] : p == 1 ? thr4.t[1] : p == 2 ? thr4.t[2] : thr4.t[3];
     select_game(e, (u64)sel[i], q + (i - counts[BUCKETS + key]) * 54u, thr, card_out, qmax_out, lane);
 }
 
@@ -381,7 +394,7 @@ __global__ void __launch_bounds__(CTA) k_select_action_all(Env e, const float* c
     const float* q = qptr[key];
     if (!q) return;                                               // no forward was supplied for this bucket
     const u32 p = key / 28u;
-    const u32 thr = p == 0 ? thr4.t[0] : p == 1 ? thr4.t[1] : p == 2 ? thr4.t[2] : thr4.t[3];
+    const u64 thr = p == 0 ? thr4.t[0] : p == 1 ? thr4.t[1] : p == 2 ? thr4.t[2] : thr4.t[3];
     select_game(e, (u64)sel[i], q + (i - counts[BUCKETS + key]) * 54u, thr, card_out, qmax_out, lane);
 }
 
@@ -431,7 +444,7 @@ __global__ void __launch_bounds__(CTA) k_obs_exchange(Env e, const int* __restri
 }
 
 __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __restrict__ p, const int* __restrict__ sel, u64 n_sel,
-                                                         u32 explore_threshold, uint8_t* __restrict__ group_out,
+                                                         u64 explore_threshold, uint8_t* __restrict__ group_out,
                                                          u64* __restrict__ discard_out) {
     const u32 lane = threadIdx.x & 31u;
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
@@ -446,24 +459,25 @@ __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __r
     const u64 gid = e.first_gid + g;
     const unsigned full = 0xFFFFFFFFu;
     // group: first argmax of p[54 .. 54+groups)
-    float bv = lane < groups ? p[i * 60u + 54u + lane] : -3.4e38f;
+    // (NaN first, the first maximum); the inactive lanes hold (-inf, 0xFF), which every real group beats
+    float bv = lane < groups ? p[i * 60u + 54u + lane] : -INFINITY;
     u32 bi = lane < groups ? lane : 0xFFu;
 #pragma unroll
     for (int d = 16; d >= 1; d >>= 1) {
         const float ov = __shfl_xor_sync(full, bv, d);
         const u32 oi = __shfl_xor_sync(full, bi, d);
-        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+        if (ranks_above(ov, bv) || (!ranks_above(bv, ov) && oi < bi)) { bv = ov; bi = oi; }
     }
     u32 group = bi;
     Words4 rnd = philox_block(e.rng, gid, ST_EXPLORE, 50u);                       // same words on every lane
-    if (explore_threshold && rnd.w[0] < explore_threshold) group = draw_from_word(rnd.w[1], e.rng, gid, ST_EXPLORE, 201u, groups);
+    if (explore_threshold && explores(rnd.w[0], explore_threshold)) group = draw_from_word(rnd.w[1], e.rng, gid, ST_EXPLORE, 201u, groups);
     const u64 order = e.torder[g];
     const u64 hand = e.hands[slot_of(decl, leader_of(meta)) * na + g];
     const u64 gb = talon_group_bits(order, k, group);
     u64 avail = (hand | gb) & DISCARDABLE;
     u64 discard = 0;
     if ((u32)__popcll(avail) < k) { if (lane == 0) { group_out[g] = (uint8_t)group; discard_out[g] = 0; } return; }   // Q19
-    if (explore_threshold && rnd.w[2] < explore_threshold) {                       // random.sample(mozno, st_kart)
+    if (explore_threshold && explores(rnd.w[2], explore_threshold)) {              // random.sample(mozno, st_kart)
         Words4 r2 = philox_block(e.rng, gid, ST_EXPLORE, 51u);
         for (u32 j = 0; j < k; j++) {
             const u32 w = j == 0 ? r2.w[0] : j == 1 ? r2.w[1] : r2.w[2];
@@ -472,7 +486,8 @@ __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __r
         }
     } else {
         for (u32 j = 0; j < k; j++) {                                              // k times: warp arg-max by (value, position)
-            float v = -3.4e38f; u32 key = 0, card = 0xFF;
+            // NaN ranks highest (np.argsort sorts it last); key 0 = no card, below every real key
+            float v = -INFINITY; u32 key = 0, card = 0xFF;
 #pragma unroll
             for (int hh = 0; hh < 2; hh++) {
                 const u32 c = lane + 32u * hh;
@@ -483,16 +498,16 @@ __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __r
                         for (u32 t = 0; t < 6; t++) if (((order >> (6 * t)) & 63ull) == c) tp = t;
                         pos = 64u + tp;
                     }
-                    const u32 kk = ((c >= 32 ? 4u : (c >> 3)) << 8) | pos;
+                    const u32 kk = (((c >= 32 ? 4u : (c >> 3)) << 8) | pos) + 1u;
                     const float pv = p[i * 60u + c];
-                    if (pv > v || (pv == v && kk > key)) { v = pv; key = kk; card = c; }
+                    if (ranks_above(pv, v) || (!ranks_above(v, pv) && kk > key)) { v = pv; key = kk; card = c; }
                 }
             }
 #pragma unroll
             for (int d = 16; d >= 1; d >>= 1) {
                 const float ov = __shfl_xor_sync(full, v, d);
                 const u32 ok2 = __shfl_xor_sync(full, key, d), oc = __shfl_xor_sync(full, card, d);
-                if (ov > v || (ov == v && ok2 > key)) { v = ov; key = ok2; card = oc; }
+                if (ranks_above(ov, v) || (!ranks_above(v, ov) && ok2 > key)) { v = ov; key = ok2; card = oc; }
             }
             const u64 bit = 1ull << card;
             avail ^= bit; discard |= bit;
