@@ -158,6 +158,38 @@ def rollout(seed, first_gid, n, mode, full=True):
     return out
 
 
+def rollout_injected(seed, first_gid, perm, contract, declarer, king=None):
+    """The given deals (uint8 [n,54]) under forced contracts (uint8 [n] each; king None = no king), game i with global id
+    first_gid + i, played like the host-buffer entries: talon group 0, Philox discards and cards.  Returns the dict of
+    ``rollout`` plus ``hist`` (int64 [10]: finished games by contract)."""
+    n = len(perm)
+    perm = np.ascontiguousarray(perm, np.uint8).reshape(n, 54)
+    contract = np.ascontiguousarray(contract, np.uint8)
+    declarer = np.ascontiguousarray(declarer, np.uint8)
+    king = None if king is None else np.ascontiguousarray(king, np.uint8)
+    assert contract.shape == declarer.shape == (n,) and (king is None or king.shape == (n,))
+    out = dict(scores=np.empty((n, 4), np.int16), plays=np.empty(n, np.uint8),
+               contract=np.empty(n, np.uint8), declarer=np.empty(n, np.uint8),
+               king=np.empty(n, np.uint8), err=np.empty(n, np.uint8), stats=np.zeros(10, np.int64),
+               perm=np.empty((n, 54), np.uint8), cards=np.empty((n, 48), np.uint8),
+               group=np.empty(n, np.uint8), discard=np.empty(n, np.uint64), hist=np.zeros(10, np.int64))
+    lib().syn_rollout_injected_batch(
+        C.c_uint64(seed), C.c_uint64(first_gid), C.c_int64(n), _p(perm), _p(contract), _p(declarer), _p(king),
+        _p(out["scores"]), _p(out["plays"]), _p(out["contract"]), _p(out["declarer"]), _p(out["king"]),
+        _p(out["err"]), _p(out["perm"]), _p(out["cards"]), _p(out["group"]), _p(out["discard"]), _p(out["stats"]),
+        _p(out["hist"]))
+    return out
+
+
+def device_stats(ref):
+    """What the device's statistics vector holds in entries 0..20 after the games of an oracle rollout (``rollout`` or
+    ``rollout_injected``): seat sums, player sums, finished games by contract, finished games, env steps, error games."""
+    fin = ref["err"] == 0
+    hist = ref["hist"] if "hist" in ref else np.bincount(ref["contract"][fin], minlength=10)
+    st = ref["stats"]
+    return np.concatenate([st[0:8], hist, [hist.sum(), st[8], st[9]]]).astype(np.int64)
+
+
 def rollout_stats_only(seed, first_gid, n, mode):
     """Timing leg for bench.py: no per-game outputs, only the 10-entry stats vector."""
     stats = np.zeros(10, np.int64)

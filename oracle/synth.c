@@ -156,43 +156,18 @@ static int nth_lowest(uint64_t m, uint32_t r) {
     return -1;
 }
 
-/* One whole deal with uniform-random players.  Returns 0, or -1 if the game hit an error state. */
-int syn_rollout(uint64_t seed, uint64_t gid, int mode, orc_game* g, uint8_t perm[54],
-                uint8_t cards[48], uint8_t* group_out, uint64_t* discard_out) {
-    syn_deal(seed, gid, perm);
-    orc_razdeli(g, perm);
-    int contract, declarer = 0, king = ORC_NO_KING;
-    if (mode == MODE_AUCTION_UNIFORM || mode == MODE_AUCTION_BOT) {
-        bid_ctx b; b.seed = seed; b.gid = gid;
-        int suit[4];
-        if (mode == MODE_AUCTION_UNIFORM) {
-            static const uint32_t n18[4] = { 18, 18, 18, 18 };
-            uint32_t idx[4];
-            syn_bdraws(seed, gid, ST_BID, ST_BID, 0, n18, 4, idx);
-            for (int s = 0; s < 4; s++) index2igra((int)idx[s], &b.tip[s], &suit[s]);
-        } else {
-            static const uint32_t n6[8] = { 6, 6, 6, 6, 6, 6, 6, 6 };
-            syn_bdraws(seed, gid, ST_BID, ST_BID, 0, n6, 8, b.digit);
-            syn_bdraws(seed, gid, ST_BID, ST_BID, 1, n6, 8, b.digit + 8);
-        }
-        orc_licitacija(mode == MODE_AUCTION_UNIFORM ? want_uniform : want_bot, &b,
-                       mode == MODE_AUCTION_UNIFORM, &declarer, &contract, 0);
-        if (contract >= ORC_TRI && contract <= ORC_ENA)
-            king = mode == MODE_AUCTION_UNIFORM ? suit[declarer] : (int)syn_draw(seed, gid, ST_FORCE, 2, 4);
-    } else {
-        static const uint32_t n344[3] = { 3, 4, 4 };      /* word 0 of the setup block: contract of the mix, declarer, king */
-        uint32_t r[3];
-        syn_bdraws(seed, gid, ST_FORCE, ST_FORCE, 0, n344, 3, r);
-        contract = mode == MODE_NAVADNA_MIX ? (int)(ORC_TRI + r[0]) : mode;
-        if (contract != ORC_KLOP) declarer = (int)r[1];
-        if (contract >= ORC_TRI && contract <= ORC_ENA) king = (int)r[2];
-    }
-    orc_zacni_igro(g, contract, declarer, king);
+/* Talon exchange and uniform-random play-out of a game whose contract is set (orc_zacni_igro done): the declarer takes
+   group 0 like Bot_igralec (Igralec.py:162), or a uniform group (word 3 of the setup block) when `random_group`, and lays
+   k uniform discards (word 1 of the setup block); every card is a uniform legal one (syn_play_draw).  Returns 0, or -1 if
+   the game is in an error state. */
+static int syn_play_out(uint64_t seed, uint64_t gid, int random_group, orc_game* g, uint8_t cards[48],
+                        uint8_t* group_out, uint64_t* discard_out) {
     *group_out = ORC_NO_GROUP; *discard_out = 0;
     memset(cards, 0xFF, 48);
-    if (g->phase == 1) {
-        int k = orc_talon_k(contract);
-        int grp = mode == MODE_AUCTION_UNIFORM ? (int)syn_draw(seed, gid, ST_FORCE, 3, g->group_cnt) : 0;
+    if (!g->error && g->phase == 1) {
+        const int declarer = g->declarer;
+        int k = orc_talon_k(g->contract);
+        int grp = random_group ? (int)syn_draw(seed, gid, ST_FORCE, 3, g->group_cnt) : 0;
         /* discardable set after the pick-up: Roka.mozno_zalozit on hand + group (Igralec.py:163-166) */
         uint64_t avail = 0;
         orc_game tmp = *g;
@@ -228,23 +203,84 @@ int syn_rollout(uint64_t seed, uint64_t gid, int mode, orc_game* g, uint8_t perm
     return g->error ? -1 : 0;
 }
 
-/* Batch driver (OpenMP over games).  Any out pointer may be NULL. */
-void syn_rollout_batch(uint64_t seed, uint64_t first_gid, int64_t n, int mode,
-                       int16_t* out_scores, uint8_t* out_plays, uint8_t* out_contract,
-                       uint8_t* out_declarer, uint8_t* out_king, uint8_t* out_err,
-                       uint8_t* out_perm, uint8_t* out_cards, uint8_t* out_group, uint64_t* out_discard,
-                       int64_t* out_stats /* [4 seat sums, 4 player sums, env steps, errors] */) {
-    int64_t st[10] = { 0 };
+/* One whole deal with uniform-random players.  Returns 0, or -1 if the game hit an error state. */
+int syn_rollout(uint64_t seed, uint64_t gid, int mode, orc_game* g, uint8_t perm[54],
+                uint8_t cards[48], uint8_t* group_out, uint64_t* discard_out) {
+    syn_deal(seed, gid, perm);
+    orc_razdeli(g, perm);
+    int contract, declarer = 0, king = ORC_NO_KING;
+    if (mode == MODE_AUCTION_UNIFORM || mode == MODE_AUCTION_BOT) {
+        bid_ctx b; b.seed = seed; b.gid = gid;
+        int suit[4];
+        if (mode == MODE_AUCTION_UNIFORM) {
+            static const uint32_t n18[4] = { 18, 18, 18, 18 };
+            uint32_t idx[4];
+            syn_bdraws(seed, gid, ST_BID, ST_BID, 0, n18, 4, idx);
+            for (int s = 0; s < 4; s++) index2igra((int)idx[s], &b.tip[s], &suit[s]);
+        } else {
+            static const uint32_t n6[8] = { 6, 6, 6, 6, 6, 6, 6, 6 };
+            syn_bdraws(seed, gid, ST_BID, ST_BID, 0, n6, 8, b.digit);
+            syn_bdraws(seed, gid, ST_BID, ST_BID, 1, n6, 8, b.digit + 8);
+        }
+        orc_licitacija(mode == MODE_AUCTION_UNIFORM ? want_uniform : want_bot, &b,
+                       mode == MODE_AUCTION_UNIFORM, &declarer, &contract, 0);
+        if (contract >= ORC_TRI && contract <= ORC_ENA)
+            king = mode == MODE_AUCTION_UNIFORM ? suit[declarer] : (int)syn_draw(seed, gid, ST_FORCE, 2, 4);
+    } else {
+        static const uint32_t n344[3] = { 3, 4, 4 };      /* word 0 of the setup block: contract of the mix, declarer, king */
+        uint32_t r[3];
+        syn_bdraws(seed, gid, ST_FORCE, ST_FORCE, 0, n344, 3, r);
+        contract = mode == MODE_NAVADNA_MIX ? (int)(ORC_TRI + r[0]) : mode;
+        if (contract != ORC_KLOP) declarer = (int)r[1];
+        if (contract >= ORC_TRI && contract <= ORC_ENA) king = (int)r[2];
+    }
+    orc_zacni_igro(g, contract, declarer, king);
+    return syn_play_out(seed, gid, mode == MODE_AUCTION_UNIFORM, g, cards, group_out, discard_out);
+}
+
+/* An injected deal (perm, Igra.razdeli order) under a forced contract, played like the host-buffer entries of the CUDA
+   path: talon group 0, discards and cards as in syn_rollout.  A row that is not a permutation of 0..53, or a declarer
+   above 3, makes an error game (as does what orc_zacni_igro rejects: an unknown contract, a king game without a suit). */
+static int syn_rollout_injected(uint64_t seed, uint64_t gid, const uint8_t perm[54], int contract, int declarer, int king,
+                                orc_game* g, uint8_t cards[48], uint8_t* group_out, uint64_t* discard_out) {
+    uint64_t seen = 0;
+    for (int i = 0; i < 54; i++) if (perm[i] < 54) seen |= 1ull << perm[i];
+    memset(g, 0, sizeof(*g));
+    if (seen != (1ull << 54) - 1 || declarer > 3) {
+        g->contract = contract; g->declarer = declarer; g->king = king;
+        g->error = 1;
+    } else {
+        orc_razdeli(g, perm);
+        orc_zacni_igro(g, contract, declarer, king);
+    }
+    return syn_play_out(seed, gid, 0, g, cards, group_out, discard_out);
+}
+
+/* Batch driver (OpenMP over games): synthetic deals and contracts of `mode`, or, with in_perm, the injected rows.  Any out
+   pointer may be NULL.  out_hist counts the finished games by contract (the device's stats[8..17]). */
+static void rollout_batch(uint64_t seed, uint64_t first_gid, int64_t n, int mode, const uint8_t* in_perm,
+                          const uint8_t* in_contract, const uint8_t* in_declarer, const uint8_t* in_king,
+                          int16_t* out_scores, uint8_t* out_plays, uint8_t* out_contract,
+                          uint8_t* out_declarer, uint8_t* out_king, uint8_t* out_err,
+                          uint8_t* out_perm, uint8_t* out_cards, uint8_t* out_group, uint64_t* out_discard,
+                          int64_t* out_stats, int64_t* out_hist) {
+    int64_t st[10] = { 0 }, hist[10] = { 0 };
 #pragma omp parallel
     {
-        int64_t loc[10] = { 0 };
+        int64_t loc[10] = { 0 }, lh[10] = { 0 };
 #pragma omp for schedule(static)
         for (int64_t i = 0; i < n; i++) {
             orc_game g;
             uint8_t perm[54], cards[48], grp;
             uint64_t dm;
             uint64_t gid = first_gid + (uint64_t)i;
-            syn_rollout(seed, gid, mode, &g, perm, cards, &grp, &dm);
+            if (in_perm) {
+                memcpy(perm, in_perm + 54 * i, 54);
+                syn_rollout_injected(seed, gid, perm, in_contract[i], in_declarer[i], in_king ? in_king[i] : ORC_NO_KING,
+                                     &g, cards, &grp, &dm);
+            } else {
+                syn_rollout(seed, gid, mode, &g, perm, cards, &grp, &dm);
+            }
             int fin = g.phase == 3 && !g.error;
             for (int s = 0; s < 4; s++) {
                 int v = fin ? g.pisejo[s] : 0;
@@ -254,6 +290,7 @@ void syn_rollout_batch(uint64_t seed, uint64_t first_gid, int64_t n, int mode,
             }
             loc[8] += g.plays;
             loc[9] += g.error ? 1 : 0;
+            if (fin && g.contract >= 0 && g.contract < 10) lh[g.contract]++;
             if (out_plays) out_plays[i] = (uint8_t)g.plays;
             if (out_contract) out_contract[i] = (uint8_t)g.contract;
             if (out_declarer) out_declarer[i] = (uint8_t)g.declarer;
@@ -265,9 +302,32 @@ void syn_rollout_batch(uint64_t seed, uint64_t first_gid, int64_t n, int mode,
             if (out_discard) out_discard[i] = dm;
         }
 #pragma omp critical
-        for (int j = 0; j < 10; j++) st[j] += loc[j];
+        for (int j = 0; j < 10; j++) { st[j] += loc[j]; hist[j] += lh[j]; }
     }
     if (out_stats) memcpy(out_stats, st, sizeof(st));
+    if (out_hist) memcpy(out_hist, hist, sizeof(hist));
+}
+
+void syn_rollout_batch(uint64_t seed, uint64_t first_gid, int64_t n, int mode,
+                       int16_t* out_scores, uint8_t* out_plays, uint8_t* out_contract,
+                       uint8_t* out_declarer, uint8_t* out_king, uint8_t* out_err,
+                       uint8_t* out_perm, uint8_t* out_cards, uint8_t* out_group, uint64_t* out_discard,
+                       int64_t* out_stats /* [4 seat sums, 4 player sums, env steps, errors] */) {
+    rollout_batch(seed, first_gid, n, mode, NULL, NULL, NULL, NULL, out_scores, out_plays, out_contract, out_declarer,
+                  out_king, out_err, out_perm, out_cards, out_group, out_discard, out_stats, NULL);
+}
+
+/* n injected deals (perm [n,54]) under forced contracts (contract/declarer [n], king [n] or NULL = none), game i with id
+   first_gid + i: what tarok_rollout_host / _records / _host_packed compute.  Same outputs as syn_rollout_batch (out_perm
+   echoes the rows) plus the histogram of the finished games by contract. */
+void syn_rollout_injected_batch(uint64_t seed, uint64_t first_gid, int64_t n, const uint8_t* perm, const uint8_t* contract,
+                                const uint8_t* declarer, const uint8_t* king,
+                                int16_t* out_scores, uint8_t* out_plays, uint8_t* out_contract,
+                                uint8_t* out_declarer, uint8_t* out_king, uint8_t* out_err,
+                                uint8_t* out_perm, uint8_t* out_cards, uint8_t* out_group, uint64_t* out_discard,
+                                int64_t* out_stats, int64_t* out_hist) {
+    rollout_batch(seed, first_gid, n, -1, perm, contract, declarer, king, out_scores, out_plays, out_contract, out_declarer,
+                  out_king, out_err, out_perm, out_cards, out_group, out_discard, out_stats, out_hist);
 }
 
 void syn_deal_batch(uint64_t seed, uint64_t first_gid, int64_t n, uint8_t* out_perm) {

@@ -532,10 +532,33 @@ def test_ragged_batch_sizes(oracle, n):
         env.close()
 
 
-def test_config5_size_properties():
-    """16,777,216 concurrent deals (BASELINE config 5 total) with bidding: size-independent invariants."""
+def _force_graph(env):
+    """TAROK_OPT_GRAPH = 2: the stepwise rollout replays its CUDA graph at every batch size (set_graph passes 0 or 1)."""
+    env._check(env._lib.tarok_set_option(env._h, 8, 2))
+
+
+def _score_windows(env, ref, windows, what):
+    for a, b in windows:
+        sc = env.scores[a:b].cpu().numpy()
+        bad = np.flatnonzero((sc != ref["scores"][a:b]).any(axis=1))
+        assert bad.size == 0, "%s: games %s of [%d, %d) differ from the oracle" % (what, (a + bad[:8]).tolist(), a, b)
+
+
+def test_config5_size_properties(oracle):
+    """16,777,216 concurrent deals (BASELINE config 5 total) with bidding: see _large_batch_against_oracle."""
+    _large_batch_against_oracle(oracle, 1 << 24, (17,))
+
+
+def test_config3_size_matches_oracle(oracle):
+    """4,194,304 concurrent deals (BASELINE config 3 at N = 1), uniform and Bot-model bids: see _large_batch_against_oracle."""
+    _large_batch_against_oracle(oracle, 1 << 22, (17, 18))
+
+
+def _large_batch_against_oracle(oracle, n, modes):
+    """Size-independent invariants, then bench.py's sequence for batch 1 of the leg against the oracle over every game.
+    Above 3 M deals the defaults change (no CUDA graph, no draw cache): the statistics and three windows of scores must also
+    hold with the draw cache forced on, through the fused kernel and through the stepwise rollout with the graph forced."""
     import tarok_b200.env as E
-    n = 1 << 24
     env = _env(n, seed=2026)
     env.rollout(E.MODE_AUCTION_UNIFORM, first_game_id=0)
     st = env.stats()
@@ -558,12 +581,40 @@ def test_config5_size_properties():
     env.rollout(E.MODE_AUCTION_UNIFORM, first_game_id=0, fused=True)
     assert (env.stats()[:21] == st[:21]).all()
     del hands, meta, err, berac, allc, plays        # zero-copy views must be dropped before the handle can be destroyed
+
+    gid0 = n                                        # bench.py's batch 1 of the leg: global game ids [total, 2 * total)
+    mid = 1 << 23 if n > 1 << 23 else n // 2
+    windows = [(0, 20000), (mid - 10000, mid + 10000), (n - 20000, n)]
+    env.set_materialise(False)
+    for mode in modes:
+        ref = oracle.rollout(2026, gid0, n, mode, full=False)
+        want = oracle.device_stats(ref)
+        for how in ("bench", "draw cache 3", "fused", "stepwise, graph forced"):
+            env.reset_stats()
+            if how == "fused":
+                env.rollout(mode, first_game_id=gid0, fused=True)
+            elif how.startswith("stepwise"):
+                _force_graph(env)
+                env.rollout(mode, first_game_id=gid0, fused=False)
+                env.set_graph(True)
+            else:
+                env.set_draw_cache(3 if how == "draw cache 3" else -1)
+                env.setup_synth(mode, gid0)
+                env.step_random(48)
+                env.score()
+            st = env.stats()[:21]
+            what = "mode %d, %s" % (mode, how)
+            assert (st == want).all(), "%s: stats %s != oracle %s" % (what, st.tolist(), want.tolist())
+            _score_windows(env, ref, windows, what)
+        env.set_draw_cache(-1)
+        del ref
     env.close()
 
 
-def test_near_maximum_batch_uses_64_bit_indices():
+def test_near_maximum_batch_uses_64_bit_indices(oracle):
     """400 M concurrent deals (61 GB of state; the handle takes up to 2^29): row offsets into the 12-row trick log and the
-    48-row history exceed 2^32 there.  Stepwise (trick log -> k_score) and fused (registers) must still agree."""
+    48-row history exceed 2^32 there.  Stepwise (trick log -> k_score) and fused (registers) must still agree, and the
+    stepwise scores of the last 100,000 games and of 100,000 games around game 2^28 must be the oracle's."""
     import torch
     free, _ = torch.cuda.mem_get_info()
     if free < 90 << 30:
@@ -573,12 +624,67 @@ def test_near_maximum_batch_uses_64_bit_indices():
     env.set_materialise(False)
     env.rollout(17, first_game_id=0, fused=False)
     a = env.stats().copy()
+    for lo in ((1 << 28) - 50_000, n - 100_000):
+        ref = oracle.rollout(7, lo, 100_000, 17, full=False)
+        sc = env.scores[lo:lo + 100_000].cpu().numpy()
+        assert (sc == ref["scores"]).all(), lo
     env.reset_stats()
     env.rollout(17, first_game_id=0, fused=True)
     b = env.stats().copy()
     env.close()
     assert (a[:21] == b[:21]).all()
     assert a[18] + a[20] == n and a[20] < n // 10000
+
+
+def test_history_past_32_bit_row_offsets(oracle):
+    """100,000,000 history-keeping deals: the [48, n] history rows start past 2^32 bytes from play 43 on (48 x n_alloc > 2^32
+    above about 91.4 M deals), so every row offset must be 64-bit.  The history, the hands as dealt and the discards of the
+    first and last 50,000 games are the oracle's, through the stepwise and the fused rollout; a 50,000-game handle that holds
+    the last games under the same ids gives the same replay targets and observations."""
+    import torch
+    free, _ = torch.cuda.mem_get_info()
+    if free < 55 << 30:
+        pytest.skip("needs 55 GB of free device memory")
+    n, w, gid0, seed, mode = 100_000_000, 50_000, 2 ** 32 + 4321, 99, 16
+    assert 47 * (n + 512) > 1 << 32
+    env = _env(n, seed=seed, history=True)
+    refs = {lo: oracle.rollout(seed, gid0 + lo, w, mode) for lo in (0, n - w)}
+    for fused in (False, True):
+        env.rollout(mode, first_game_id=gid0, fused=fused)
+        for lo, ref in refs.items():
+            what = "%s rollout, games [%d, %d)" % ("fused" if fused else "stepwise", lo, lo + w)
+            rep = oracle.replay(ref["perm"], ref["contract"], ref["declarer"], ref["king"], ref["group"], ref["discard"],
+                                ref["cards"], want_state=False)
+            hist = env.hist[:, lo:lo + w].cpu().numpy().T
+            want = np.where(ref["cards"] == 0xFF, 0xFF, (rep["seat"] << 6) | ref["cards"]).astype(np.uint8)
+            assert (hist == want).all(), what
+            hands0 = u64(env.hands0[:, lo:lo + w])
+            for s in range(4):
+                bits = np.uint64(1) << ref["perm"][:, 12 * s:12 * s + 12].astype(np.uint64)
+                assert (hands0[s] == np.bitwise_or.reduce(bits, axis=1)).all(), (what, s)
+            assert (u64(env.discard[lo:lo + w]) == ref["discard"]).all(), what
+            assert (env.scores[lo:lo + w].cpu().numpy() == ref["scores"]).all(), what
+
+    small = _env(w, seed=seed, history=True)
+    small.rollout(mode, first_game_id=gid0 + n - w, fused=True)
+    sel = np.arange(n - w, n, dtype=np.int32)
+    big_t, small_t = env.targets(sel), small.targets()
+    for x, y in zip(big_t, small_t):
+        assert (x.cpu().numpy() == y.cpu().numpy()).all()
+    seat, rows = small_t[1].cpu().numpy(), small_t[2].cpu().numpy()
+    sub = np.arange(4096)
+    for t in (0, 21, 47):
+        played = seat[sub, t] != 0xFF                  # the observation a replay sample of play t was made from: (type, T)
+        for T in np.unique(rows[sub, t][played]):
+            games = sub[played & (rows[sub, t] == T)].astype(np.int32)
+            a, ok_a = env.obs_expand(1, int(T), games + (n - w), play=t)
+            b, ok_b = small.obs_expand(1, int(T), games, play=t)
+            assert ok_b.cpu().numpy().all() and (ok_a.cpu().numpy() == ok_b.cpu().numpy()).all(), (t, T)
+            for x, y in zip(a, b):
+                assert (x.cpu().numpy() == y.cpu().numpy()).all(), (t, T)
+    del big_t, small_t
+    small.close()
+    env.close()
 
 
 @pytest.mark.parametrize("mode", [0, 7, 9, 16, 17, 18])

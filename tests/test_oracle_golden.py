@@ -5,6 +5,7 @@ import json
 import os
 
 import numpy as np
+import pytest
 
 from conftest import GOLDEN
 
@@ -120,3 +121,18 @@ def test_cpu_rollout_teacher_forced_consistency(oracle):
         assert (rep["plays"][ok] == r["plays"][ok]).all()
         assert r["stats"][8] == r["plays"].astype(np.int64).sum()
 
+
+
+@pytest.mark.parametrize("first_gid", [2 ** 32 + 7, 1000])          # odd / even: two games share a Philox play block
+@pytest.mark.parametrize("mode", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 16])
+def test_injected_rollout_reproduces_the_synthetic_one(oracle, mode, first_gid):
+    """The host-buffer reference (the rows and forced contracts given, talon group 0) on what the synthetic rollout dealt
+    and chose plays the same games: the two share the exchange and play-out, and differ only in where the deal and
+    the contract come from."""
+    n = 4000
+    r = oracle.rollout(31, first_gid, n, mode)
+    k = oracle.rollout_injected(31, first_gid, r["perm"], r["contract"], r["declarer"], r["king"])
+    for key in ("scores", "cards", "plays", "err", "stats", "contract", "declarer", "king", "group", "discard"):
+        assert (k[key] == r[key]).all(), key
+    assert (k["hist"] == np.bincount(r["contract"][r["err"] == 0], minlength=10)).all()
+    assert k["hist"].sum() == n - r["stats"][9]
