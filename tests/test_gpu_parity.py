@@ -705,7 +705,9 @@ def test_scores_only_path_matches_oracle(oracle, mode):
                                            (3, True, True), (3, False, True)])
 def test_every_play_step_variant_matches_oracle(oracle, impl, pdl, lock):
     """The selectable play_step implementations (plain / TMA-staged general path / persistent prefetching lock-step kernel, PDL
-    on/off, lock-step specialisation on/off) all produce the oracle's games, graph-backed or not."""
+    on/off, lock-step specialisation on/off) all produce the oracle's games through the stepwise rollout (graph-backed, except
+    with impl 2) and external cards (impl 3 takes the plain kernel for those).  70,001 deals are 137 tiles, less than one
+    wave of the persistent grids, so each of their CTAs handles one tile: tests/test_gpu_step_variants.py covers the loops."""
     n, seed = 70001, 31
     for mode in (17, 0):
         ref = oracle.rollout(seed, 10, n, mode)
