@@ -76,7 +76,10 @@ enum { TAROK_F_HANDS = 0,   /* uint64 [4, n_alloc]  hand bitboards (Roka, Roka.p
        TAROK_F_QMAX_HIST = 11 /* float [48, n_alloc] next_Q_max recorded by tarok_select_action at play t; HISTORY flag */
 };
 /* stats vector: [0..3] score sum by seat, [4..7] score sum by player ((seat+game_id)%4, Tarok.py:34,59-61),
-   [8..17] contract histogram, [18] finished deals, [19] env-steps (card plays), [20] error games */
+   [8..17] contract histogram, [18] finished deals, [19] env-steps (card plays), [20] error games (these at scoring);
+   [21] error events: counted at once by the stepwise call that makes a game an error game (tarok_set_deals,
+   tarok_auction, tarok_force_contract, tarok_exchange, tarok_step, tarok_setup_synth), so at most once per game and
+   deal; the fused kernel does not count them. */
 #define TAROK_STATS_LEN 32
 
 /* ---- life cycle ---------------------------------------------------------------------------- */
@@ -120,7 +123,8 @@ int tarok_export_perm(tarok_t* h, uint8_t* out_dev, void* stream);
 /* intent_dev: uint8 [n_games, 4]; one bid intent per seat as an index into
    Nevronski_igralec.index2igra (Igralec.py:717-745): 0 Naprej, 1-12 (Tri|Dve|Ena, king suit),
    13-15 Solo_tri/dve/ena, 16 Berac, 17 Solo_brez; additionally 18 Odprti_berac, 19 Klop.
-   Fixed-intent semantics of Nevronski_igralec.licitiram (Igralec.py:294-306). */
+   Fixed-intent semantics of Nevronski_igralec.licitiram (Igralec.py:294-306): every seat is asked at least once, so a
+   game with any intent in 20..255 becomes an error game (the reference's index2igra[idx] raises). */
 int tarok_auction(tarok_t* h, const uint8_t* intent_dev, void* stream);
 int tarok_auction_synth(tarok_t* h, uint32_t mode /* 17 | 18 */, void* stream);
 /* Bypass bidding like the per-contract constructors Klop(...)/Navadna_igra(...)/Berac(...).

@@ -204,6 +204,7 @@ int orc_zacni_igro(orc_game* g, int contract, int declarer, int king) {   /* Igr
     g->contract = contract; g->declarer = declarer;
     g->king = is_king_game(contract) ? king : ORC_NO_KING;   /* king only asked for Ena/Dve/Tri, Igra.py:42-43 */
     memset(g->ekipa, 0, sizeof(g->ekipa));
+    if (declarer < 0 || declarer > 3) { g->error = 1; return -1; }   /* no such player, whatever the contract (Klop too) */
     if (is_navadna(contract)) {
         if (is_king_game(contract)) {                         /* Navadna_igra.py:20-25 */
             if (king < 0 || king > 3) { g->error = 1; return -1; }   /* assert barva_kralja != TAROK */
@@ -243,9 +244,10 @@ int orc_menjaj(orc_game* g, int group, const uint8_t* discards, int k) {
         g->error = 1; return -1;
     }
     int d = g->declarer;
-    for (int j = 0; j < g->group_sz; j++) roka_append(g, d, g->group[group][j]);
+    orc_game t = *g;                                           /* a refused exchange leaves the game as it was */
+    for (int j = 0; j < t.group_sz; j++) roka_append(&t, d, t.group[group][j]);
     uint8_t mozno[16];
-    int nm = orc_mozno_zalozit(g, d, mozno);
+    int nm = orc_mozno_zalozit(&t, d, mozno);
     if (nm < k) { g->error = 1; return -1; }                   /* random.sample would raise (Q19) */
     for (int i = 0; i < k; i++) {
         int ok = 0;
@@ -254,12 +256,13 @@ int orc_menjaj(orc_game* g, int group, const uint8_t* discards, int k) {
         if (!ok) { g->error = 1; return -1; }
     }
     for (int i = 0; i < k; i++) {
-        g->pile[d][g->pile_n[d]++] = discards[i];              /* kupcek.extend(izberi) */
-        roka_remove(g, d, discards[i]);
+        t.pile[d][t.pile_n[d]++] = discards[i];                /* kupcek.extend(izberi) */
+        roka_remove(&t, d, discards[i]);
     }
-    g->chosen_group = (uint8_t)group;
-    g->group_alive[group] = 0;                                 /* del kupcki_talona[stevilka_kupcka] */
-    g->phase = 2;
+    t.chosen_group = (uint8_t)group;
+    t.group_alive[group] = 0;                                  /* del kupcki_talona[stevilka_kupcka] */
+    t.phase = 2;
+    *g = t;
     return 0;
 }
 
@@ -476,13 +479,36 @@ static uint64_t pile_mask(const orc_game* g, int s) {
 }
 static uint64_t talon_mask(const orc_game* g) {
     uint64_t m = 0;
-    if (is_navadna(g->contract)) {
+    if (is_navadna(g->contract) && g->group_cnt) {             /* (a rejected contract never split the talon) */
         for (int i = 0; i < g->group_cnt; i++)
             if (g->group_alive[i]) for (int j = 0; j < g->group_sz; j++) m |= 1ull << g->group[i][j];
     } else {
         for (int i = 0; i < g->talon_n; i++) m |= 1ull << g->talon[i];
     }
     return m;
+}
+
+/* Deal + contract of one game of the batch drivers.  A row that is not a permutation of 0..53 is an error game with
+   nothing dealt, the rule k_set_deals applies; orc_razdeli would index past its lists. */
+static void deal_and_start(orc_game* g, const uint8_t perm[54], int contract, int declarer, int king) {
+    uint64_t seen = 0;
+    for (int i = 0; i < 54; i++) if (perm[i] < 54) seen |= 1ull << perm[i];
+    if (seen != (1ull << 54) - 1) {
+        memset(g, 0, sizeof(*g));
+        g->error = 1;
+        return;
+    }
+    orc_razdeli(g, perm);
+    orc_zacni_igro(g, contract, declarer, king);
+}
+
+/* The exchange as a discard bitboard: a mask with more than three cards or a bit above card 53 is an invalid exchange. */
+static void menjaj_mask(orc_game* g, int group, uint64_t mask) {
+    uint8_t d[3] = { 0, 0, 0 };
+    int k = 0;
+    for (int c = 0; c < 54 && k < 3; c++) if ((mask >> c) & 1) d[k++] = (uint8_t)c;
+    int kk = __builtin_popcountll(mask);
+    orc_menjaj(g, group, d, (kk > 3 || (mask >> 54)) ? 99 : kk);
 }
 
 void orc_replay_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, const uint8_t* declarer,
@@ -493,15 +519,8 @@ void orc_replay_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, c
 #pragma omp parallel for schedule(static)
     for (int64_t i = 0; i < n; i++) {
         orc_game g;
-        orc_razdeli(&g, perm + 54 * i);
-        orc_zacni_igro(&g, contract[i], declarer[i], king[i]);
-        if (!g.error && g.phase == 1) {
-            uint8_t d[3];
-            int k = 0;
-            for (int c = 0; c < 54 && k < 3; c++) if ((discard_mask[i] >> c) & 1) d[k++] = (uint8_t)c;
-            int kk = __builtin_popcountll(discard_mask[i]);
-            orc_menjaj(&g, group[i], d, kk > 3 ? 99 : kk);
-        }
+        deal_and_start(&g, perm + 54 * i, contract[i], declarer[i], king[i]);
+        if (!g.error && g.phase == 1) menjaj_mask(&g, group[i], discard_mask[i]);
         for (int t = 0; t < 48; t++) { if (out_seat) out_seat[48 * i + t] = 0xFF; if (out_mask) out_mask[48 * i + t] = 0; }
         for (int t = 0; t < 12; t++) if (out_winner) out_winner[12 * i + t] = 0xFF;
         int t = 0;
@@ -538,8 +557,7 @@ void orc_lists_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, co
 #pragma omp parallel for schedule(static)
     for (int64_t i = 0; i < n; i++) {
         orc_game g;
-        orc_razdeli(&g, perm + 54 * i);
-        orc_zacni_igro(&g, contract[i], declarer[i], king[i]);
+        deal_and_start(&g, perm + 54 * i, contract[i], declarer[i], king[i]);
         memset(out_mozne + 48 * 16 * i, 0xFF, 48 * 16);
         memset(out_mozne_n + 48 * i, 0, 48);
         memset(out_seat + 48 * i, 0xFF, 48);
@@ -555,11 +573,7 @@ void orc_lists_batch(int64_t n, const uint8_t* perm, const uint8_t* contract, co
                 for (int j = 0; j < tmp.group_sz; j++) roka_append(&tmp, tmp.declarer, tmp.group[group[i]][j]);
                 out_zalozit_n[i] = (uint8_t)orc_mozno_zalozit(&tmp, tmp.declarer, out_zalozit + 16 * i);
             }
-            uint8_t d[3];
-            int k = 0;
-            for (int c = 0; c < 54 && k < 3; c++) if ((discard_mask[i] >> c) & 1) d[k++] = (uint8_t)c;
-            int kk = __builtin_popcountll(discard_mask[i]);
-            orc_menjaj(&g, group[i], d, kk > 3 ? 99 : kk);
+            menjaj_mask(&g, group[i], discard_mask[i]);
         }
         int t = 0;
         while (!g.error && g.phase == 2 && t < 48) {

@@ -462,6 +462,9 @@ __device__ __forceinline__ void resolve_contract(const Rng& rng, u64 gid, u32 mo
         contract = (u32)k; declarer = (u32)d;
         // king = the suit attached to the declarer's ORIGINAL intent (Igralec.py:298,308-310)
         king = d == 0 ? su[0] : d == 1 ? su[1] : d == 2 ? su[2] : su[3];
+        // every seat is asked at least once, so every intent counts: one past index 19 (index2igra[idx] would raise in
+        // the reference) makes an error game through begin_contract's unknown-contract check
+        if (max(max((u32)in.x, (u32)in.y), max((u32)in.z, (u32)in.w)) > 19u) contract = C_NONE;
     } else {
         if (mode == 17u) {          // TAROK_MODE_AUCTION_UNIFORM: four batched draws of [0,18) from word 0 of the bid block
             u32 x = philox_block(rng, gid, ST_BID, 0u).w[0];

@@ -237,7 +237,8 @@ __device__ __forceinline__ void licitacija(Want& want, int& declarer, int& contr
     contract = mx;
 }
 
-// Nevronski_igralec.index2igra (Igralec.py:717-745) + two raw extras (18 Odprti_berac, 19 Klop)
+// Nevronski_igralec.index2igra (Igralec.py:717-745) + two raw extras (18 Odprti_berac, 19 Klop); idx <= 19 (callers reject
+// larger indices: tarok_auction makes them error games)
 __device__ __forceinline__ void index2igra(u32 idx, int& tip, u32& suit) {
     suit = NO_KING;
     if (idx == 0) tip = C_NAPREJ;

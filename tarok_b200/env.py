@@ -215,7 +215,8 @@ class TarokEnv:
 
     # ------------------------------------------------------------------ auction / dispatch
     def auction(self, intents):
-        """intents: uint8 [n,4] indices into ``Nevronski_igralec.index2igra`` (Igralec.py:717-745)."""
+        """intents: uint8 [n,4] indices into ``Nevronski_igralec.index2igra`` (Igralec.py:717-745), 0..19 (18 Odprti_berac,
+        19 Klop); a game with any intent in 20..255 becomes an error game."""
         x = self._dev_u8(intents, (self.n, 4))
         self._check(self._lib.tarok_auction(self._h, C.c_void_p(x.data_ptr()), self._stream()))
 

@@ -136,3 +136,95 @@ def test_injected_rollout_reproduces_the_synthetic_one(oracle, mode, first_gid):
         assert (k[key] == r[key]).all(), key
     assert (k["hist"] == np.bincount(r["contract"][r["err"] == 0], minlength=10)).all()
     assert k["hist"].sum() == n - r["stats"][9]
+
+
+# ---- inputs a caller can get wrong: the oracle's verdict, and the state it leaves, are defined for every byte -----------
+
+IDENTITY = np.arange(54, dtype=np.uint8)   # seat s holds ids 12s..12s+11, the talon 48..53 in order
+
+
+def _one(O, perm, contract, declarer, king=7, group=0xFF, discard=0, cards=()):
+    """replay and lists of hand-built rows (one per entry of the lists)."""
+    n = len(perm)
+    c = np.full((n, 48), 0xFF, np.uint8)
+    for i, row in enumerate(cards or [()] * n):
+        c[i, :len(row)] = row
+    bc = lambda x: np.broadcast_to(np.asarray(x), (n,))
+    args = (np.asarray(perm, np.uint8), bc(contract).astype(np.uint8), bc(declarer).astype(np.uint8),
+            bc(king).astype(np.uint8), bc(group).astype(np.uint8), bc(discard).astype(np.uint64), c)
+    return O.replay(*args), O.lists(*args)
+
+
+def _dealt(perm):
+    hands = np.zeros(4, np.uint64)
+    for s in range(4):
+        for c in perm[12 * s:12 * s + 12]:
+            hands[s] |= np.uint64(1 << int(c))
+    talon = np.uint64(sum(1 << int(c) for c in perm[48:]))
+    return hands, talon
+
+
+def test_oracle_rejects_rows_that_are_not_permutations(oracle):
+    """A duplicate id, an id 54..63 or an id 64..255, in a hand or in the talon, makes an error game before anything is
+    dealt (k_set_deals' rule): no plays, no score, empty hands, piles and talon, empty lists -- whatever the contract."""
+    rows = []
+    for pos in (0, 11, 47, 48, 53):
+        for bad in ("dup", 54, 63, 64, 200, 255):
+            p = IDENTITY.copy()
+            p[pos] = p[(pos + 1) % 54] if bad == "dup" else bad
+            rows.append(p)
+    n = len(rows)
+    for contract, declarer, king in ((0, 0, 7), (1, 2, 1), (4, 3, 7), (7, 1, 7)):
+        first = [[0] * 4] * n                                 # cards that would be legal in a valid deal
+        rep, lst = _one(oracle, rows, contract, declarer, king, group=0, discard=0b111, cards=first)
+        assert (rep["err"] == 1).all() and (rep["plays"] == 0).all() and (rep["scores"] == 0).all()
+        assert (rep["hands"] == 0).all() and (rep["piles"] == 0).all() and (rep["talon"] == 0).all()
+        assert (rep["seat"] == 0xFF).all() and (rep["mask"] == 0).all()
+        assert (lst["mozne_n"] == 0).all() and (lst["zalozit_n"] == 0).all() and (lst["groups"] == 0xFF).all()
+        assert (lst["seat"] == 0xFF).all()
+
+
+@pytest.mark.parametrize("contract", range(10))
+def test_oracle_rejects_a_declarer_above_3_for_every_contract(oracle, contract):
+    """Declarer 4, 5 or 255 is an error game under every contract, Klop included (begin_contract's rule; the reference has no
+    such player).  The deal stays as dealt; a valid declarer still plays."""
+    dh, dt = _dealt(IDENTITY)
+    rep, lst = _one(oracle, [IDENTITY] * 4, contract, [4, 5, 255, 3], king=1, group=0xFF, discard=0)
+    assert rep["err"][:3].tolist() == [1, 1, 1]
+    assert (rep["hands"][:3] == dh).all() and (rep["talon"][:3] == dt).all() and (rep["piles"][:3] == 0).all()
+    assert (lst["mozne_n"][:3] == 0).all()
+    exchange = 1 <= contract <= 6                             # declarer 3 then waits for the exchange this row does not make
+    assert rep["err"][3] == (1 if exchange else 0)
+    if not exchange:
+        assert lst["mozne_n"][3, 0] > 0
+
+
+def test_oracle_rejects_discard_bits_above_53_and_leaves_a_refused_exchange_untouched(oracle):
+    """Tri (k = 3), declarer 0, talon group 0 = ids 48..50.  A discard mask with a bit in 54..63 is an invalid exchange even
+    when its other bits are a valid set; so are kings, trula cards, cards of another seat or of a group not chosen, and a
+    wrong count.  A refused exchange leaves hands, piles and talon as dealt; a valid one (picked-up cards included) plays."""
+    dh, dt = _dealt(IDENTITY)
+    b = lambda *ids: sum(1 << i for i in ids)
+    cases = [
+        (b(0, 1, 60), 1), (b(0, 1, 2, 54), 1), (b(0, 1, 63), 1), (b(0, 1, 2) | (1 << 63), 1),
+        (b(0, 1, 7), 1),                    # the kara king
+        (b(0, 1, 32), 1), (b(0, 1, 52), 1), # pagat / mond (seat 0 holds neither: also another seat's)
+        (b(0, 1, 12), 1),                   # seat 1's card
+        (b(0, 1, 51), 1),                   # group 1's card
+        (b(0, 1), 1), (b(0, 1, 2, 3), 1), (0, 1),
+        (b(0, 1, 2), 0), (b(0, 1, 48), 1),  # XVII is not discardable (Karta.vrednost 5 above VII)
+        (b(5, 6, 8), 0),
+    ]
+    perm = [IDENTITY] * len(cases)
+    rep, _ = _one(oracle, perm, 1, 0, king=1, group=0, discard=[m for m, _ in cases])
+    assert rep["err"].tolist() == [e for _, e in cases]
+    bad = rep["err"] == 1
+    assert (rep["hands"][bad] == dh).all() and (rep["piles"][bad] == 0).all() and (rep["talon"][bad] == dt).all()
+    grp0 = np.uint64(b(48, 49, 50))
+    for i in np.nonzero(~bad)[0]:
+        m = np.uint64(cases[i][0])
+        assert rep["hands"][i, 0] == (dh[0] | grp0) & ~m and rep["piles"][i, 0] == m
+        assert rep["talon"][i] == dt & ~grp0
+    # groups past the last (6 / k = 2 for Tri), 7 and 255 are invalid too
+    rep, _ = _one(oracle, [IDENTITY] * 3, 1, 0, king=1, group=[2, 7, 255], discard=b(0, 1, 2))
+    assert (rep["err"] == 1).all() and (rep["hands"] == dh).all() and (rep["talon"] == dt).all()
