@@ -302,6 +302,37 @@ int tarok_obs_exchange(tarok_t* h, const int32_t* sel_dev, uint64_t n_sel, float
 int tarok_select_exchange(tarok_t* h, const float* p_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
                           uint8_t* group_dev, uint64_t* discard_dev, void* stream);
 
+/* ---- mixed precision: the observation and selection entries above in bf16 / fp16 ----------- */
+/* Element type of the observation outputs and of the network outputs the selections read.  Every observation value is
+   exactly 0 or 1, so bf16 and fp16 observations equal the fp32 ones converted, bit for bit, at half the bytes.  Network
+   outputs are widened to fp32 (exact) and then selected by the fp32 rules: the first NaN wins, -inf and -max are ordinary
+   values, +0 == -0, ties go by the reference's `mozne` order (cards) and by the stable mozno_zalozit order (discards).
+   qmax_dev, TAROK_F_QMAX_HIST and tarok_targets stay fp32. */
+#define TAROK_DTYPE_F32 0
+#define TAROK_DTYPE_BF16 1
+#define TAROK_DTYPE_F16 2
+/* Each *_ex entry is the entry of the same name with buffers of element type `dtype` (an unknown dtype is an error); the
+   fp32 entries are these at TAROK_DTYPE_F32.  Alignment at every dtype: opp / hand 16 bytes; talon, talon_klop, discard,
+   mozne and the exchange hand / talon two elements (8 bytes fp32, 4 bytes bf16 / fp16); king / decl 4 bytes; every other
+   buffer one element.  A call that fails its checks writes nothing. */
+int tarok_obs_expand_at_ex(tarok_t* h, int dtype, int play, int net_type, uint32_t rows, const int32_t* sel_dev, uint64_t n_sel,
+                           void* opp_dev, void* hand_dev, void* talon_dev, void* king_dev, void* decl_dev,
+                           void* discard_dev, void* mozne_dev, uint8_t* ok_dev, void* stream);
+int tarok_obs_expand_buckets_ex(tarok_t* h, int dtype, const int32_t* sel_dev, const uint8_t* selkey_dev, const uint32_t* counts_dev,
+                                uint64_t n_total, void* opp_dev, void* hand_dev, void* talon_dev, void* talon_klop_dev,
+                                void* king_dev, void* decl_dev, void* discard_dev, void* stream);
+int tarok_obs_hands_ex(tarok_t* h, int dtype, void* out_dev, void* stream);
+int tarok_obs_exchange_ex(tarok_t* h, int dtype, const int32_t* sel_dev, uint64_t n_sel, void* hand_dev, void* talon_dev,
+                          void* game_dev, uint8_t* ok_dev, void* stream);
+int tarok_select_action_ex(tarok_t* h, int dtype, const void* q_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
+                           uint8_t* card_dev, float* qmax_dev, void* stream);
+/* One dtype for every pointer of the table. */
+int tarok_select_action_buckets_tab_ex(tarok_t* h, int dtype, const void* const* q_ptrs_host, const int32_t* sel_dev,
+                                       const uint8_t* selkey_dev, const uint32_t* counts_dev, uint64_t n_total,
+                                       const float* random_card4, uint8_t* card_dev, float* qmax_dev, void* stream);
+int tarok_select_exchange_ex(tarok_t* h, int dtype, const void* p_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
+                             uint8_t* group_dev, uint64_t* discard_dev, void* stream);
+
 /* ---- zero-copy views ------------------------------------------------------------------------- */
 /* Lends a field as a DLPack tensor that aliases the handle's device memory.  The caller (e.g.
    torch.from_dlpack) must call the deleter; the handle cannot be destroyed before that. */

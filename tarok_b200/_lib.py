@@ -64,6 +64,13 @@ SIGNATURES = {
     "tarok_obs_hands": (_I, [_VP, _VP, _VP]),
     "tarok_obs_exchange": (_I, [_VP, _VP, _U64, _VP, _VP, _VP, _VP, _VP]),
     "tarok_select_exchange": (_I, [_VP, _VP, _VP, _U64, C.c_float, _VP, _VP, _VP]),
+    "tarok_obs_expand_at_ex": (_I, [_VP, _I, _I, _I, _U32, _VP, _U64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "tarok_obs_expand_buckets_ex": (_I, [_VP, _I, _VP, _VP, _VP, _U64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "tarok_obs_hands_ex": (_I, [_VP, _I, _VP, _VP]),
+    "tarok_obs_exchange_ex": (_I, [_VP, _I, _VP, _U64, _VP, _VP, _VP, _VP, _VP]),
+    "tarok_select_action_ex": (_I, [_VP, _I, _VP, _VP, _U64, C.c_float, _VP, _VP, _VP]),
+    "tarok_select_action_buckets_tab_ex": (_I, [_VP, _I, _VP, _VP, _VP, _VP, _U64, _VP, _VP, _VP, _VP]),
+    "tarok_select_exchange_ex": (_I, [_VP, _I, _VP, _VP, _U64, C.c_float, _VP, _VP, _VP]),
     "tarok_export": (_I, [_VP, _I, C.POINTER(_VP)]),
     "tarok_field_ptr": (_VP, [_VP, _I]),
     "tarok_launch_count": (_U64, [_VP]),

@@ -188,6 +188,17 @@ static int random_chain(tarok_env* h, uint32_t count, cudaStream_t s) {
     return 0;
 }
 
+// TAROK_DTYPE_* -> the element type of the observation / network-output buffers: f(tag) with a value of that type.
+template <class F> static int with_dtype(tarok_env* h, int dtype, F&& f) {
+    switch (dtype) {
+        case TAROK_DTYPE_F32: return f(float{});
+        case TAROK_DTYPE_BF16: return f(__nv_bfloat16{});
+        case TAROK_DTYPE_F16: return f(__half{});
+    }
+    return fail(h, -1, "dtype must be TAROK_DTYPE_F32, TAROK_DTYPE_BF16 or TAROK_DTYPE_F16 (got %d)", dtype);
+}
+static inline bool misaligned(const void* p, uintptr_t bytes) { return ((uintptr_t)p) & (bytes - 1); }
+
 extern "C" {
 
 // The captured graphs freeze every option (kernel variant, launch attributes, parameters): any change drops them.
@@ -879,23 +890,34 @@ int tarok_obs_buckets_host(tarok_t* h, int players, int32_t* sel_dev, uint32_t* 
 int tarok_obs_expand_buckets(tarok_t* h, const int32_t* sel_dev, const uint8_t* selkey_dev, const uint32_t* counts_dev,
                              uint64_t n_total, float* opp_dev, float* hand_dev, float* talon_dev, float* talon_klop_dev,
                              float* king_dev, float* decl_dev, float* discard_dev, void* stream) {
+    return tarok_obs_expand_buckets_ex(h, TAROK_DTYPE_F32, sel_dev, selkey_dev, counts_dev, n_total, opp_dev, hand_dev, talon_dev,
+                                       talon_klop_dev, king_dev, decl_dev, discard_dev, stream);
+}
+
+int tarok_obs_expand_buckets_ex(tarok_t* h, int dtype, const int32_t* sel_dev, const uint8_t* selkey_dev, const uint32_t* counts_dev,
+                                uint64_t n_total, void* opp_dev, void* hand_dev, void* talon_dev, void* talon_klop_dev,
+                                void* king_dev, void* decl_dev, void* discard_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!h->e.hist) return fail(h, -1, "observations need TAROK_FLAG_HISTORY at tarok_create");
-    if (!sel_dev || !selkey_dev || !counts_dev) return fail(h, -1, "sel_dev/selkey_dev/counts_dev is null");
-    if (!opp_dev || !hand_dev || !talon_dev || !talon_klop_dev || !king_dev || !decl_dev || !discard_dev)
-        return fail(h, -1, "every arena pointer is required");
-    if ((((uintptr_t)opp_dev) | ((uintptr_t)hand_dev)) & 15u) return fail(h, -1, "opp_dev/hand_dev must be 16-byte aligned");
-    if ((((uintptr_t)talon_dev) | ((uintptr_t)talon_klop_dev) | ((uintptr_t)discard_dev)) & 7u)
-        return fail(h, -1, "talon/discard arenas must be 8-byte aligned");
-    if (n_total == 0) return 0;
-    if (n_total > h->e.n) return fail(h, -1, "n_total exceeds the number of games");
-    DeviceGuard dg(h->device);
-    tk::ObsArena a = {opp_dev, hand_dev, talon_dev, talon_klop_dev, king_dev, decl_dev, discard_dev};
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_obs_expand_all<<<(unsigned)((n_total + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, (const int*)sel_dev, selkey_dev, counts_dev, n_total, a);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using O = decltype(tag);
+        if (!h->e.hist) return fail(h, -1, "observations need TAROK_FLAG_HISTORY at tarok_create");
+        if (!sel_dev || !selkey_dev || !counts_dev) return fail(h, -1, "sel_dev/selkey_dev/counts_dev is null");
+        if (!opp_dev || !hand_dev || !talon_dev || !talon_klop_dev || !king_dev || !decl_dev || !discard_dev)
+            return fail(h, -1, "every arena pointer is required");
+        if (misaligned(opp_dev, 16) || misaligned(hand_dev, 16)) return fail(h, -1, "opp_dev/hand_dev must be 16-byte aligned");
+        if (misaligned(talon_dev, 2 * sizeof(O)) || misaligned(talon_klop_dev, 2 * sizeof(O)) || misaligned(discard_dev, 2 * sizeof(O)))
+            return fail(h, -1, "talon/discard arenas must be %d-byte aligned", (int)(2 * sizeof(O)));
+        if (misaligned(king_dev, 4) || misaligned(decl_dev, 4)) return fail(h, -1, "king/decl arenas must be 4-byte aligned");
+        if (n_total == 0) return 0;
+        if (n_total > h->e.n) return fail(h, -1, "n_total exceeds the number of games");
+        DeviceGuard dg(h->device);
+        tk::ObsArena<O> a = {(O*)opp_dev, (O*)hand_dev, (O*)talon_dev, (O*)talon_klop_dev, (O*)king_dev, (O*)decl_dev, (O*)discard_dev};
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_obs_expand_all<O><<<(unsigned)((n_total + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, (const int*)sel_dev, selkey_dev, counts_dev, n_total, a);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 // random.random() < random_card as "Philox word < threshold" over 64 bits: random_card = 1 gives 2^32, above every word.
@@ -925,24 +947,37 @@ int tarok_select_action_buckets(tarok_t* h, const float* const* q_ptrs_dev, cons
 int tarok_select_action_buckets_tab(tarok_t* h, const float* const* q_ptrs_host, const int32_t* sel_dev, const uint8_t* selkey_dev,
                                     const uint32_t* counts_dev, uint64_t n_total, const float* random_card4, uint8_t* card_dev,
                                     float* qmax_dev, void* stream) {
+    return tarok_select_action_buckets_tab_ex(h, TAROK_DTYPE_F32, (const void* const*)q_ptrs_host, sel_dev, selkey_dev, counts_dev,
+                                              n_total, random_card4, card_dev, qmax_dev, stream);
+}
+
+int tarok_select_action_buckets_tab_ex(tarok_t* h, int dtype, const void* const* q_ptrs_host, const int32_t* sel_dev,
+                                       const uint8_t* selkey_dev, const uint32_t* counts_dev, uint64_t n_total,
+                                       const float* random_card4, uint8_t* card_dev, float* qmax_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!q_ptrs_host || !sel_dev || !selkey_dev || !counts_dev || !card_dev || !random_card4)
-        return fail(h, -1, "q_ptrs_host/sel_dev/selkey_dev/counts_dev/card_dev/random_card4 is null");
-    tk::Thresholds4 t4;
-    for (int p = 0; p < 4; p++) {
-        if (!(random_card4[p] >= 0.f && random_card4[p] <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
-        t4.t[p] = explore_threshold(random_card4[p]);
-    }
-    if (n_total == 0) return 0;
-    if (n_total > h->e.n) return fail(h, -1, "n_total exceeds the number of games");
-    DeviceGuard dg(h->device);
-    tk::QTable qt;
-    memcpy(qt.p, q_ptrs_host, sizeof(qt.p));
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_select_action_all_tab<<<(unsigned)((n_total + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, qt, (const int*)sel_dev, selkey_dev, counts_dev, n_total, t4, card_dev, qmax_dev);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using Q = decltype(tag);
+        if (!q_ptrs_host || !sel_dev || !selkey_dev || !counts_dev || !card_dev || !random_card4)
+            return fail(h, -1, "q_ptrs_host/sel_dev/selkey_dev/counts_dev/card_dev/random_card4 is null");
+        tk::Thresholds4 t4;
+        for (int p = 0; p < 4; p++) {
+            if (!(random_card4[p] >= 0.f && random_card4[p] <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
+            t4.t[p] = explore_threshold(random_card4[p]);
+        }
+        tk::QTable<Q> qt;
+        for (u32 k = 0; k < tk::BUCKETS; k++) {
+            if (misaligned(q_ptrs_host[k], sizeof(Q))) return fail(h, -1, "q_ptrs_host[%u] is not aligned to its element type", k);
+            qt.p[k] = (const Q*)q_ptrs_host[k];
+        }
+        if (n_total == 0) return 0;
+        if (n_total > h->e.n) return fail(h, -1, "n_total exceeds the number of games");
+        DeviceGuard dg(h->device);
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_select_action_all_tab<Q><<<(unsigned)((n_total + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, qt, (const int*)sel_dev, selkey_dev, counts_dev, n_total, t4, card_dev, qmax_dev);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_obs_expand(tarok_t* h, int net_type, uint32_t rows, const int32_t* sel_dev, uint64_t n_sel, float* opp_dev,
@@ -955,74 +990,124 @@ int tarok_obs_expand(tarok_t* h, int net_type, uint32_t rows, const int32_t* sel
 int tarok_obs_expand_at(tarok_t* h, int play, int net_type, uint32_t rows, const int32_t* sel_dev, uint64_t n_sel,
                         float* opp_dev, float* hand_dev, float* talon_dev, float* king_dev, float* decl_dev,
                         float* discard_dev, float* mozne_dev, uint8_t* ok_dev, void* stream) {
+    return tarok_obs_expand_at_ex(h, TAROK_DTYPE_F32, play, net_type, rows, sel_dev, n_sel, opp_dev, hand_dev, talon_dev, king_dev,
+                                  decl_dev, discard_dev, mozne_dev, ok_dev, stream);
+}
+
+int tarok_obs_expand_at_ex(tarok_t* h, int dtype, int play, int net_type, uint32_t rows, const int32_t* sel_dev, uint64_t n_sel,
+                           void* opp_dev, void* hand_dev, void* talon_dev, void* king_dev, void* decl_dev,
+                           void* discard_dev, void* mozne_dev, uint8_t* ok_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (play >= 48) return fail(h, -1, "play must be < 48");
-    if (!h->e.hist) return fail(h, -1, "observations need TAROK_FLAG_HISTORY at tarok_create");
-    if (net_type < 0 || net_type > 3) return fail(h, -1, "net_type must be 0..3");
-    if (rows == 0 || (rows & 7u) || rows > 56) return fail(h, -1, "rows must be a multiple of 8 in 8..56");
-    if (!opp_dev || !hand_dev) return fail(h, -1, "opp_dev/hand_dev is null");
-    if ((((uintptr_t)opp_dev) | ((uintptr_t)hand_dev)) & 15u) return fail(h, -1, "opp_dev/hand_dev must be 16-byte aligned");
-    if (n_sel == 0) return 0;
-    DeviceGuard dg(h->device);
-    tk::ObsOut o = {opp_dev, hand_dev, talon_dev, king_dev, decl_dev, discard_dev, mozne_dev, ok_dev};
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_obs_expand<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, net_type, rows, (const int*)sel_dev, n_sel, o, play < 0 ? -1 : play);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using O = decltype(tag);
+        if (play >= 48) return fail(h, -1, "play must be < 48");
+        if (!h->e.hist) return fail(h, -1, "observations need TAROK_FLAG_HISTORY at tarok_create");
+        if (net_type < 0 || net_type > 3) return fail(h, -1, "net_type must be 0..3");
+        if (rows == 0 || (rows & 7u) || rows > 56) return fail(h, -1, "rows must be a multiple of 8 in 8..56");
+        if (!opp_dev || !hand_dev) return fail(h, -1, "opp_dev/hand_dev is null");
+        if (misaligned(opp_dev, 16) || misaligned(hand_dev, 16)) return fail(h, -1, "opp_dev/hand_dev must be 16-byte aligned");
+        if (misaligned(talon_dev, 2 * sizeof(O)) || misaligned(discard_dev, 2 * sizeof(O)) || misaligned(mozne_dev, 2 * sizeof(O)))
+            return fail(h, -1, "talon/discard/mozne must be %d-byte aligned", (int)(2 * sizeof(O)));
+        if (misaligned(king_dev, 4) || misaligned(decl_dev, 4)) return fail(h, -1, "king/decl must be 4-byte aligned");
+        if (n_sel == 0) return 0;
+        DeviceGuard dg(h->device);
+        tk::ObsOut<O> o = {(O*)opp_dev, (O*)hand_dev, (O*)talon_dev, (O*)king_dev, (O*)decl_dev, (O*)discard_dev, (O*)mozne_dev, ok_dev};
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_obs_expand<O><<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, net_type, rows, (const int*)sel_dev, n_sel, o, play < 0 ? -1 : play);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_select_action(tarok_t* h, const float* q_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
                         uint8_t* card_dev, float* qmax_dev, void* stream) {
+    return tarok_select_action_ex(h, TAROK_DTYPE_F32, q_dev, sel_dev, n_sel, random_card, card_dev, qmax_dev, stream);
+}
+
+int tarok_select_action_ex(tarok_t* h, int dtype, const void* q_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
+                           uint8_t* card_dev, float* qmax_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!q_dev || !card_dev) return fail(h, -1, "q_dev/card_dev is null");
-    if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
-    if (n_sel == 0) return 0;
-    DeviceGuard dg(h->device);
-    const u64 threshold = explore_threshold(random_card);
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_select_action<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, q_dev, (const int*)sel_dev, n_sel, threshold, card_dev, qmax_dev);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using Q = decltype(tag);
+        if (!q_dev || !card_dev) return fail(h, -1, "q_dev/card_dev is null");
+        if (misaligned(q_dev, sizeof(Q))) return fail(h, -1, "q_dev is not aligned to its element type");
+        if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
+        if (n_sel == 0) return 0;
+        DeviceGuard dg(h->device);
+        const u64 threshold = explore_threshold(random_card);
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_select_action<Q><<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, (const Q*)q_dev, (const int*)sel_dev, n_sel, threshold, card_dev, qmax_dev);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_obs_hands(tarok_t* h, float* out_dev, void* stream) {
+    return tarok_obs_hands_ex(h, TAROK_DTYPE_F32, out_dev, stream);
+}
+
+int tarok_obs_hands_ex(tarok_t* h, int dtype, void* out_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!out_dev) return fail(h, -1, "out_dev is null");
-    DeviceGuard dg(h->device);
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_obs_hands<<<(unsigned)((h->e.n + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(h->e, out_dev);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using O = decltype(tag);
+        if (!out_dev) return fail(h, -1, "out_dev is null");
+        if (misaligned(out_dev, sizeof(O))) return fail(h, -1, "out_dev is not aligned to its element type");
+        DeviceGuard dg(h->device);
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_obs_hands<O><<<(unsigned)((h->e.n + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(h->e, (O*)out_dev);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_obs_exchange(tarok_t* h, const int32_t* sel_dev, uint64_t n_sel, float* hand_dev, float* talon_dev, float* game_dev,
                        uint8_t* ok_dev, void* stream) {
+    return tarok_obs_exchange_ex(h, TAROK_DTYPE_F32, sel_dev, n_sel, hand_dev, talon_dev, game_dev, ok_dev, stream);
+}
+
+int tarok_obs_exchange_ex(tarok_t* h, int dtype, const int32_t* sel_dev, uint64_t n_sel, void* hand_dev, void* talon_dev,
+                          void* game_dev, uint8_t* ok_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!hand_dev || !talon_dev || !game_dev) return fail(h, -1, "hand_dev/talon_dev/game_dev is null");
-    if (n_sel == 0) return 0;
-    DeviceGuard dg(h->device);
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_obs_exchange<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, (const int*)sel_dev, n_sel, hand_dev, talon_dev, game_dev, ok_dev);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using O = decltype(tag);
+        if (!hand_dev || !talon_dev || !game_dev) return fail(h, -1, "hand_dev/talon_dev/game_dev is null");
+        if (misaligned(hand_dev, 2 * sizeof(O)) || misaligned(talon_dev, 2 * sizeof(O)))
+            return fail(h, -1, "hand_dev/talon_dev must be %d-byte aligned", (int)(2 * sizeof(O)));
+        if (misaligned(game_dev, sizeof(O))) return fail(h, -1, "game_dev is not aligned to its element type");
+        if (n_sel == 0) return 0;
+        DeviceGuard dg(h->device);
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_obs_exchange<O><<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, (const int*)sel_dev, n_sel, (O*)hand_dev, (O*)talon_dev, (O*)game_dev, ok_dev);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_select_exchange(tarok_t* h, const float* p_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
                           uint8_t* group_dev, uint64_t* discard_dev, void* stream) {
+    return tarok_select_exchange_ex(h, TAROK_DTYPE_F32, p_dev, sel_dev, n_sel, random_card, group_dev, discard_dev, stream);
+}
+
+int tarok_select_exchange_ex(tarok_t* h, int dtype, const void* p_dev, const int32_t* sel_dev, uint64_t n_sel, float random_card,
+                             uint8_t* group_dev, uint64_t* discard_dev, void* stream) {
     TK_CHECK_HANDLE(h);
-    if (!p_dev || !group_dev || !discard_dev) return fail(h, -1, "p_dev/group_dev/discard_dev is null");
-    if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
-    if (n_sel == 0) return 0;
-    DeviceGuard dg(h->device);
-    const u64 threshold = explore_threshold(random_card);
-    const u64 warps_per_cta = tk::CTA / 32;
-    tk::k_select_exchange<<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
-        h->e, p_dev, (const int*)sel_dev, n_sel, threshold, group_dev, (u64*)discard_dev);
-    TK_LAUNCH_OK(h);
-    return 0;
+    return with_dtype(h, dtype, [&](auto tag) -> int {
+        using Q = decltype(tag);
+        if (!p_dev || !group_dev || !discard_dev) return fail(h, -1, "p_dev/group_dev/discard_dev is null");
+        if (misaligned(p_dev, sizeof(Q))) return fail(h, -1, "p_dev is not aligned to its element type");
+        if (!(random_card >= 0.f && random_card <= 1.f)) return fail(h, -1, "random_card must be in [0,1]");
+        if (n_sel == 0) return 0;
+        DeviceGuard dg(h->device);
+        const u64 threshold = explore_threshold(random_card);
+        const u64 warps_per_cta = tk::CTA / 32;
+        tk::k_select_exchange<Q><<<(unsigned)((n_sel + warps_per_cta - 1) / warps_per_cta), tk::CTA, 0, S(stream)>>>(
+            h->e, (const Q*)p_dev, (const int*)sel_dev, n_sel, threshold, group_dev, (u64*)discard_dev);
+        TK_LAUNCH_OK(h);
+        return 0;
+    });
 }
 
 int tarok_targets(tarok_t* h, const int32_t* sel_dev, uint64_t n_sel, float final_reword_factor, float* dy_dev,

@@ -15,7 +15,15 @@
 //  * talon_input: Navadna/Solo [6,55] row j = j-th talon card one-hot, column 54 = "in the chosen group"
 //    (only once the exchange is in the history; Solo_brez never has one); Klop [54] multi-hot of the talon cards
 //    revealed so far; Berac none.  zalozil[54] = own discards, only for the seat that exchanged.
+//
+// Element types: the observation kernels are templates over the OUTPUT type O (float, __nv_bfloat16, __half) and the
+// selection kernels over the INPUT type Q of the network outputs.  Every observation value is exactly 0 or 1, so all three
+// hold it exactly; network outputs are widened to fp32 (exact) before any comparison, so a selection on bf16 / fp16
+// outputs is the fp32 selection of the widened values.  qmax / next_Q_max and the replay targets stay fp32.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "tarok_kernels.cuh"
 
 namespace tk {
@@ -129,35 +137,60 @@ __global__ void __launch_bounds__(CTA) k_bucket_scatter(Env e, u32 players, cons
     if (selkey) selkey[at] = (uint8_t)key;
 }
 
-struct ObsOut {
-    float* opp;      // [n_sel, T, 3, 54]
-    float* hand;     // [n_sel, T, 54]
-    float* talon;    // [n_sel, 6, 55] (Navadna, Solo) | [n_sel, 54] (Klop) | unused (Berac)
-    float* king;     // [n_sel, 4]      (Navadna)
-    float* decl;     // [n_sel, 4]      (Navadna, Solo, Berac)
-    float* discard;  // [n_sel, 54]     (Navadna, Solo)
-    float* mozne;    // [n_sel, 54]
+template <class O> struct ObsOut {
+    O* opp;          // [n_sel, T, 3, 54]
+    O* hand;         // [n_sel, T, 54]
+    O* talon;        // [n_sel, 6, 55] (Navadna, Solo) | [n_sel, 54] (Klop) | unused (Berac)
+    O* king;         // [n_sel, 4]      (Navadna)
+    O* decl;         // [n_sel, 4]      (Navadna, Solo, Berac)
+    O* discard;      // [n_sel, 54]     (Navadna, Solo)
+    O* mozne;        // [n_sel, 54]
     uint8_t* ok;     // [n_sel] 1 = game matched (net_type, T) and was expanded
 };
 
-__device__ __forceinline__ void warp_zero(float* p, u32 count, u32 lane) {       // count % 2 == 0, p 8-byte aligned
-    float2* q = reinterpret_cast<float2*>(p);
-    for (u32 i = lane; i < count / 2; i += 32) q[i] = make_float2(0.f, 0.f);
+// 0 or 1 as an observation element (b is 0 or 1): 1.0 is 0x3F80 in bf16 and 0x3C00 in fp16.
+template <class O> __device__ __forceinline__ O obs_bit(u64 b);
+template <> __device__ __forceinline__ float obs_bit<float>(u64 b) { return (float)b; }
+template <> __device__ __forceinline__ __nv_bfloat16 obs_bit<__nv_bfloat16>(u64 b) { return __ushort_as_bfloat16((unsigned short)(b * 0x3F80u)); }
+template <> __device__ __forceinline__ __half obs_bit<__half>(u64 b) { return __ushort_as_half((unsigned short)(b * 0x3C00u)); }
+
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+
+// Zero fill in element pairs: 8-byte stores for fp32, 4-byte stores for the half types.  count % 2 == 0, p aligned to a pair.
+template <class O> __device__ __forceinline__ void warp_zero(O* p, u32 count, u32 lane) {
+    if constexpr (sizeof(O) == 4) {
+        float2* q = reinterpret_cast<float2*>(p);
+        for (u32 i = lane; i < count / 2; i += 32) q[i] = make_float2(0.f, 0.f);
+    } else {
+        u32* q = reinterpret_cast<u32*>(p);
+        for (u32 i = lane; i < count / 2; i += 32) q[i] = 0u;
+    }
 }
-__device__ __forceinline__ void warp_zero4(float* p, u32 count, u32 lane) {      // count % 4 == 0, p 16-byte aligned
-    float4* q = reinterpret_cast<float4*>(p);
-    for (u32 i = lane; i < count / 4; i += 32) q[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+// Zero fill in 16-byte stores: count * sizeof(O) % 16 == 0, p 16-byte aligned.
+template <class O> __device__ __forceinline__ void warp_zero4(O* p, u32 count, u32 lane) {
+    if constexpr (sizeof(O) == 4) {
+        float4* q = reinterpret_cast<float4*>(p);
+        for (u32 i = lane; i < count / 4; i += 32) q[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    } else {
+        uint4* q = reinterpret_cast<uint4*>(p);
+        for (u32 i = lane; i < count / 8; i += 32) q[i] = make_uint4(0u, 0u, 0u, 0u);
+    }
 }
-__device__ __forceinline__ void warp_bits(float* p, u64 bits, u32 lane) {         // 54 floats from a bitboard
-    p[lane] = (float)((bits >> lane) & 1ull);
-    if (lane + 32 < 54) p[lane + 32] = (float)((bits >> (lane + 32)) & 1ull);
+template <class O> __device__ __forceinline__ void warp_bits(O* p, u64 bits, u32 lane) {     // 54 elements from a bitboard
+    p[lane] = obs_bit<O>((bits >> lane) & 1ull);
+    if (lane + 32 < 54) p[lane + 32] = obs_bit<O>((bits >> (lane + 32)) & 1ull);
 }
 
 // `upto` < 0: the observation of the seat to move NOW.  `upto` = t >= 0: the observation the seat that made play t
 // had at that decision (history truncated to the first t plays) -- the `stanje` of a replay sample; the legal-mask
 // vector is not produced in that mode (it is not a network input, Igralec.py:333).
-// One warp expands one game; `o` points at THIS game's blocks (null = not wanted).
-__device__ __forceinline__ void obs_expand_game(const Env& e, u64 g, int net_type, u32 T, const ObsOut& o, int upto, u32 lane) {
+// One warp expands one game; `o` points at THIS game's blocks (null = not wanted).  Half outputs: opp / hand (T * 324 and
+// T * 108 bytes, 16-byte multiples as T % 8 == 0) are zeroed in 16-byte stores, talon / discard / mozne / king / decl in
+// 4-byte stores (their blocks are even element counts at 4-byte aligned starts).
+template <class O>
+__device__ __forceinline__ void obs_expand_game(const Env& e, u64 g, int net_type, u32 T, const ObsOut<O>& o, int upto, u32 lane) {
     const u64 na = e.n_alloc;
     const bool in_range = g < e.n;
     u64 meta = in_range ? e.meta[g] : meta_pad();
@@ -173,13 +206,18 @@ __device__ __forceinline__ void obs_expand_game(const Env& e, u64 g, int net_typ
     const u32 plays = mget(meta, M_PLAYS, 6);
     const bool match = mget(meta, M_PHASE, 2) == PH_PLAY && net_type_of(contract) == (u32)net_type
                     && padded_rows(history_len(meta)) == T;
-    float* opp = o.opp;
-    float* hand = o.hand;
+    O* opp = o.opp;
+    O* hand = o.hand;
     warp_zero4(opp, T * 162u, lane);                                 // T % 8 == 0: both blocks are 16-byte multiples
     warp_zero4(hand, T * 54u, lane);
     if (o.talon && net_type != NET_BERAC) warp_zero(o.talon, net_type == NET_KLOP ? 54u : 330u, lane);
-    if (o.king && lane < 4) o.king[lane] = 0.f;
-    if (o.decl && lane < 4) o.decl[lane] = 0.f;
+    if constexpr (sizeof(O) == 4) {
+        if (o.king && lane < 4) o.king[lane] = 0.f;
+        if (o.decl && lane < 4) o.decl[lane] = 0.f;
+    } else {
+        if (o.king) warp_zero(o.king, 4u, lane);
+        if (o.decl) warp_zero(o.decl, 4u, lane);
+    }
     if (o.discard) warp_zero(o.discard, 54u, lane);
     if (o.mozne) warp_zero(o.mozne, 54u, lane);
     if (o.ok && lane == 0) *o.ok = match ? 1 : 0;
@@ -194,8 +232,8 @@ __device__ __forceinline__ void obs_expand_game(const Env& e, u64 g, int net_typ
     if (lane + 32 < plays) h1 = e.hist[(u64)(lane + 32) * na + g];
     const bool own0 = h0 != 0xFF && (h0 >> 6) == self, own1 = h1 != 0xFF && (h1 >> 6) == self;
     // opponents' plays: one 1.0 each
-    if (h0 != 0xFF && !own0) { u32 s = h0 >> 6; opp[(u64)lane * 162u + (s < self ? s : s - 1) * 54u + (h0 & 63u)] = 1.f; }
-    if (h1 != 0xFF && !own1) { u32 s = h1 >> 6; opp[(u64)(lane + 32) * 162u + (s < self ? s : s - 1) * 54u + (h1 & 63u)] = 1.f; }
+    if (h0 != 0xFF && !own0) { u32 s = h0 >> 6; opp[(u64)lane * 162u + (s < self ? s : s - 1) * 54u + (h0 & 63u)] = obs_bit<O>(1); }
+    if (h1 != 0xFF && !own1) { u32 s = h1 >> 6; opp[(u64)(lane + 32) * 162u + (s < self ? s : s - 1) * 54u + (h1 & 63u)] = obs_bit<O>(1); }
     // own plays: exclusive prefix-OR of the own cards played before each row (warp scan over 64 slots)
     u64 b0 = own0 ? 1ull << (h0 & 63u) : 0ull, b1 = own1 ? 1ull << (h1 & 63u) : 0ull;
     u64 inc0 = b0, inc1 = b1;
@@ -220,29 +258,30 @@ __device__ __forceinline__ void obs_expand_game(const Env& e, u64 g, int net_typ
     const u64 order = e.torder[g];
     if (o.talon && net_type == NET_KLOP) {
         const u32 shown = min(mget(meta, M_TRICKS, 4), 6u);           // Klop.py:69 pops from the end
-        if (lane < shown) o.talon[(order >> (6 * (5 - lane))) & 63ull] = 1.f;
+        if (lane < shown) o.talon[(order >> (6 * (5 - lane))) & 63ull] = obs_bit<O>(1);
     } else if (o.talon && (net_type == NET_NAVADNA || net_type == NET_SOLO)) {
         const u32 grp = mget(meta, M_GROUP, 3), k = talon_k(contract);
         if (grp != NO_GROUP && lane < 6) {
-            float* row = o.talon + lane * 55u;
-            row[(order >> (6 * lane)) & 63ull] = 1.f;
-            if (lane / k == grp) row[54] = 1.f;
+            O* row = o.talon + lane * 55u;
+            row[(order >> (6 * lane)) & 63ull] = obs_bit<O>(1);
+            if (lane / k == grp) row[54] = obs_bit<O>(1);
         }
     }
-    if (o.king && lane == 0) { u32 kg = mget(meta, M_KING, 3); if (kg < 4) o.king[kg] = 1.f; }
-    if (o.decl && lane == 0) o.decl[decl == self ? 3u : (decl < self ? decl : decl - 1)] = 1.f;
+    if (o.king && lane == 0) { u32 kg = mget(meta, M_KING, 3); if (kg < 4) o.king[kg] = obs_bit<O>(1); }
+    if (o.decl && lane == 0) o.decl[decl == self ? 3u : (decl < self ? decl : decl - 1)] = obs_bit<O>(1);
     if (o.discard && self == decl && mget(meta, M_GROUP, 3) != NO_GROUP) warp_bits(o.discard, e.discard[g], lane);
     if (o.mozne && upto < 0) warp_bits(o.mozne, e.mask[g], lane);
 }
 
 // One (net type, T) bucket: `o` holds the bases of the bucket's arrays, game i of the selection gets block i.
+template <class O>
 __global__ void __launch_bounds__(CTA) k_obs_expand(Env e, int net_type, u32 T, const int* __restrict__ sel, u64 n_sel,
-                                                    ObsOut o, int upto) {
+                                                    ObsOut<O> o, int upto) {
     const u32 lane = threadIdx.x & 31u;
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;        // one warp per selected game
     if (i >= n_sel) return;
     const u64 g = sel ? (u64)sel[i] : i;
-    ObsOut m;
+    ObsOut<O> m;
     m.opp = o.opp + i * (u64)T * 162u;
     m.hand = o.hand + i * (u64)T * 54u;
     m.talon = o.talon ? o.talon + i * (net_type == NET_KLOP ? 54u : 330u) : nullptr;
@@ -257,17 +296,18 @@ __global__ void __launch_bounds__(CTA) k_obs_expand(Env e, int net_type, u32 T, 
 // EVERY bucket of a step in one launch (after tarok_obs_buckets): position i of `sel` belongs to bucket selkey[i] =
 // player * 28 + net * 7 + (T / 8 - 1); its rows go to the bucket's block of the arenas -- opp / hand at row counts[256 + key]
 // + (i - counts[128 + key]) * T, the per-game vectors at index i -- so that each bucket's inputs are contiguous tensors.
-struct ObsArena { float* opp; float* hand; float* talon; float* talon_klop; float* king; float* decl; float* discard; };
+template <class O> struct ObsArena { O* opp; O* hand; O* talon; O* talon_klop; O* king; O* decl; O* discard; };
 
+template <class O>
 __global__ void __launch_bounds__(CTA) k_obs_expand_all(Env e, const int* __restrict__ sel, const uint8_t* __restrict__ selkey,
-                                                        const u32* __restrict__ counts, u64 n_total, ObsArena a) {
+                                                        const u32* __restrict__ counts, u64 n_total, ObsArena<O> a) {
     const u32 lane = threadIdx.x & 31u;
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
     if (i >= n_total) return;
     const u32 key = selkey[i];
     const u32 net = (key % 28u) / 7u, T = 8u * (key % 7u + 1u);
     const u64 row = (u64)counts[2 * BUCKETS + key] + (i - counts[BUCKETS + key]) * T;
-    ObsOut m;
+    ObsOut<O> m;
     m.opp = a.opp + row * 162u;
     m.hand = a.hand + row * 54u;
     m.talon = net == NET_KLOP ? a.talon_klop + i * 54u : net == NET_BERAC ? nullptr : a.talon + i * 330u;
@@ -298,7 +338,8 @@ __device__ __forceinline__ bool ranks_above(float a, float b) { return a > b || 
 // 2^32 = always), so random_card = 1 explores at every word, 0xFFFFFFFF included.
 __device__ __forceinline__ bool explores(u32 w, u64 explore_threshold) { return (u64)w < explore_threshold; }
 
-__device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __restrict__ qrow, u64 explore_threshold,
+template <class Q>
+__device__ __forceinline__ void select_game(const Env& e, u64 g, const Q* __restrict__ qrow, u64 explore_threshold,
                                             uint8_t* __restrict__ card_out, float* __restrict__ qmax_out, u32 lane) {
     const u64 na = e.n_alloc;
     const u64 meta = e.meta[g];
@@ -328,7 +369,7 @@ __device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __
                 for (u32 j = 0; j < 6; j++) if (((order >> (6 * j)) & 63ull) == c) tp = j;
                 key = 64u + tp;
             }
-            const float v = qrow[c];
+            const float v = to_f32(qrow[c]);
             if (ranks_above(v, best) || (!ranks_above(best, v) && key < best_key)) { best = v; best_key = key; best_card = c; }
         }
     }
@@ -352,7 +393,8 @@ __device__ __forceinline__ void select_game(const Env& e, u64 g, const float* __
     }
 }
 
-__global__ void __launch_bounds__(CTA) k_select_action(Env e, const float* __restrict__ q, const int* __restrict__ sel,
+template <class Q>
+__global__ void __launch_bounds__(CTA) k_select_action(Env e, const Q* __restrict__ q, const int* __restrict__ sel,
                                                        u64 n_sel, u64 explore_threshold, uint8_t* __restrict__ card_out,
                                                        float* __restrict__ qmax_out) {
     const u32 lane = threadIdx.x & 31u;
@@ -367,8 +409,10 @@ __global__ void __launch_bounds__(CTA) k_select_action(Env e, const float* __res
 // forward pass (a table of device pointers the host fills), thr4[player] = the player's epsilon as a 32-bit threshold.
 struct Thresholds4 { u64 t[4]; };
 // The same with the table of bucket outputs passed BY VALUE (1 KB of kernel parameters): no device table to fill and copy.
-struct QTable { const float* p[BUCKETS]; };
-__global__ void __launch_bounds__(CTA) k_select_action_all_tab(Env e, QTable qt, const int* __restrict__ sel,
+// One element type for the whole table.
+template <class Q> struct QTable { const Q* p[BUCKETS]; };
+template <class Q>
+__global__ void __launch_bounds__(CTA) k_select_action_all_tab(Env e, QTable<Q> qt, const int* __restrict__ sel,
                                                                const uint8_t* __restrict__ selkey, const u32* __restrict__ counts,
                                                                u64 n_total, Thresholds4 thr4, uint8_t* __restrict__ card_out,
                                                                float* __restrict__ qmax_out) {
@@ -376,7 +420,7 @@ __global__ void __launch_bounds__(CTA) k_select_action_all_tab(Env e, QTable qt,
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
     if (i >= n_total) return;
     const u32 key = selkey[i];
-    const float* q = qt.p[key & (BUCKETS - 1)];
+    const Q* q = qt.p[key & (BUCKETS - 1)];
     if (!q) return;                                               // no forward was supplied for this bucket
     const u32 p = key / 28u;
     const u64 thr = p == 0 ? thr4.t[0] : p == 1 ? thr4.t[1] : p == 2 ? thr4.t[2] : thr4.t[3];
@@ -410,7 +454,8 @@ __global__ void __launch_bounds__(CTA) k_select_action_all(Env e, const float* c
 //     cards in talon order), i.e. what a stable sort gives.  Each of the two choices is replaced by a uniform one
 //     with probability random_card.
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(CTA) k_obs_hands(Env e, float* __restrict__ out) {
+template <class O>
+__global__ void __launch_bounds__(CTA) k_obs_hands(Env e, O* __restrict__ out) {
     const u32 lane = threadIdx.x & 31u;
     const u64 g = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
     if (g >= e.n) return;
@@ -420,8 +465,11 @@ __global__ void __launch_bounds__(CTA) k_obs_hands(Env e, float* __restrict__ ou
     for (int s = 0; s < 4; s++) warp_bits(out + (g * 4 + s) * 54u, e.hands[slot_of((u32)s, leader) * na + g], lane);
 }
 
-__global__ void __launch_bounds__(CTA) k_obs_exchange(Env e, const int* __restrict__ sel, u64 n_sel, float* __restrict__ hand,
-                                                      float* __restrict__ talon, float* __restrict__ game, uint8_t* __restrict__ ok) {
+// Half outputs: hand [54] and talon [324] in 4-byte stores, the game one-hot [15] (30 bytes, so game i starts 2-byte aligned
+// only) in 2-byte stores.
+template <class O>
+__global__ void __launch_bounds__(CTA) k_obs_exchange(Env e, const int* __restrict__ sel, u64 n_sel, O* __restrict__ hand,
+                                                      O* __restrict__ talon, O* __restrict__ game, uint8_t* __restrict__ ok) {
     const u32 lane = threadIdx.x & 31u;
     const u64 i = ((u64)blockIdx.x * CTA + threadIdx.x) >> 5;
     if (i >= n_sel) return;
@@ -431,7 +479,7 @@ __global__ void __launch_bounds__(CTA) k_obs_exchange(Env e, const int* __restri
     const bool match = mget(meta, M_PHASE, 2) == PH_EXCHANGE;
     warp_zero(hand + i * 54u, 54u, lane);
     warp_zero(talon + i * 324u, 324u, lane);
-    if (lane < 15) game[i * 15u + lane] = 0.f;
+    if (lane < 15) game[i * 15u + lane] = obs_bit<O>(0);
     if (ok && lane == 0) ok[i] = match ? 1 : 0;
     __syncwarp();
     if (!match) return;
@@ -439,11 +487,12 @@ __global__ void __launch_bounds__(CTA) k_obs_exchange(Env e, const int* __restri
     const u32 k = talon_k(contract);
     warp_bits(hand + i * 54u, e.hands[slot_of(decl, leader_of(meta)) * na + g], lane);
     const u64 order = e.torder[g];
-    if (lane < 6) talon[i * 324u + ((order >> (6 * lane)) & 63ull) * 6u + lane / k] = 1.f;
-    if (lane == 0) game[i * 15u + (is_king_game(contract) ? (contract - C_TRI) * 4u + king : 12u + (contract - C_SOLO_TRI))] = 1.f;
+    if (lane < 6) talon[i * 324u + ((order >> (6 * lane)) & 63ull) * 6u + lane / k] = obs_bit<O>(1);
+    if (lane == 0) game[i * 15u + (is_king_game(contract) ? (contract - C_TRI) * 4u + king : 12u + (contract - C_SOLO_TRI))] = obs_bit<O>(1);
 }
 
-__global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __restrict__ p, const int* __restrict__ sel, u64 n_sel,
+template <class Q>
+__global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const Q* __restrict__ p, const int* __restrict__ sel, u64 n_sel,
                                                          u64 explore_threshold, uint8_t* __restrict__ group_out,
                                                          u64* __restrict__ discard_out) {
     const u32 lane = threadIdx.x & 31u;
@@ -460,7 +509,7 @@ __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __r
     const unsigned full = 0xFFFFFFFFu;
     // group: first argmax of p[54 .. 54+groups)
     // (NaN first, the first maximum); the inactive lanes hold (-inf, 0xFF), which every real group beats
-    float bv = lane < groups ? p[i * 60u + 54u + lane] : -INFINITY;
+    float bv = lane < groups ? to_f32(p[i * 60u + 54u + lane]) : -INFINITY;
     u32 bi = lane < groups ? lane : 0xFFu;
 #pragma unroll
     for (int d = 16; d >= 1; d >>= 1) {
@@ -499,7 +548,7 @@ __global__ void __launch_bounds__(CTA) k_select_exchange(Env e, const float* __r
                         pos = 64u + tp;
                     }
                     const u32 kk = (((c >= 32 ? 4u : (c >> 3)) << 8) | pos) + 1u;
-                    const float pv = p[i * 60u + c];
+                    const float pv = to_f32(p[i * 60u + c]);
                     if (ranks_above(pv, v) || (!ranks_above(v, pv) && kk > key)) { v = pv; key = kk; card = c; }
                 }
             }

@@ -30,6 +30,22 @@ FLAG_HISTORY = 1
 (F_HANDS, F_PILES, F_TALON, F_TALON_ORDER, F_META, F_MASK, F_SCORES, F_HIST, F_STATS, F_HANDS0,
  F_DISCARD, F_QMAX_HIST) = range(12)
 
+# element types of the observation outputs and of the network outputs the selections read (TAROK_DTYPE_*)
+DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
+
+
+def dtype_code(dtype) -> int:
+    """TAROK_DTYPE_* of a torch dtype; ValueError for anything but fp32 / bf16 / fp16."""
+    if dtype not in DTYPES:
+        raise ValueError("observations and network outputs must be float32, bfloat16 or float16, not %s" % (dtype,))
+    return DTYPES[dtype]
+
+
+def _net_out(q, dev):
+    """Network outputs as the selections read them: fp32 / bf16 / fp16 pass through, any other dtype is cast to fp32."""
+    return q.to(device=dev, dtype=q.dtype if q.dtype in DTYPES else torch.float32).contiguous()
+
+
 # stats vector layout (include/tarok_b200.h)
 S_SEAT, S_PLAYER, S_CONTRACT, S_FINISHED, S_STEPS, S_ERRORS, S_ERR_EVENTS = 0, 4, 8, 18, 19, 20, 21
 
@@ -355,28 +371,40 @@ class TarokEnv:
         return sel, host.numpy().view(np.uint32)
 
     def obs_expand_buckets(self, n_total: int, opp, hand, talon, talon_klop, king, decl, discard):
-        """ONE launch for every bucket of the last ``obs_buckets``: the arenas (flat fp32 CUDA tensors, capacities n * 56
-        rows / n entries) receive each bucket's inputs as contiguous blocks (layout in include/tarok_b200.h)."""
+        """ONE launch for every bucket of the last ``obs_buckets``: the arenas (flat CUDA tensors of one dtype -- fp32, bf16 or
+        fp16 -- capacities n * 56 rows / n entries) receive each bucket's inputs as contiguous blocks (layout in
+        include/tarok_b200.h)."""
+        arenas = (opp, hand, talon, talon_klop, king, decl, discard)
+        dtypes = {t.dtype for t in arenas}
+        if len(dtypes) != 1:
+            raise ValueError("the observation arenas mix dtypes: %s" % sorted(str(d) for d in dtypes))
+        code = dtype_code(dtypes.pop())
         sel, cnt, _, selkey = self._bk[:4]
         p = lambda t: C.c_void_p(t.data_ptr())
-        self._check(self._lib.tarok_obs_expand_buckets(self._h, p(sel), p(selkey), p(cnt), int(n_total), p(opp), p(hand), p(talon),
-                                                       p(talon_klop), p(king), p(decl), p(discard), self._stream()))
+        self._check(self._lib.tarok_obs_expand_buckets_ex(self._h, code, p(sel), p(selkey), p(cnt), int(n_total),
+                                                          *[p(t) for t in arenas], self._stream()))
 
     def select_action_buckets(self, n_total: int, q_by_key: dict, random_card4, cards, qmax=None):
-        """ONE launch of ``select_action`` for every bucket: ``q_by_key[key]`` = that bucket's [size, 54] fp32 network output
-        (contiguous CUDA tensors, kept alive by the caller until the stream has run the launch)."""
+        """ONE launch of ``select_action`` for every bucket: ``q_by_key[key]`` = that bucket's [size, 54] network output
+        (contiguous CUDA tensors, kept alive by the caller until the stream has run the launch).  fp32, bf16 and fp16 outputs
+        are read as they are (one dtype for the whole table); other dtypes are cast to fp32."""
+        dtypes = {q.dtype for q in q_by_key.values()}
+        if len(dtypes) > 1:
+            raise ValueError("the bucket outputs mix dtypes: %s" % sorted(str(d) for d in dtypes))
+        q_by_key = {k: _net_out(q, self.torch_device) for k, q in q_by_key.items()}
+        code = DTYPES[next(iter(q_by_key.values())).dtype] if q_by_key else 0
         sel, cnt, _, selkey = self._bk[:4]
         tab = (C.c_void_p * 128)()                                   # travels as kernel parameters
         for k, q in q_by_key.items():
             tab[k] = q.data_ptr()
         eps = (C.c_float * 4)(*[float(x) for x in random_card4])
         p = lambda t: C.c_void_p(t.data_ptr())
-        self._check(self._lib.tarok_select_action_buckets_tab(self._h, tab, p(sel), p(selkey), p(cnt), int(n_total), eps, p(cards),
-                                                              p(qmax) if qmax is not None else None, self._stream()))
+        self._check(self._lib.tarok_select_action_buckets_tab_ex(self._h, code, tab, p(sel), p(selkey), p(cnt), int(n_total), eps,
+                                                                 p(cards), p(qmax) if qmax is not None else None, self._stream()))
 
-    def obs_expand(self, net_type: int, rows: int, sel=None, play=None):
+    def obs_expand(self, net_type: int, rows: int, sel=None, play=None, dtype=torch.float32):
         """The network inputs of ``Nevronski_igralec.stanje_v_vektor_rek_navadna`` for the seat to move of the
-        selected games (int32 indices; None = all), as fp32 tensors in the reference's list order
+        selected games (int32 indices; None = all), as ``dtype`` tensors (fp32, bf16 or fp16) in the reference's list order
         (A.4): Navadna [opp, king, hand, talon, decl, discard, mozne]; Solo [opp, hand, talon, decl, discard, mozne];
         Klop [opp, hand, talon, mozne]; Berac [opp, hand, decl, mozne].  Returns (list of tensors, ok uint8 [n_sel]).
         ``play=t`` gives the observation as it was at card play t, for the seat that made it (replay samples)."""
@@ -387,7 +415,8 @@ class TarokEnv:
         else:
             sel = torch.as_tensor(sel, dtype=torch.int32, device=self.torch_device).contiguous()
             n_sel, sel_ptr = int(sel.numel()), C.c_void_p(sel.data_ptr())
-        dev, f = self.torch_device, torch.float32
+        code = dtype_code(dtype)
+        dev, f = self.torch_device, dtype
         opp = torch.empty((n_sel, rows, 3, 54), dtype=f, device=dev)
         hand = torch.empty((n_sel, rows, 54), dtype=f, device=dev)
         talon = torch.empty((n_sel, 54) if net_type == 0 else (n_sel, 6, 55), dtype=f, device=dev) if net_type != 3 else None
@@ -397,18 +426,19 @@ class TarokEnv:
         mozne = torch.empty((n_sel, 54), dtype=f, device=dev)
         ok = torch.empty(n_sel, dtype=torch.uint8, device=dev)
         p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-        self._check(self._lib.tarok_obs_expand_at(self._h, -1 if play is None else int(play), int(net_type), int(rows), sel_ptr,
-                                                  n_sel, p(opp), p(hand), p(talon), p(king), p(decl), p(disc), p(mozne), p(ok),
-                                                  self._stream()))
+        self._check(self._lib.tarok_obs_expand_at_ex(self._h, code, -1 if play is None else int(play), int(net_type), int(rows),
+                                                     sel_ptr, n_sel, p(opp), p(hand), p(talon), p(king), p(decl), p(disc), p(mozne),
+                                                     p(ok), self._stream()))
         order = {1: [opp, king, hand, talon, decl, disc, mozne], 2: [opp, hand, talon, decl, disc, mozne],
                  0: [opp, hand, talon, mozne], 3: [opp, hand, decl, mozne]}[int(net_type)]
         return order, ok
 
     def select_action(self, q, sel=None, random_card: float = 0.0, cards=None, qmax=None):
-        """``Nevronski_igralec.igraj_karto`` (Igralec.py:344-355) for the selected games: first argmax of ``q`` (fp32
-        [n_sel,54]) over the legal cards in the reference's ``mozne`` order, epsilon-greedy with ``random_card``.
-        Writes into ``cards`` (uint8 [n], by game index; allocated if None) and returns (cards, qmax)."""
-        q = q.to(device=self.torch_device, dtype=torch.float32).contiguous()
+        """``Nevronski_igralec.igraj_karto`` (Igralec.py:344-355) for the selected games: first argmax of ``q`` ([n_sel,54];
+        fp32, bf16 and fp16 are read as they are, other dtypes cast to fp32) over the legal cards in the reference's ``mozne``
+        order, epsilon-greedy with ``random_card``.  Writes into ``cards`` (uint8 [n], by game index; allocated if None) and
+        returns (cards, qmax fp32)."""
+        q = _net_out(q, self.torch_device)
         if sel is None:
             n_sel, sel_ptr = self.n, None
         else:
@@ -420,8 +450,9 @@ class TarokEnv:
             cards = torch.full((self.n_alloc,), 0xFF, dtype=torch.uint8, device=self.torch_device)
         if qmax is None:
             qmax = torch.zeros(self.n, dtype=torch.float32, device=self.torch_device)
-        self._check(self._lib.tarok_select_action(self._h, C.c_void_p(q.data_ptr()), sel_ptr, n_sel, float(random_card),
-                                                  C.c_void_p(cards.data_ptr()), C.c_void_p(qmax.data_ptr()), self._stream()))
+        self._check(self._lib.tarok_select_action_ex(self._h, DTYPES[q.dtype], C.c_void_p(q.data_ptr()), sel_ptr, n_sel,
+                                                     float(random_card), C.c_void_p(cards.data_ptr()), C.c_void_p(qmax.data_ptr()),
+                                                     self._stream()))
         return cards, qmax
 
     def targets(self, sel=None, final_reword_factor: float = 0.1):
@@ -437,10 +468,11 @@ class TarokEnv:
                                             C.c_void_p(seat.data_ptr()), C.c_void_p(rows.data_ptr()), self._stream()))
         return dy, seat, rows
 
-    def obs_hands(self) -> torch.Tensor:
-        """``pripavi_licitiram`` (Igralec.py:278-281): fp32 [n,4,54], the hand of every seat."""
-        out = torch.empty((self.n, 4, 54), dtype=torch.float32, device=self.torch_device)
-        self._check(self._lib.tarok_obs_hands(self._h, C.c_void_p(out.data_ptr()), self._stream()))
+    def obs_hands(self, dtype=torch.float32) -> torch.Tensor:
+        """``pripavi_licitiram`` (Igralec.py:278-281): [n,4,54] in ``dtype`` (fp32, bf16 or fp16), the hand of every seat."""
+        code = dtype_code(dtype)
+        out = torch.empty((self.n, 4, 54), dtype=dtype, device=self.torch_device)
+        self._check(self._lib.tarok_obs_hands_ex(self._h, code, C.c_void_p(out.data_ptr()), self._stream()))
         return out
 
     def _sel(self, sel):
@@ -449,29 +481,33 @@ class TarokEnv:
         sel = torch.as_tensor(sel, dtype=torch.int32, device=self.torch_device).contiguous()
         return int(sel.numel()), C.c_void_p(sel.data_ptr()), sel
 
-    def obs_exchange(self, sel=None):
-        """``menjaj_talon_v_vektor`` (Igralec.py:535-543): ([hand (B,54), talon (B,54,6), game (B,15)], ok)."""
+    def obs_exchange(self, sel=None, dtype=torch.float32):
+        """``menjaj_talon_v_vektor`` (Igralec.py:535-543): ([hand (B,54), talon (B,54,6), game (B,15)] in ``dtype``, ok)."""
+        code = dtype_code(dtype)
         n_sel, sel_ptr, keep = self._sel(sel)
-        dev, f = self.torch_device, torch.float32
+        dev, f = self.torch_device, dtype
         hand = torch.empty((n_sel, 54), dtype=f, device=dev)
         talon = torch.empty((n_sel, 54, 6), dtype=f, device=dev)
         game = torch.empty((n_sel, 15), dtype=f, device=dev)
         ok = torch.empty(n_sel, dtype=torch.uint8, device=dev)
-        self._check(self._lib.tarok_obs_exchange(self._h, sel_ptr, n_sel, C.c_void_p(hand.data_ptr()), C.c_void_p(talon.data_ptr()),
-                                                 C.c_void_p(game.data_ptr()), C.c_void_p(ok.data_ptr()), self._stream()))
+        self._check(self._lib.tarok_obs_exchange_ex(self._h, code, sel_ptr, n_sel, C.c_void_p(hand.data_ptr()),
+                                                    C.c_void_p(talon.data_ptr()), C.c_void_p(game.data_ptr()), C.c_void_p(ok.data_ptr()),
+                                                    self._stream()))
         return [hand, talon, game], ok
 
     def select_exchange(self, p, sel=None, random_card: float = 0.0, group_out=None, discard_out=None):
-        """``menjaj_iz_talona`` (Igralec.py:365-385) from the exchange net's 60 outputs: (group uint8 [n], discard int64 [n]);
-        ``group_out`` / ``discard_out`` let several calls (one per player) fill the same arrays."""
+        """``menjaj_iz_talona`` (Igralec.py:365-385) from the exchange net's 60 outputs (fp32, bf16 and fp16 read as they are,
+        other dtypes cast to fp32): (group uint8 [n], discard int64 [n]); ``group_out`` / ``discard_out`` let several calls
+        (one per player) fill the same arrays."""
         n_sel, sel_ptr, keep = self._sel(sel)
-        p = p.to(device=self.torch_device, dtype=torch.float32).contiguous()
+        p = _net_out(p, self.torch_device)
         if tuple(p.shape) != (n_sel, 60):
             raise ValueError("p must have shape (n_sel, 60)")
         group = group_out if group_out is not None else torch.full((self.n,), 0xFF, dtype=torch.uint8, device=self.torch_device)
         discard = discard_out if discard_out is not None else torch.zeros(self.n, dtype=torch.int64, device=self.torch_device)
-        self._check(self._lib.tarok_select_exchange(self._h, C.c_void_p(p.data_ptr()), sel_ptr, n_sel, float(random_card),
-                                                    C.c_void_p(group.data_ptr()), C.c_void_p(discard.data_ptr()), self._stream()))
+        self._check(self._lib.tarok_select_exchange_ex(self._h, DTYPES[p.dtype], C.c_void_p(p.data_ptr()), sel_ptr, n_sel,
+                                                       float(random_card), C.c_void_p(group.data_ptr()), C.c_void_p(discard.data_ptr()),
+                                                       self._stream()))
         return group, discard
 
     # ------------------------------------------------------------------ helpers

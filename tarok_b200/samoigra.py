@@ -19,9 +19,14 @@ once per step -- the only synchronisation of a step -- and walks the non-empty r
 The environment, the bucketing, the observation expansion and the action selection are the CUDA kernels of this
 repository; the forward passes stay in the reference's networks (here the PyTorch restatement in ``tarok_b200.mreze``,
 because the upstream ``torch_models.py`` is missing).
+
+Mixed precision: ``Samoigra(..., dtype=torch.bfloat16)`` (or ``torch.float16``) plays with observations written in that
+dtype (every value is 0 or 1, so they are exact) and with inference copies of the nets cast to it; the selections read the
+half outputs as they come.  The fp32 master nets, ``nauci`` and ``vzorci`` stay fp32.
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 import os
 from typing import Dict, List, Optional, Sequence, Union
@@ -69,8 +74,7 @@ class _Arena:
     every bucket of every step (the launches of one stream are ordered, so a bucket's forward has consumed its inputs before
     the next expansion overwrites them)."""
 
-    def __init__(self, n, dev):
-        f = torch.float32
+    def __init__(self, n, dev, f=torch.float32):
         self.opp = torch.empty(n * 56 * 162, dtype=f, device=dev)
         self.hand = torch.empty(n * 56 * 54, dtype=f, device=dev)
         self.talon = torch.empty(n * 330, dtype=f, device=dev)
@@ -83,10 +87,13 @@ class _Arena:
 class Samoigra:
     """``igralci`` = 4 (default): four players with their own networks and epsilon, as in the reference; ``igralci`` = 1:
     one shared set plays every seat.  ``mreze``: None (fresh random nets), one dict (shared, implies one player) or a
-    sequence of four dicts; ``random_card``: one epsilon or one per player (``Nevronski_igralec.random_card``)."""
+    sequence of four dicts; ``random_card``: one epsilon or one per player (``Nevronski_igralec.random_card``);
+    ``dtype``: element type of the observations and of the inference forwards (fp32, bf16 or fp16)."""
 
     def __init__(self, n_envs: int, mreze: Union[None, dict, Sequence[dict]] = None, device: int = 0,
-                 seed: Optional[int] = None, random_card: Union[float, Sequence[float]] = 0.05, igralci: int = 4):
+                 seed: Optional[int] = None, random_card: Union[float, Sequence[float]] = 0.05, igralci: int = 4,
+                 dtype: torch.dtype = torch.float32):
+        E.dtype_code(dtype)                                            # ValueError for anything but fp32 / bf16 / fp16
         if seed is None:
             seed = int.from_bytes(os.urandom(8), "little")
         self.env = E.TarokEnv(n_envs, seed=seed, device=device, history=True)
@@ -109,6 +116,8 @@ class Samoigra:
         self.random_card = eps
         self.gen = torch.Generator(device=self.dev)
         self.gen.manual_seed(seed & 0x7FFFFFFFFFFFFFFF)
+        self.dtype = dtype
+        self._kopije = {}                # (player, net name) -> (master net, its copy cast to dtype)
         self._arena = None
         self.zadnji_koraki = None        # per step: number of buckets walked (diagnostics)
 
@@ -137,20 +146,40 @@ class Samoigra:
             return [opp, hand, talon, decl, disc]
         return [opp, a.king[off * 4: (off + B) * 4].view(B, 4), hand, talon, decl, disc]
 
+    def _mreze_igre(self) -> List[dict]:
+        """The nets the forwards of ``odigraj`` run: the fp32 masters themselves, or for another dtype copies cast to it that
+        take the masters' current weights and buffers at every rollout (a few hundred KB)."""
+        if self.dtype == torch.float32:
+            return self.mreze
+        out = []
+        for p, d in enumerate(self.mreze):
+            c = {}
+            for k, m in d.items():
+                izvor, kopija = self._kopije.get((p, k), (None, None))
+                if izvor is not m:
+                    kopija = copy.deepcopy(m).to(self.dtype)
+                    self._kopije[(p, k)] = (m, kopija)
+                else:
+                    for a, b in zip(kopija.state_dict().values(), m.state_dict().values()):
+                        a.copy_(b)
+                c[k] = kopija.eval()
+            out.append(c)
+        return out
+
     # ------------------------------------------------------------------ one rollout
     @torch.no_grad()
     def odigraj(self, first_game_id: int = 0, meri: bool = False):
         """Plays the whole batch once.  Returns (stats int64[32], per-section milliseconds or None)."""
-        env, n, ura, P = self.env, self.n, _Ura(meri), self.igralci
+        env, n, ura, P, dt, mreze = self.env, self.n, _Ura(meri), self.igralci, self.dtype, self._mreze_igre()
         if self._arena is None:
-            self._arena = _Arena(n, self.dev)
+            self._arena = _Arena(n, self.dev, dt)
         env.reset_stats()
         with ura("env"):
             env.deal(first_game_id)
         kdo = self._igralec_sedeza(first_game_id)                              # [n,4] player of each seat
         # ---- bidding: Nevronski_igralec.pripavi_licitiram / predict_licitiram / licitiram (Igralec.py:278-306)
         with ura("obs"):
-            x = env.obs_hands()                                                # [n,4,54]
+            x = env.obs_hands(dt)                                              # [n,4,54]
         namen = torch.empty((n, 4), dtype=torch.int64, device=self.dev)
         vrsta_iger = torch.arange(n, device=self.dev)
         for p in range(P):
@@ -159,12 +188,12 @@ class Samoigra:
                     sedez = (p - (vrsta_iger + int(first_game_id))) & 3
                     xp = x[vrsta_iger, sedez]
                 with ura("forward"):
-                    y = self.mreze[p]["Vrednotenje_roke"](xp)                  # [n,18]
+                    y = mreze[p]["Vrednotenje_roke"](xp)                       # [n,18]
                 with ura("select"):
                     namen[vrsta_iger, sedez] = y.argmax(dim=-1)
             else:
                 with ura("forward"):
-                    y = self.mreze[0]["Vrednotenje_roke"](x.view(n * 4, 54)).view(n, 4, 18)
+                    y = mreze[0]["Vrednotenje_roke"](x.view(n * 4, 54)).view(n, 4, 18)
                 with ura("select"):
                     namen = y.argmax(dim=-1)
         with ura("select"):                                                    # random.random() < random_card (Igralec.py:300-301)
@@ -189,9 +218,9 @@ class Samoigra:
             if sel.numel() == 0:
                 continue
             with ura("obs"):
-                vhod, _ = env.obs_exchange(sel)
+                vhod, _ = env.obs_exchange(sel, dt)
             with ura("forward"):
-                q = self.mreze[p]["Zalaganje"](vhod)
+                q = mreze[p]["Zalaganje"](vhod)
             with ura("select"):
                 env.select_exchange(q, sel, self.random_card[p], group_out=kupcek, discard_out=zalozi)
         with ura("env"):
@@ -216,7 +245,7 @@ class Samoigra:
                 for k in polni:
                     p, vr, T = k // 28, (k % 28) // 7, 8 * (k % 7 + 1)
                     vhod = self._vhod(vr, T, int(stevci[k]), int(stevci[128 + k]), int(stevci[256 + k]))
-                    q[k] = self.mreze[p][_NET_OF_KIND[vr]](vhod).contiguous()      # the legal-mask vector is not a net input (Igralec.py:333)
+                    q[k] = mreze[p][_NET_OF_KIND[vr]](vhod).contiguous()           # the legal-mask vector is not a net input (Igralec.py:333)
             with ura("select"):                                                # every bucket's argmax / epsilon in one launch
                 env.select_action_buckets(skupaj, q, eps4, karte, qmax)
             with ura("env"):
