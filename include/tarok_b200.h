@@ -78,8 +78,8 @@ enum { TAROK_F_HANDS = 0,   /* uint64 [4, n_alloc]  hand bitboards (Roka, Roka.p
 /* stats vector: [0..3] score sum by seat, [4..7] score sum by player ((seat+game_id)%4, Tarok.py:34,59-61),
    [8..17] contract histogram, [18] finished deals, [19] env-steps (card plays), [20] error games (these at scoring);
    [21] error events: counted at once by the stepwise call that makes a game an error game (tarok_set_deals,
-   tarok_auction, tarok_force_contract, tarok_exchange, tarok_step, tarok_setup_synth), so at most once per game and
-   deal; the fused kernel does not count them. */
+   tarok_auction, tarok_force_contract, tarok_exchange, tarok_step, tarok_setup_synth and the *_bots entries), so at most
+   once per game and deal; the fused kernel does not count them. */
 #define TAROK_STATS_LEN 32
 
 /* ---- life cycle ---------------------------------------------------------------------------- */
@@ -132,6 +132,30 @@ int tarok_auction_synth(tarok_t* h, uint32_t mode /* 17 | 18 */, void* stream);
 int tarok_force_contract(tarok_t* h, const uint8_t* contract_dev, const uint8_t* declarer_dev,
                          const uint8_t* king_dev, void* stream);
 int tarok_force_contract_synth(tarok_t* h, uint32_t mode /* 0..9 | 16 */, void* stream);
+
+/* ---- mixed tables: Bot_igralec seats beside caller-driven (neural) seats ----------------------------------------------
+   bots_dev: uint8 [n_games], a per-game seat mask: bit s set = seat s of that game is a Bot_igralec (Igralec.py:145-171)
+   whose decisions are drawn in-kernel from the same stateless Philox draws as the all-bot paths -- its bids from the bid
+   block (mode 18), its king from setup-block word 2, its exchange from words 1 (group 0), its cards from play_draw -- so a
+   bot seat can sit anywhere and every game stays replayable from (seed, global game id).  A game whose byte has any of
+   bits 4-7 set becomes an error game (counted once in stats[21]).  A NULL bots_dev, or a pointer that breaks an alignment
+   rule, fails the call (< 0) and writes nothing.  With bots_dev all zero each entry computes what its plain namesake does;
+   with 0x0F everywhere, deal + the three entries + score compute what deal + tarok_auction_synth(18) +
+   tarok_exchange_synth(0) + 48 x tarok_step_random + score do.
+   tarok_auction_bots: tarok_auction where bot seats draw a fresh bid at every licitiram call (the draw mode 18 takes at the
+     same overall call number) and their intent bytes are ignored; a bot declarer of a king game calls the king mode 18
+     would, a neural one the suit of its original intent.  intent_dev 4-byte aligned, as for tarok_auction.
+   tarok_exchange_bots: tarok_exchange where games whose declarer's seat is a bot take the Bot exchange (group 0, uniform
+     discards) and ignore their group / discard entries.  discard_dev 8-byte aligned.
+   tarok_step_bots: tarok_step where a bot to move plays the uniform legal card tarok_step_random would play at that game's
+     play index; its card byte is ignored, except TAROK_CARD_SKIP, which still holds the game for this launch.  card_dev and
+     bots_dev 2-byte aligned.  This entry always runs the plain play_step kernel (TAROK_OPT_STEP_IMPL 2 / 3 select
+     persistent variants for the other step entries only), keeps the lock-step specialisation and PDL, and neither reads
+     nor writes the draw cache of the random chains. */
+int tarok_auction_bots(tarok_t* h, const uint8_t* intent_dev, const uint8_t* bots_dev, void* stream);
+int tarok_exchange_bots(tarok_t* h, const uint8_t* group_dev, const uint64_t* discard_dev, const uint8_t* bots_dev,
+                        void* stream);
+int tarok_step_bots(tarok_t* h, const uint8_t* card_dev, const uint8_t* bots_dev, void* stream);
 
 /* ---- talon exchange: Navadna_igra.odpri_talon + start (Navadna_igra.py:36-68),
         Roka.mozno_zalozit (Roka.py:23-27), player side Igralec.py:161-171 ---------------------- */

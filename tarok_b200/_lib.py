@@ -31,6 +31,9 @@ SIGNATURES = {
     "tarok_force_contract_synth": (_I, [_VP, _U32, _VP]),
     "tarok_exchange": (_I, [_VP, _VP, _VP, _VP]),
     "tarok_exchange_synth": (_I, [_VP, _U32, _VP]),
+    "tarok_auction_bots": (_I, [_VP, _VP, _VP, _VP]),
+    "tarok_exchange_bots": (_I, [_VP, _VP, _VP, _VP, _VP]),
+    "tarok_step_bots": (_I, [_VP, _VP, _VP, _VP]),
     "tarok_legal_mask": (_I, [_VP, _VP, _VP]),
     "tarok_hands_by_seat": (_I, [_VP, _VP, _VP]),
     "tarok_step": (_I, [_VP, _VP, _VP]),

@@ -125,11 +125,12 @@ struct DeviceGuard {
 // play_step launcher.  Default: the plain kernel, one 512-game tile per CTA, compiled per trick position for lock-step
 // batches (the hint) with programmatic dependent launch; TAROK_OPT_STEP_IMPL=2 selects the persistent TMA-staged variant
 // (one CTA per resident slot, 4 per SM), which measures slower on B200 and is kept for comparison (tools/step_ab.py).
-template <bool RANDOM, bool MASK = true, bool GRAPH = false>
-static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s) {
+// BOTS (tarok_step_bots, `bots` = the per-game seat masks) always takes the plain kernel: the persistent variants do not cover it.
+template <bool RANDOM, bool MASK = true, bool GRAPH = false, bool BOTS = false>
+static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s, const uint8_t* bots = nullptr) {
     const unsigned tiles = grid2(h->e.n_alloc);
     const unsigned resident = (unsigned)h->sm_count * 4u;
-    const bool tma = h->step_impl == 2;
+    const bool tma = h->step_impl == 2 && !BOTS;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(tma ? (tiles < resident ? tiles : resident) : tiles);
     cfg.blockDim = dim3(tk::CTA);
@@ -159,11 +160,11 @@ static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s) {
     else {
         const int hint = h->lockstep ? h->lock_plays : -1;
         switch (hint >= 0 ? (hint & 3) : 4) {
-            case 0: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 0, MASK, GRAPH>, h->e, action, hint); break;
-            case 1: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 1, MASK, GRAPH>, h->e, action, hint); break;
-            case 2: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 2, MASK, GRAPH>, h->e, action, hint); break;
-            case 3: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 3, MASK, GRAPH>, h->e, action, hint); break;
-            default: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, -1, MASK, GRAPH>, h->e, action, hint); break;
+            case 0: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 0, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+            case 1: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+            case 2: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 2, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+            case 3: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 3, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+            default: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, -1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
         }
     }
     // lock-step bookkeeping (only a hint to the kernel, which verifies it per warp): every live game has made
@@ -377,6 +378,16 @@ int tarok_auction(tarok_t* h, const uint8_t* intent_dev, void* stream) {
     return 0;
 }
 
+int tarok_auction_bots(tarok_t* h, const uint8_t* intent_dev, const uint8_t* bots_dev, void* stream) {
+    TK_CHECK_HANDLE(h);
+    if (!intent_dev || !bots_dev) return fail(h, -1, "intent_dev/bots_dev is null");
+    if (((uintptr_t)intent_dev) & 3u) return fail(h, -1, "intent_dev must be 4-byte aligned");
+    DeviceGuard dg(h->device);
+    tk::k_begin<tk::SRC_MIXED><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, 0u, intent_dev, bots_dev, nullptr);
+    TK_LAUNCH_OK(h);
+    return 0;
+}
+
 int tarok_auction_synth(tarok_t* h, uint32_t mode, void* stream) {
     TK_CHECK_HANDLE(h);
     if (mode != TAROK_MODE_AUCTION_UNIFORM && mode != TAROK_MODE_AUCTION_BOT) return fail(h, -1, "bad auction mode %u", mode);
@@ -411,7 +422,17 @@ int tarok_exchange(tarok_t* h, const uint8_t* group_dev, const uint64_t* discard
     TK_CHECK_HANDLE(h);
     if (!group_dev || !discard_dev) return fail(h, -1, "group_dev/discard_dev is null");
     DeviceGuard dg(h->device);
-    tk::k_exchange<false><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, 0u, group_dev, (const u64*)discard_dev);
+    tk::k_exchange<false><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, 0u, group_dev, (const u64*)discard_dev, nullptr);
+    TK_LAUNCH_OK(h);
+    return 0;
+}
+
+int tarok_exchange_bots(tarok_t* h, const uint8_t* group_dev, const uint64_t* discard_dev, const uint8_t* bots_dev, void* stream) {
+    TK_CHECK_HANDLE(h);
+    if (!group_dev || !discard_dev || !bots_dev) return fail(h, -1, "group_dev/discard_dev/bots_dev is null");
+    if (((uintptr_t)discard_dev) & 7u) return fail(h, -1, "discard_dev must be 8-byte aligned");
+    DeviceGuard dg(h->device);
+    tk::k_exchange<false, true><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, 0u, group_dev, (const u64*)discard_dev, bots_dev);
     TK_LAUNCH_OK(h);
     return 0;
 }
@@ -419,7 +440,7 @@ int tarok_exchange(tarok_t* h, const uint8_t* group_dev, const uint64_t* discard
 int tarok_exchange_synth(tarok_t* h, uint32_t random_group, void* stream) {
     TK_CHECK_HANDLE(h);
     DeviceGuard dg(h->device);
-    tk::k_exchange<true><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, random_group, nullptr, nullptr);
+    tk::k_exchange<true><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, random_group, nullptr, nullptr, nullptr);
     TK_LAUNCH_OK(h);
     return 0;
 }
@@ -451,6 +472,16 @@ int tarok_step(tarok_t* h, const uint8_t* card_dev, void* stream) {
     if (((uintptr_t)card_dev) & 1u) return fail(h, -1, "card_dev must be 2-byte aligned");
     DeviceGuard dg(h->device);
     launch_step<false>(h, card_dev, S(stream));
+    TK_LAUNCH_OK(h);
+    return 0;
+}
+
+int tarok_step_bots(tarok_t* h, const uint8_t* card_dev, const uint8_t* bots_dev, void* stream) {
+    TK_CHECK_HANDLE(h);
+    if (!card_dev || !bots_dev) return fail(h, -1, "card_dev/bots_dev is null");
+    if ((((uintptr_t)card_dev) | ((uintptr_t)bots_dev)) & 1u) return fail(h, -1, "card_dev and bots_dev must be 2-byte aligned");
+    DeviceGuard dg(h->device);
+    launch_step<false, true, false, true>(h, card_dev, S(stream), bots_dev);
     TK_LAUNCH_OK(h);
     return 0;
 }
@@ -536,7 +567,7 @@ int tarok_allreduce_stats(tarok_t* h, void* nccl_comm, int64_t* out_dev, void* s
 // ---- whole deals --------------------------------------------------------------------------------------
 
 static int play_out_stepwise(tarok_t* h, uint32_t random_group, void* stream) {
-    tk::k_exchange<true><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, random_group, nullptr, nullptr);
+    tk::k_exchange<true><<<grid1(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, random_group, nullptr, nullptr, nullptr);
     TK_LAUNCH_OK(h);
     if (int rc = random_chain(h, 48, S(stream))) return rc;
     if (h->materialise) tk::k_score<true><<<grid2(h->e.n_alloc), tk::CTA, 0, S(stream)>>>(h->e, h->e.scores, h->e.n_alloc);

@@ -35,6 +35,9 @@ constexpr int TILE = 2 * CTA;          // games per CTA in the 2-games-per-lane 
 #ifndef TK_STEP_BLOCKS_FORCED
 #define TK_STEP_BLOCKS_FORCED 5   // 46-48 registers: 8.63 -> 8.22 us per launch at 1 M deals (6 blocks = 40 registers spills and loses)
 #endif
+#ifndef TK_STEP_BLOCKS_BOTS
+#define TK_STEP_BLOCKS_BOTS 4     // tarok_step_bots: the forced path plus a Philox block and a pick; 64 registers keep it spill-free
+#endif
 #ifndef TK_SETUP_BLOCKS
 #define TK_SETUP_BLOCKS 3
 #endif
@@ -413,16 +416,24 @@ __global__ void __launch_bounds__(CTA) k_export_perm(Env e, uint8_t* __restrict_
 // ------------------------------------------------------------------------------------------------
 // contract start: auction (Igra.licitacija) or forced contract, then Igra.start dispatch + teams.
 // ------------------------------------------------------------------------------------------------
-enum : int { SRC_FORCED = 0, SRC_INTENTS = 1, SRC_SYNTH = 2 };
+// SRC_MIXED: per-seat players, fixed intents (a) beside Bot_igralec seats (bit s of the mask byte b[g]): tarok_auction_bots
+enum : int { SRC_FORCED = 0, SRC_INTENTS = 1, SRC_SYNTH = 2, SRC_MIXED = 3 };
 
 struct WantFixed { int tip[4]; __device__ int operator()(int seat, int) const {
-    return seat == 0 ? tip[0] : seat == 1 ? tip[1] : seat == 2 ? tip[2] : tip[3]; } };
+    return seat == 0 ? tip[0] : seat == 1 ? tip[1] : seat == 2 ? tip[2] : tip[3]; }
+    __device__ bool fixed(int) const { return true; } };
 // np.random.choice([Naprej,Tri,Dve,Ena], p=[.5,1/6,1/6,1/6]) at EVERY call (Igralec.py:151): call i takes the i-th of the
 // sixteen base-6 digits decoded from words 0 and 1 of the bid block (eight batched draws per word); an auction of
 // Bot players never needs more (the bids only rise Tri -> Dve -> Ena), calls past 16 would use one word each.
 struct WantBot { const Rng& rng; u64 gid; u64 digits; __device__ int operator()(int, int call) const {
     const u32 u = call < 16 ? (u32)(digits >> (3 * call)) & 7u : draw(rng, gid, ST_BID, 64u + (u32)call, 6u);
-    return u < 3u ? (int)C_NAPREJ : (int)(C_TRI + (u - 3u)); } };
+    return u < 3u ? (int)C_NAPREJ : (int)(C_TRI + (u - 3u)); }
+    __device__ bool fixed(int) const { return false; } };
+// Bot seats (bit s of `bots`) ask WantBot afresh at every call -- at overall call c the draw mode 18 takes at call c --, the
+// other seats keep their fixed intent.
+struct WantMixed { WantFixed f; WantBot b; u32 bots;
+    __device__ bool fixed(int seat) const { return !((bots >> seat) & 1u); }
+    __device__ int operator()(int seat, int call) const { return fixed(seat) ? f(seat, call) : b(seat, call); } };
 
 constexpr u64 BOUNDS8_6x8 = 0x0606060606060606ull;
 __device__ __forceinline__ u32 bot_digits8(u32 x, const Rng& rng, u64 gid, u32 word) {    // eight draws of [0,6) -> 3 bits each
@@ -458,13 +469,38 @@ __device__ __forceinline__ void resolve_contract(const Rng& rng, u64 gid, u32 mo
         index2igra(in.x, w.tip[0], su[0]); index2igra(in.y, w.tip[1], su[1]);
         index2igra(in.z, w.tip[2], su[2]); index2igra(in.w, w.tip[3], su[3]);
         int d, k;
-        licitacija<true>(w, d, k);
+        licitacija(w, d, k);
         contract = (u32)k; declarer = (u32)d;
         // king = the suit attached to the declarer's ORIGINAL intent (Igralec.py:298,308-310)
         king = d == 0 ? su[0] : d == 1 ? su[1] : d == 2 ? su[2] : su[3];
         // every seat is asked at least once, so every intent counts: one past index 19 (index2igra[idx] would raise in
         // the reference) makes an error game through begin_contract's unknown-contract check
         if (max(max((u32)in.x, (u32)in.y), max((u32)in.z, (u32)in.w)) > 19u) contract = C_NONE;
+    } else if (SRC == SRC_MIXED) {
+        const uchar4 in = reinterpret_cast<const uchar4*>(a)[g];
+        const u32 bots = b[g];
+        // the bid block is only needed when a bot seat bids (words 0-1: sixteen base-6 digits, as in mode 18)
+        u64 digits = 0;
+        if (bots & 15u) {
+            const Words4 bb = philox_block(rng, gid, ST_BID, 0u);
+            digits = (u64)bot_digits8(bb.w[0], rng, gid, 0u) | ((u64)bot_digits8(bb.w[1], rng, gid, 1u) << 24);
+        }
+        WantMixed w{WantFixed{}, WantBot{rng, gid, digits}, bots};
+        u32 su[4];
+        index2igra(in.x, w.f.tip[0], su[0]); index2igra(in.y, w.f.tip[1], su[1]);
+        index2igra(in.z, w.f.tip[2], su[2]); index2igra(in.w, w.f.tip[3], su[3]);
+        int d, k;
+        licitacija(w, d, k);
+        contract = (u32)k; declarer = (u32)d;
+        // a bot declarer of a king game calls the king of setup-block word 2 (as mode 18), a neural one the suit of its
+        // original intent (as tarok_auction)
+        const u32 sd = d == 0 ? su[0] : d == 1 ? su[1] : d == 2 ? su[2] : su[3];
+        king = ((bots >> d) & 1u) ? (is_king_game(contract) ? draw(rng, gid, ST_FORCE, 2u, 4u) : NO_KING) : sd;
+        // the intent of a bot seat is never read; one past index 19 at another seat, or a mask bit above seat 3, makes an
+        // error game through begin_contract's unknown-contract check
+        const u32 top = max(max((bots & 1u) ? 0u : (u32)in.x, (bots & 2u) ? 0u : (u32)in.y),
+                            max((bots & 4u) ? 0u : (u32)in.z, (bots & 8u) ? 0u : (u32)in.w));
+        if (top > 19u || bots > 15u) contract = C_NONE;
     } else {
         if (mode == 17u) {          // TAROK_MODE_AUCTION_UNIFORM: four batched draws of [0,18) from word 0 of the bid block
             u32 x = philox_block(rng, gid, ST_BID, 0u).w[0];
@@ -480,14 +516,14 @@ __device__ __forceinline__ void resolve_contract(const Rng& rng, u64 gid, u32 mo
 #pragma unroll
             for (int s = 0; s < 4; s++) index2igra(idx[s], w.tip[s], su[s]);
             int d, k;
-            licitacija<true>(w, d, k);
+            licitacija(w, d, k);
             contract = (u32)k; declarer = (u32)d;
             king = d == 0 ? su[0] : d == 1 ? su[1] : d == 2 ? su[2] : su[3];
         } else if (mode == 18u) {   // TAROK_MODE_AUCTION_BOT
             const Words4 bb = philox_block(rng, gid, ST_BID, 0u);
             WantBot w{rng, gid, (u64)bot_digits8(bb.w[0], rng, gid, 0u) | ((u64)bot_digits8(bb.w[1], rng, gid, 1u) << 24)};
             int d, k;
-            licitacija<false>(w, d, k);
+            licitacija(w, d, k);
             contract = (u32)k; declarer = (u32)d;
             king = is_king_game(contract) ? draw_from_word(sb.w[2], rng, gid, ST_FORCE, 2u, 4u) : NO_KING;   // Igralec.py:155-156
         } else {
@@ -584,9 +620,11 @@ __device__ __forceinline__ bool exchange_game(const Rng& rng, u64 gid, u32 rando
     return true;
 }
 
-template <bool SYNTH>
+// BOTS (tarok_exchange_bots): a game whose declarer's seat has its bit set in bots[g] takes the synthetic Bot exchange
+// (group 0, the discards of setup-block word 1) and ignores its group / discard entries; a mask byte above 15 is an error.
+template <bool SYNTH, bool BOTS = false>
 __global__ void __launch_bounds__(CTA) k_exchange(Env e, u32 random_group, const uint8_t* __restrict__ group,
-                                                  const u64* __restrict__ discard) {
+                                                  const u64* __restrict__ discard, const uint8_t* __restrict__ bots) {
     u64 g = (u64)blockIdx.x * CTA + threadIdx.x;
     if (g >= e.n) return;
     u64 meta = e.meta[g];
@@ -601,8 +639,13 @@ __global__ void __launch_bounds__(CTA) k_exchange(Env e, u32 random_group, const
     u64 talon = e.talon[g], order = e.torder[g], dout = 0;
     Words4 sb = {{0, 0, 0, 0}};
     const u64 gid = e.first_gid + g;
-    if (SYNTH) sb = setup_block(e.rng, gid);
-    bool ok = exchange_game<SYNTH>(e.rng, gid, random_group, sb, meta, hand, pile, talon, order,
+    const u32 bm = BOTS ? (u32)bots[g] : 0u;
+    const bool bot = BOTS && ((bm >> decl) & 1u);
+    if (SYNTH || bot) sb = setup_block(e.rng, gid);
+    bool ok;
+    if (BOTS && bm > 15u) ok = false;
+    else if (bot) ok = exchange_game<true>(e.rng, gid, 0u, sb, meta, hand, pile, talon, order, 0u, 0ull, dout);
+    else ok = exchange_game<SYNTH>(e.rng, gid, random_group, sb, meta, hand, pile, talon, order,
                                    SYNTH ? 0u : (u32)group[g], SYNTH ? 0ull : discard[g], dout);
     if (!ok) {
         meta = mset(meta, M_PHASE, 2, PH_DONE) | (1ull << M_ERR);
@@ -718,17 +761,29 @@ __device__ __forceinline__ void store_masks(const Env& e, u32 g, const ulonglong
     if (!sk1) e.mask[g + 1] = k1;
 }
 
+// ---- action sources of play_step: RANDOM = in-kernel uniform-random players (tarok_step_random); otherwise the caller's
+// card bytes (tarok_step), and with BOTS (tarok_step_bots) the per-game seat mask `bm` (bit s = seat s is a Bot_igralec):
+// a bot mover plays the uniform legal card tarok_step_random would play at that play index (play_draw on (gid, plays)) and
+// its card byte is ignored, except CARD_SKIP, which holds the game as for everybody.  A mask byte above 15 makes the game an
+// error game (counted at once, like an illegal card).
+__device__ __forceinline__ bool bot_moves(u64 meta, u32 bm) { return (bm >> mover_of(meta)) & 1u; }
+__device__ __forceinline__ u64 input_error(const Env& e, u64 meta) {
+    atomicAdd((unsigned long long*)&e.stats[S_ERR_EVENTS], 1ull);
+    return mset(meta, M_PHASE, 2, PH_DONE) | (1ull << M_ERR);
+}
+
 // ---- general path: any mix of trick positions; the four slots of the game are in registers ----------------------
-template <bool RANDOM, bool MASK>
+template <bool RANDOM, bool MASK, bool BOTS = false>
 __device__ __forceinline__ void step_game_any(const Env& e, u32 g, u64& meta, u64 s0, u64 s1, u64 s2, u64 s3, u32 card,
-                                              const Words4& rnd, u64& next_mask) {
+                                              const Words4& rnd, u64& next_mask, u32 bm = 0u) {
     const u32 na = (u32)e.n_alloc;
     const u32 lo = (u32)meta, hi = (u32)(meta >> 32);
     const u32 pos = (lo >> M_POS) & 3u, leader = (lo >> M_LEADER) & 3u, kf = (lo >> M_KLOPFAM) & 1u;
     const u32 mover = (leader + pos) & 3u;
     const u32 plays = (hi >> (M_PLAYS - 32)) & 63u;
     u64 hand = sel4(s0, s1, s2, s3, pos);                          // the seat to move sits in slot `pos`
-    if (RANDOM) {
+    if (BOTS && bm > 15u) { meta = input_error(e, meta); next_mask = 0; return; }
+    if (RANDOM || (BOTS && ((bm >> mover) & 1u))) {
         const u64 legal = legal_moves(hand, pos != 0, hi & 63u, kf);
         card = nth_set_bit(legal, play_draw<-1>(rnd, e.rng, e.first_gid + g, plays, (u32)__popcll(legal)));
     }
@@ -767,14 +822,19 @@ __device__ __forceinline__ void pair_blocks(const Env& e, u32 g, u32 t0, u32 t1,
     if (((gid & 1ull) || t0 != t1) && a1) r1 = play_block(e.rng, gid + 1, t1);
 }
 
-template <bool RANDOM, bool MASK = true>
+template <bool RANDOM, bool MASK = true, bool BOTS = false>
 __device__ __forceinline__ void step_pair_any(const Env& e, u32 g, ulonglong2& m, bool a0, bool a1, ulonglong2 s0,
-                                              ulonglong2 s1, ulonglong2 s2, ulonglong2 s3, u32 act) {
+                                              ulonglong2 s1, ulonglong2 s2, ulonglong2 s3, u32 act, u32 bm2 = 0u) {
     Words4 r0 = {{0, 0, 0, 0}}, r1 = {{0, 0, 0, 0}};
-    if (RANDOM) pair_blocks(e, g, ((u32)(m.x >> 32) >> (M_PLAYS - 30)) & 15u, ((u32)(m.y >> 32) >> (M_PLAYS - 30)) & 15u, a1, r0, r1);
+    const u32 t0 = ((u32)(m.x >> 32) >> (M_PLAYS - 30)) & 15u, t1 = ((u32)(m.y >> 32) >> (M_PLAYS - 30)) & 15u;
+    if (RANDOM) pair_blocks(e, g, t0, t1, a1, r0, r1);
+    if (BOTS) {                                                    // Philox only for a pair with a bot to move
+        const bool b1 = a1 && bot_moves(m.y, bm2 >> 8);
+        if ((a0 && bot_moves(m.x, bm2 & 0xFFu)) || b1) pair_blocks(e, g, t0, t1, b1, r0, r1);
+    }
     u64 k0 = 0, k1 = 0;
-    if (a0) step_game_any<RANDOM, MASK>(e, g, m.x, s0.x, s1.x, s2.x, s3.x, act & 0xFFu, r0, k0);
-    if (a1) step_game_any<RANDOM, MASK>(e, g + 1, m.y, s0.y, s1.y, s2.y, s3.y, act >> 8, r1, k1);
+    if (a0) step_game_any<RANDOM, MASK, BOTS>(e, g, m.x, s0.x, s1.x, s2.x, s3.x, act & 0xFFu, r0, k0, bm2 & 0xFFu);
+    if (a1) step_game_any<RANDOM, MASK, BOTS>(e, g + 1, m.y, s0.y, s1.y, s2.y, s3.y, act >> 8, r1, k1, bm2 >> 8);
     st2(e.meta + g, m.x, m.y);
     store_masks<RANDOM, MASK>(e, g, m, a0, a1, k0, k1);
 }
@@ -783,9 +843,9 @@ __device__ __forceinline__ void step_pair_any(const Env& e, u32 g, ulonglong2& m
 // whose warp vote failed: slot HAVE in `hm`, slot HAVE + 1 in `n0`, for HAVE == 3 also slots 1, 2 in `n1`, `n2`), or -1.
 // Using them here also keeps those loads above the vote: one memory round trip on the lock-step side.
 // MASK = false: the caller did not load the next seat's slot (n0) for HAVE < 3; it is fetched here.
-template <bool RANDOM, int HAVE, bool MASK = true>
+template <bool RANDOM, int HAVE, bool MASK = true, bool BOTS = false>
 __device__ __forceinline__ void step_pair_general(const Env& e, u32 g, ulonglong2 m, bool a0, bool a1, u32 act,
-                                                  ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2) {
+                                                  ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2, u32 bm2 = 0u) {
     const u32 na = (u32)e.n_alloc;
     ulonglong2 s0, s1, s2, s3;
     if (HAVE >= 0 && HAVE < 3 && !MASK) n0 = ld2(e.hands + ((HAVE + 1) * na + g));
@@ -794,7 +854,7 @@ __device__ __forceinline__ void step_pair_general(const Env& e, u32 g, ulonglong
     else if (HAVE == 2) { s2 = hm; s3 = n0; s0 = ld2(e.hands + g); s1 = ld2(e.hands + (na + g)); }
     else if (HAVE == 3) { s3 = hm; s0 = n0; s1 = n1; s2 = n2; }
     else { s0 = ld2(e.hands + g); s1 = ld2(e.hands + (na + g)); s2 = ld2(e.hands + (2 * na + g)); s3 = ld2(e.hands + (3 * na + g)); }
-    step_pair_any<RANDOM, MASK>(e, g, m, a0, a1, s0, s1, s2, s3, act);
+    step_pair_any<RANDOM, MASK, BOTS>(e, g, m, a0, a1, s0, s1, s2, s3, act, bm2);
 }
 
 // Cold paths of the lock-step kernels, kept out of line so that their registers and code do not weigh on the hot path:
@@ -810,10 +870,10 @@ __device__ __forceinline__ void step_pair_general(const Env& e, u32 g, ulonglong
 #else
 #define TK_COLD __forceinline__
 #endif
-template <bool RANDOM, int HAVE, bool MASK>
+template <bool RANDOM, int HAVE, bool MASK, bool BOTS = false>
 __device__ TK_COLD void step_pair_general_cold(const Env& e, u32 g, ulonglong2 m, bool a0, bool a1, u32 act,
-                                                    ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2) {
-    step_pair_general<RANDOM, HAVE, MASK>(e, g, m, a0, a1, act, hm, n0, n1, n2);
+                                                    ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2, u32 bm2 = 0u) {
+    step_pair_general<RANDOM, HAVE, MASK, BOTS>(e, g, m, a0, a1, act, hm, n0, n1, n2, bm2);
 }
 template <int POS>
 __device__ TK_COLD u32 pair_lanes_cold(const Env& e, u32 g, u32 trick, bool a1) {
@@ -826,9 +886,10 @@ __device__ TK_COLD u32 pair_lanes_cold(const Env& e, u32 g, u32 trick, bool a1) 
 // ---- lock-step path: every live game of the warp has made `hint` plays, so the trick position POS = hint & 3 is a
 // compile-time constant: the mover is slot POS for everybody, the trick-position arithmetic and the trick-end branch fold.
 // hm = slot POS (the mover's hand); POS < 3: n0 = slot POS + 1 (the next seat); POS == 3: n0, n1, n2 = slots 0, 1, 2.
-template <bool RANDOM, int POS, bool MASK>
+template <bool RANDOM, int POS, bool MASK, bool BOTS = false>
 __device__ __forceinline__ void step_game_lock(const Env& e, u32 g, u64& meta, u64& hm, u64& n0, u64& n1, u64& n2, u32 card,
-                                               u32 x16, u64& next_mask, u32& log_out, const uint8_t* __restrict__ sel8, u64 fgid) {
+                                               u32 x16, u64& next_mask, u32& log_out, const uint8_t* __restrict__ sel8, u64 fgid,
+                                               u32 bm = 0u) {
     const u32 na = (u32)e.n_alloc;
     const u32 lo = (u32)meta, hi = (u32)(meta >> 32);
     const u32 leader = (lo >> M_LEADER) & 3u, kf = (lo >> M_KLOPFAM) & 1u;
@@ -837,6 +898,13 @@ __device__ __forceinline__ void step_game_lock(const Env& e, u32 g, u64& meta, u
     if (RANDOM) {
         const u64 legal = legal_moves(hm, POS != 0, hi & 63u, kf);
         card = nth_set_bit_lut(legal, play_pick(x16, e.rng, fgid + g, plays, (u32)__popcll(legal)), sel8);
+    }
+    if (BOTS) {                                                    // no byte-select table in shared memory here
+        if (bm > 15u) { meta = input_error(e, meta); next_mask = 0; return; }
+        if ((bm >> mover) & 1u) {
+            const u64 legal = legal_moves(hm, POS != 0, hi & 63u, kf);
+            card = nth_set_bit(legal, play_pick(x16, e.rng, fgid + g, plays, (u32)__popcll(legal)));
+        }
     }
     PlayResult pr;
     meta = play_card<!RANDOM, POS, false>(meta, hm, card, 0ull, 0ull, pr);
@@ -858,10 +926,10 @@ __device__ __forceinline__ void step_game_lock(const Env& e, u32 g, u64& meta, u
 
 // The work of a lock-step launch on one lane's game pair once its state is in registers: m = meta, hm = slot POS (the
 // mover's hand), n0 = slot POS + 1 (MASK or POS == 3), n1 / n2 = slots 1 / 2 (POS == 3), rc = the draw-cache entry.
-template <bool RANDOM, int POS, bool MASK>
+template <bool RANDOM, int POS, bool MASK, bool BOTS = false>
 __device__ __forceinline__ void step_lock_body(const Env& e, u32 g, int hint, u64 fgid, u32 tag, bool cached, ulonglong2 m,
                                                ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2, uint2 rc, u32 act,
-                                               const uint8_t* __restrict__ sel8) {
+                                               const uint8_t* __restrict__ sel8, u32 bm2 = 0u) {
     const u32 na = (u32)e.n_alloc;
     const bool a0 = (((u32)m.x >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act & 0xFFu) != CARD_SKIP),
                a1 = (((u32)m.y >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act >> 8) != CARD_SKIP);
@@ -870,7 +938,7 @@ __device__ __forceinline__ void step_lock_body(const Env& e, u32 g, int hint, u6
                       && (!a1 || ((u32)(m.y >> 32) >> (M_PLAYS - 32)) == (u32)hint);
     const bool lock = __all_sync(0xFFFFFFFFu, in_step);            // the hint is only a hint: each warp checks it
     if (!a0 && !a1) return;
-    if (!lock) { step_pair_general_cold<RANDOM, POS, MASK>(e, g, m, a0, a1, act, hm, n0, n1, n2); return; }
+    if (!lock) { step_pair_general_cold<RANDOM, POS, MASK, BOTS>(e, g, m, a0, a1, act, hm, n0, n1, n2, bm2); return; }
     u32 x0 = 0, x1 = 0;                            // the two games' 16-bit lanes of this play
     if (RANDOM) {
         if (POS > 0 && cached && rc.x == tag) {
@@ -892,10 +960,19 @@ __device__ __forceinline__ void step_lock_body(const Env& e, u32 g, int hint, u6
             }
         }
     }
+    if (BOTS) {                                    // Philox only for a pair with a bot to move; the draw cache is neither read nor written
+        const bool b1 = a1 && bot_moves(m.y, bm2 >> 8);
+        if ((a0 && bot_moves(m.x, bm2 & 0xFFu)) || b1) {
+            Words4 r0, r1;
+            pair_blocks(e, g, (u32)hint >> 2, (u32)hint >> 2, b1, r0, r1);
+            x0 = play_lane<POS>(r0, fgid + g, (u32)hint);
+            x1 = play_lane<POS>(r1, fgid + g + 1, (u32)hint);
+        }
+    }
     u64 k0 = 0, k1 = 0;
     u32 l0 = 0, l1 = 0;                            // trick-log entries (POS == 3); 0 = nothing to append
-    if (a0) step_game_lock<RANDOM, POS, MASK>(e, g, m.x, hm.x, n0.x, n1.x, n2.x, act & 0xFFu, x0, k0, l0, sel8, fgid);
-    if (a1) step_game_lock<RANDOM, POS, MASK>(e, g + 1, m.y, hm.y, n0.y, n1.y, n2.y, act >> 8, x1, k1, l1, sel8, fgid);
+    if (a0) step_game_lock<RANDOM, POS, MASK, BOTS>(e, g, m.x, hm.x, n0.x, n1.x, n2.x, act & 0xFFu, x0, k0, l0, sel8, fgid, bm2 & 0xFFu);
+    if (a1) step_game_lock<RANDOM, POS, MASK, BOTS>(e, g + 1, m.y, hm.y, n0.y, n1.y, n2.y, act >> 8, x1, k1, l1, sel8, fgid, bm2 >> 8);
     st2(e.hands + (POS * na + g), hm.x, hm.y);     // a game that did not move gets its slot back unchanged
     if (POS == 3) {
         st2(e.hands + g, n0.x, n0.y); st2(e.hands + (na + g), n1.x, n1.y); st2(e.hands + (2 * na + g), n2.x, n2.y);
@@ -911,15 +988,15 @@ __device__ __forceinline__ void step_lock_body(const Env& e, u32 g, int hint, u6
     if (MASK || !RANDOM || POS == 3) store_masks<RANDOM, MASK>(e, g, m, a0, a1, k0, k1);
 }
 
-template <bool RANDOM, int POS, bool MASK>
-__device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restrict__ action, int hint) {
+template <bool RANDOM, int POS, bool MASK, bool BOTS = false>
+__device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restrict__ action, int hint, const uint8_t* __restrict__ bots) {
     const u32 g = (blockIdx.x * CTA + threadIdx.x) * 2;
     const u32 na = (u32)e.n_alloc;                 // the grid covers n_alloc exactly: no partial warps
     __shared__ __align__(16) uint8_t sel8[RANDOM ? SELECT8_SMEM : 16];
     uint2 sel8_mine = {0u, 0u};                    // this thread's 8 bytes of the byte-select table (tarok_rules.cuh): independent of
     if (RANDOM) sel8_mine = select8_fetch();       // the previous launch, so the load is issued before the dependency wait
     // the run parameters: launch parameters, overwritten from the device record first thing in the GRAPH kernel variants
-    const u64 fgid = RANDOM ? e.first_gid : 0ull;
+    const u64 fgid = (RANDOM || BOTS) ? e.first_gid : 0ull;
     const u32 tag = (RANDOM ? e.rc_epoch : 0u) | ((u32)hint >> 2);
 #if !TK_SEL8_LATE
     if (RANDOM) { select8_store(sel8, sel8_mine); __syncthreads(); }
@@ -931,8 +1008,9 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
     ulonglong2 n0 = {0, 0}, n1 = {0, 0}, n2 = {0, 0};
     if (MASK || POS == 3) n0 = ld2(e.hands + (((POS + 1) & 3) * na + g));     // the next seat's slot is only read for its mask
     if (POS == 3) { n1 = ld2(e.hands + (na + g)); n2 = ld2(e.hands + (2 * na + g)); }
-    u32 act = 0;
+    u32 act = 0, bm2 = 0;
     if (!RANDOM) act = load_actions(action, g, e.n);
+    if (BOTS) bm2 = load_actions(bots, g, e.n);   // the seat masks of the pair: one more coalesced 2-byte load
     // draw cache: the pair's Philox block is computed by the position-0 launch of a trick, which leaves the lanes of
     // positions 1-3 behind ({tag, lanes}, 8 B per pair and position); the three launches that follow read 8 B instead of
     // running the ten rounds again.  The tag (epoch of first_gid | trick) makes a stale or never-written entry harmless:
@@ -949,7 +1027,7 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
         __syncthreads();
     }
 #endif
-    step_lock_body<RANDOM, POS, MASK>(e, g, hint, fgid, tag, cached, m, hm, n0, n1, n2, rc, act, sel8);
+    step_lock_body<RANDOM, POS, MASK, BOTS>(e, g, hint, fgid, tag, cached, m, hm, n0, n1, n2, rc, act, sel8, bm2);
 }
 
 // `hint` = the number of plays every live game has made so far (lock-step pipelines know it on the host); POS = hint & 3
@@ -958,22 +1036,25 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
 // in-kernel random steps (tarok_steps_random, the stepwise rollouts) launches its interior steps with MASK = false: no
 // caller can see those masks, so the next seat's slot is neither read nor its legal set computed or stored -- 16 of the
 // 48 bytes a step moves at trick positions 0-2 -- and only the chain's last launch produces the masks.
-template <bool RANDOM, int POS, bool MASK = true, bool GRAPH = false>
-__global__ void __launch_bounds__(CTA, RANDOM ? ((POS >= 0 && POS < 3) ? TK_STEP_BLOCKS_RANDOM_012 : TK_STEP_BLOCKS_RANDOM) : TK_STEP_BLOCKS_FORCED)
-k_step(Env e, const uint8_t* __restrict__ action, int hint) {
+// BOTS (with RANDOM = false): the third action source, tarok_step_bots -- `bots` = the per-game seat masks.
+template <bool RANDOM, int POS, bool MASK = true, bool GRAPH = false, bool BOTS = false>
+__global__ void __launch_bounds__(CTA, RANDOM ? ((POS >= 0 && POS < 3) ? TK_STEP_BLOCKS_RANDOM_012 : TK_STEP_BLOCKS_RANDOM)
+                                           : BOTS ? TK_STEP_BLOCKS_BOTS : TK_STEP_BLOCKS_FORCED)
+k_step(Env e, const uint8_t* __restrict__ action, int hint, const uint8_t* __restrict__ bots) {
     pdl_launch_dependents();
     if constexpr (GRAPH) load_run_params(e);       // written before the graph started: no need to wait for the previous kernel
     if constexpr (POS >= 0) {
-        step_lock<RANDOM, POS, MASK>(e, action, hint);
+        step_lock<RANDOM, POS, MASK, BOTS>(e, action, hint, bots);
     } else {
         const u32 g = (blockIdx.x * CTA + threadIdx.x) * 2;
         pdl_wait();
         const ulonglong2 m = ld2(e.meta + g), z = {0, 0};
-        u32 act = 0;
+        u32 act = 0, bm2 = 0;
         if (!RANDOM) act = load_actions(action, g, e.n);
+        if (BOTS) bm2 = load_actions(bots, g, e.n);
         const bool a0 = (((u32)m.x >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act & 0xFFu) != CARD_SKIP),
                    a1 = (((u32)m.y >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act >> 8) != CARD_SKIP);
-        if (a0 || a1) step_pair_general<RANDOM, -1, MASK>(e, g, m, a0, a1, act, z, z, z, z);
+        if (a0 || a1) step_pair_general<RANDOM, -1, MASK, BOTS>(e, g, m, a0, a1, act, z, z, z, z, bm2);
     }
 }
 

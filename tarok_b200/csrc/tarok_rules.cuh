@@ -183,16 +183,18 @@ __device__ __forceinline__ int bid_filter(int want, int min_igra, int obv, bool 
 }
 
 // Igra.licitacija (Igra.py:75-114) as a state machine over a bidder functor
-//   int Want::operator()(int seat, int call_index)   -> the Tip code the seat wants at this call.
-// FIXED = Nevronski_igralec semantics: the first answer is kept and overwritten by every returned
-// value (Igralec.py:295-304); otherwise (Bot_igralec, Igralec.py:151) every call asks afresh.
-template <bool FIXED, class Want>
+//   int Want::operator()(int seat, int call_index)   -> the Tip code the seat wants at this call;
+//   bool Want::fixed(int seat)                        -> the seat's bidding semantics, per seat:
+// fixed = Nevronski_igralec: the first answer is kept and overwritten by every returned value (Igralec.py:295-304);
+// otherwise (Bot_igralec, Igralec.py:151) every call asks afresh.
+template <class Want>
 __device__ __forceinline__ void licitacija(Want& want, int& declarer, int& contract) {
     int intent[4] = {C_NONE, C_NONE, C_NONE, C_NONE};
     int calls = 0;
     auto call = [&](int seat, int mn, int obv, bool pred) -> int {
+        const bool fixed = want.fixed(seat);
         int w;
-        if (FIXED) {
+        if (fixed) {
             if (intent[seat] == C_NONE) intent[seat] = want(seat, calls);
             w = intent[seat];
         } else {
@@ -200,7 +202,7 @@ __device__ __forceinline__ void licitacija(Want& want, int& declarer, int& contr
         }
         calls++;
         int r = bid_filter(w, mn, obv, pred);
-        if (FIXED) intent[seat] = r;
+        if (fixed) intent[seat] = r;
         return r;
     };
     u32 lic = 0;

@@ -230,11 +230,20 @@ class TarokEnv:
         return out
 
     # ------------------------------------------------------------------ auction / dispatch
-    def auction(self, intents):
+    def _bots(self, bots):
+        """The per-game seat mask of a mixed table (uint8 [n], bit s = seat s is a Bot_igralec) as a device tensor."""
+        return self._dev_u8(bots, (self.n,))
+
+    def auction(self, intents, bots=None):
         """intents: uint8 [n,4] indices into ``Nevronski_igralec.index2igra`` (Igralec.py:717-745), 0..19 (18 Odprti_berac,
-        19 Klop); a game with any intent in 20..255 becomes an error game."""
+        19 Klop); a game with any intent in 20..255 becomes an error game.  ``bots`` (uint8 [n], bit s = seat s is a
+        Bot_igralec): those seats bid as Bot_igralec and their intents are ignored (``tarok_auction_bots``)."""
         x = self._dev_u8(intents, (self.n, 4))
-        self._check(self._lib.tarok_auction(self._h, C.c_void_p(x.data_ptr()), self._stream()))
+        if bots is None:
+            self._check(self._lib.tarok_auction(self._h, C.c_void_p(x.data_ptr()), self._stream()))
+        else:
+            b = self._bots(bots)
+            self._check(self._lib.tarok_auction_bots(self._h, C.c_void_p(x.data_ptr()), C.c_void_p(b.data_ptr()), self._stream()))
 
     def auction_synth(self, mode: int):
         self._check(self._lib.tarok_auction_synth(self._h, int(mode), self._stream()))
@@ -251,14 +260,21 @@ class TarokEnv:
         self._check(self._lib.tarok_force_contract_synth(self._h, int(mode), self._stream()))
 
     # ------------------------------------------------------------------ talon exchange
-    def exchange(self, group, discard):
+    def exchange(self, group, discard, bots=None):
+        """group: uint8 [n], discard: [n] bitboards of the k cards laid down.  ``bots`` (uint8 [n] seat masks): games whose
+        declarer is a bot seat take Bot_igralec's exchange and ignore their entries (``tarok_exchange_bots``)."""
         g = self._dev_u8(group, (self.n,))
         if not isinstance(discard, torch.Tensor):
             discard = torch.from_numpy(np.ascontiguousarray(discard).astype(np.uint64).view(np.int64))
         d = discard.to(device=self.torch_device, dtype=torch.int64).contiguous()
         if tuple(d.shape) != (self.n,):
             raise ValueError("discard must have shape (n,)")
-        self._check(self._lib.tarok_exchange(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(d.data_ptr()), self._stream()))
+        if bots is None:
+            self._check(self._lib.tarok_exchange(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(d.data_ptr()), self._stream()))
+        else:
+            b = self._bots(bots)
+            self._check(self._lib.tarok_exchange_bots(self._h, C.c_void_p(g.data_ptr()), C.c_void_p(d.data_ptr()),
+                                                      C.c_void_p(b.data_ptr()), self._stream()))
 
     def exchange_synth(self, random_group: bool = False):
         self._check(self._lib.tarok_exchange_synth(self._h, 1 if random_group else 0, self._stream()))
@@ -270,14 +286,20 @@ class TarokEnv:
         self._check(self._lib.tarok_legal_mask(self._h, C.c_void_p(out.data_ptr()), self._stream()))
         return out[: self.n]
 
-    def step(self, cards):
-        """One card per live game (``igraj_karto``); cards: uint8 [n] card ids."""
+    def step(self, cards, bots=None):
+        """One card per live game (``igraj_karto``); cards: uint8 [n] card ids.  ``bots`` (uint8 [n] seat masks): a bot to
+        move plays the uniform legal card ``step_random`` would and its card byte is ignored, except 0xFE (skip), which
+        still holds the game (``tarok_step_bots``)."""
         if isinstance(cards, torch.Tensor) and cards.dtype == torch.uint8 and cards.device == self.torch_device \
                 and cards.is_contiguous() and cards.numel() in (self.n, self.n_alloc):
             x = cards                    # used in place (the kernel reads the first n_games bytes only)
         else:
             x = self._dev_u8(cards, (self.n,))
-        self._check(self._lib.tarok_step(self._h, C.c_void_p(x.data_ptr()), self._stream()))
+        if bots is None:
+            self._check(self._lib.tarok_step(self._h, C.c_void_p(x.data_ptr()), self._stream()))
+        else:
+            b = self._bots(bots)
+            self._check(self._lib.tarok_step_bots(self._h, C.c_void_p(x.data_ptr()), C.c_void_p(b.data_ptr()), self._stream()))
 
     def step_random(self, count: int = 1):
         """``count`` back-to-back steps with in-kernel uniform-random legal cards (Bot_igralec, Igralec.py:158-159)."""

@@ -20,6 +20,12 @@ The environment, the bucketing, the observation expansion and the action selecti
 repository; the forward passes stay in the reference's networks (here the PyTorch restatement in ``tarok_b200.mreze``,
 because the upstream ``torch_models.py`` is missing).
 
+Mixed tables: ``Samoigra(..., boti=(2, 3))`` seats ``Bot_igralec`` players beside the neural ones (the usual yardstick of a
+self-play net is its score against uniform-random players).  A bot player needs no nets; its bids, king call, exchange and
+cards are drawn in-kernel by the ``*_bots`` entries (``tarok_auction_bots`` / ``tarok_exchange_bots`` /
+``tarok_step_bots``) from a per-game seat mask built once per rollout, its forwards are skipped (a bucket without a forward
+is left alone by the action selection), it yields no replay samples, and ``stats[4 + p]`` is its score like anybody's.
+
 Mixed precision: ``Samoigra(..., dtype=torch.bfloat16)`` (or ``torch.float16``) plays with observations written in that
 dtype (every value is 0 or 1, so they are exact) and with inference copies of the nets cast to it; the selections read the
 half outputs as they come.  The fp32 master nets, ``nauci`` and ``vzorci`` stay fp32.
@@ -88,12 +94,19 @@ class Samoigra:
     """``igralci`` = 4 (default): four players with their own networks and epsilon, as in the reference; ``igralci`` = 1:
     one shared set plays every seat.  ``mreze``: None (fresh random nets), one dict (shared, implies one player) or a
     sequence of four dicts; ``random_card``: one epsilon or one per player (``Nevronski_igralec.random_card``);
-    ``dtype``: element type of the observations and of the inference forwards (fp32, bf16 or fp16)."""
+    ``dtype``: element type of the observations and of the inference forwards (fp32, bf16 or fp16); ``boti``: the players
+    (0..3, with ``igralci`` = 4) that are ``Bot_igralec`` -- their entry of ``mreze`` may be None and their ``random_card``
+    is ignored."""
 
     def __init__(self, n_envs: int, mreze: Union[None, dict, Sequence[dict]] = None, device: int = 0,
                  seed: Optional[int] = None, random_card: Union[float, Sequence[float]] = 0.05, igralci: int = 4,
-                 dtype: torch.dtype = torch.float32):
+                 dtype: torch.dtype = torch.float32, boti: Sequence[int] = ()):
         E.dtype_code(dtype)                                            # ValueError for anything but fp32 / bf16 / fp16
+        boti = frozenset(int(p) for p in boti)
+        if boti and (igralci != 4 or isinstance(mreze, dict)):
+            raise ValueError("Bot_igralec players need the four players of igralci=4")
+        if any(p < 0 or p > 3 for p in boti):
+            raise ValueError("boti holds player indices 0..3, got %s" % sorted(boti))
         if seed is None:
             seed = int.from_bytes(os.urandom(8), "little")
         self.env = E.TarokEnv(n_envs, seed=seed, device=device, history=True)
@@ -104,11 +117,15 @@ class Samoigra:
         if igralci not in (1, 4):
             raise ValueError("igralci must be 1 (one shared set of nets) or 4 (the reference's four players)")
         self.igralci = igralci
-        self.mreze: List[dict] = list(mreze) if mreze is not None else [ustvari_mreze(self.dev) for _ in range(igralci)]
+        self.boti = boti
+        self.mreze: List[Optional[dict]] = list(mreze) if mreze is not None else \
+            [None if p in boti else ustvari_mreze(self.dev) for p in range(igralci)]
         if len(self.mreze) != igralci:
             raise ValueError("need %d sets of nets" % igralci)
+        if any(d is None for p, d in enumerate(self.mreze) if p not in boti):
+            raise ValueError("every player that is not a bot needs its nets")
         for d in self.mreze:
-            for m in d.values():
+            for m in (d or {}).values():
                 m.eval()                                               # Igralec.py:335
         eps = [float(random_card)] * igralci if isinstance(random_card, (int, float)) else [float(x) for x in random_card]
         if len(eps) != igralci:
@@ -128,6 +145,11 @@ class Samoigra:
             return torch.zeros((self.n, 4), dtype=torch.int64, device=self.dev)
         gid = torch.arange(self.n, dtype=torch.int64, device=self.dev) + int(first_game_id)
         return (gid[:, None] + torch.arange(4, dtype=torch.int64, device=self.dev)[None, :]) & 3
+
+    def _maska_botov(self, kdo: torch.Tensor) -> torch.Tensor:
+        """uint8 [n]: bit s set = the player of seat s (``kdo``) is a bot -- the seat mask of the ``*_bots`` entries."""
+        bot = torch.isin(kdo, torch.tensor(sorted(self.boti), dtype=kdo.dtype, device=self.dev))
+        return (bot.to(torch.uint8) << torch.arange(4, dtype=torch.uint8, device=self.dev)).sum(dim=1, dtype=torch.uint8)
 
     def _vhod(self, vr: int, T: int, B: int, off: int, row: int):
         """The input list of one bucket (reference order, A.4) as views of the arenas ``obs_expand_buckets`` filled:
@@ -153,6 +175,9 @@ class Samoigra:
             return self.mreze
         out = []
         for p, d in enumerate(self.mreze):
+            if d is None:                                              # a bot player
+                out.append(None)
+                continue
             c = {}
             for k, m in d.items():
                 izvor, kopija = self._kopije.get((p, k), (None, None))
@@ -177,12 +202,15 @@ class Samoigra:
         with ura("env"):
             env.deal(first_game_id)
         kdo = self._igralec_sedeza(first_game_id)                              # [n,4] player of each seat
+        boti = self._maska_botov(kdo) if self.boti else None                  # seat masks of the *_bots entries
         # ---- bidding: Nevronski_igralec.pripavi_licitiram / predict_licitiram / licitiram (Igralec.py:278-306)
         with ura("obs"):
             x = env.obs_hands(dt)                                              # [n,4,54]
-        namen = torch.empty((n, 4), dtype=torch.int64, device=self.dev)
+        namen = torch.zeros((n, 4), dtype=torch.int64, device=self.dev)
         vrsta_iger = torch.arange(n, device=self.dev)
         for p in range(P):
+            if p in self.boti:                                                 # bids in-kernel: no forward
+                continue
             if P == 4:                                                         # one seat per game belongs to player p
                 with ura("bucket"):
                     sedez = (p - (vrsta_iger + int(first_game_id))) & 3
@@ -203,7 +231,7 @@ class Samoigra:
                 nakljucno = torch.randint(0, 18, (n, 4), device=self.dev, generator=self.gen)
                 namen = torch.where(razisci, nakljucno, namen)
         with ura("env"):
-            env.auction(namen.to(torch.uint8))
+            env.auction(namen.to(torch.uint8), bots=boti)
         # ---- talon exchange (Igralec.py:357-385): the declarer's player decides
         with ura("bucket"):
             meta = env.meta[:n]
@@ -213,6 +241,8 @@ class Samoigra:
         kupcek = torch.full((n,), 0xFF, dtype=torch.uint8, device=self.dev)
         zalozi = torch.zeros(n, dtype=torch.int64, device=self.dev)
         for p in range(P):
+            if p in self.boti:                                                 # exchanges in-kernel
+                continue
             with ura("bucket"):
                 sel = torch.nonzero(menja & (lastnik == p)).flatten().to(torch.int32)
             if sel.numel() == 0:
@@ -224,7 +254,7 @@ class Samoigra:
             with ura("select"):
                 env.select_exchange(q, sel, self.random_card[p], group_out=kupcek, discard_out=zalozi)
         with ura("env"):
-            env.exchange(kupcek, zalozi)
+            env.exchange(kupcek, zalozi, bots=boti)
         # ---- 48 card plays (Igralec.py:312-355)
         karte = torch.full((env.n_alloc,), 0xFF, dtype=torch.uint8, device=self.dev)
         qmax = torch.zeros(n, dtype=torch.float32, device=self.dev)
@@ -238,7 +268,7 @@ class Samoigra:
                 break
             with ura("obs"):                                                   # every bucket's inputs in one launch
                 env.obs_expand_buckets(skupaj, ar.opp, ar.hand, ar.talon, ar.talon_klop, ar.king, ar.decl, ar.disc)
-            polni = [k for k in range(127) if stevci[k]]
+            polni = [k for k in range(127) if stevci[k] and k // 28 not in self.boti]   # a bot's bucket: no forward
             koraki.append(len(polni))
             q = {}
             with ura("forward"):
@@ -249,7 +279,7 @@ class Samoigra:
             with ura("select"):                                                # every bucket's argmax / epsilon in one launch
                 env.select_action_buckets(skupaj, q, eps4, karte, qmax)
             with ura("env"):
-                env.step(karte)
+                env.step(karte, bots=boti)
         with ura("env"):
             env.score()
         self.zadnji_koraki = koraki
@@ -269,11 +299,13 @@ class Samoigra:
         kind = torch.where((vrsta >= 1) & (vrsta <= 3), torch.ones_like(kind), kind)
         kind = torch.where((vrsta == 7) | (vrsta == 9), torch.full_like(kind, 3), kind)
         gid = torch.arange(n, dtype=torch.int64, device=self.dev) + int(first_game_id)
+        boti = torch.tensor(sorted(self.boti), dtype=torch.int64, device=self.dev)
         for t in range(48):
             igrano = seat[:, t] != 0xFF
             if not bool(igrano.any()):
                 break
             igralec = ((seat[:, t].to(torch.int64) + gid) & 3) if self.igralci == 4 else torch.zeros_like(gid)
+            igrano &= ~torch.isin(igralec, boti)                          # a bot's plays are no samples
             kljuc = igralec * 256 + kind * 64 + rows[:, t].to(kind.dtype)
             for k in torch.unique(kljuc[igrano]).tolist():
                 p, vr, T = k // 256, (k % 256) // 64, k % 64
@@ -286,7 +318,7 @@ class Samoigra:
         loss and optimiser of the reference's models (train.py:23-25; Igralec.py:545-607 fits them with Lightning).
         Training is outside the accelerated path; this exists so the self-play loop closes.  Returns {(player, net): loss}."""
         opt = {(p, k): torch.optim.Adam(self.mreze[p][k].parameters(), lr=lr)
-               for p in range(self.igralci) for k in _NET_OF_KIND.values()}
+               for p in range(self.igralci) if p not in self.boti for k in _NET_OF_KIND.values()}
         izguba, stevec = {}, {}
         for p, ime, T, stanje, dy in self.vzorci(final_reword_factor, first_game_id):
             m = self.mreze[p][ime]

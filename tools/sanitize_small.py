@@ -26,5 +26,7 @@ env.close()
 from tarok_b200.samoigra import Samoigra
 s = Samoigra(512, device=0, seed=1, random_card=[0.1] * 4)
 s.odigraj(0); s.zapri()
+s = Samoigra(512, device=0, seed=1, random_card=[0.1] * 4, boti=(2, 3))    # tarok_auction_bots / _exchange_bots / _step_bots
+s.odigraj(1); s.zapri()
 torch.cuda.synchronize()
 print("sanitize_small ok")
