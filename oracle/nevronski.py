@@ -140,6 +140,53 @@ def dense(o, g, with_mozne=True):
     return out + [unpack(o["mozne"][g])] if with_mozne else out
 
 
+def _bits(b):
+    """Bitboards [...] -> 0/1 uint8 [..., 54], like ``unpack`` but through np.unpackbits (a byte per element, no uint64
+    intermediate): the bulk form for whole batches."""
+    b = np.ascontiguousarray(b, "<u8")
+    return np.unpackbits(b.view(np.uint8).reshape(b.shape + (8,)), axis=-1, bitorder="little")[..., :54]
+
+
+def _one_hot4(idx):
+    idx = np.asarray(idx, np.int64)
+    return ((idx[:, None] == np.arange(4)[None, :]) & (idx[:, None] >= 0)).astype(np.uint8)
+
+
+def dense_batch(o, games, with_mozne=True):
+    """``dense`` for many games at once: ``games`` must share one net type and one T.  Returns the input list with a
+    leading batch axis (uint8), equal game by game to ``dense(o, g)``."""
+    games = np.asarray(games, np.int64)
+    T, kind = int(o["T"][games[0]]), int(o["kind"][games[0]])
+    assert (o["T"][games] == T).all() and (o["kind"][games] == kind).all()
+    B, r = len(games), min(T, 48)
+    opp = np.zeros((B, T, 3, 54), np.uint8)
+    hand = np.zeros((B, T, 54), np.uint8)
+    opp[:, :r] = _bits(o["opp"][games, :r])
+    hand[:, :r] = _bits(o["hand"][games, :r])
+    talon = _bits(o["klop_talon"][games]) if kind == 0 else np.asarray(o["talon"][games], np.uint8)
+    king, decl, disc = _one_hot4(o["king"][games]), _one_hot4(o["decl"][games]), _bits(o["discard"][games])
+    out = {0: [opp, hand, talon], 1: [opp, king, hand, talon, decl, disc], 2: [opp, hand, talon, decl, disc],
+           3: [opp, hand, decl]}[kind]
+    return out + [_bits(o["mozne"][games])] if with_mozne else out
+
+
+def exchange_observation(perm, contract, declarer, king):
+    """menjaj_talon_v_vektor (Igralec.py:535-543) for games waiting for the exchange, from the deal: [hand (n,54) = the
+    declarer's hand as dealt, talon (n,54,6) = talon card perm[48 + j] in column j // k (its group), game (n,15) = one-hot
+    of igra_zalozi2index: (Tri|Dve|Ena, king suit) -> 0..11, Solo_tri/dve/ena -> 12..14], 0/1 uint8."""
+    perm = np.asarray(perm, np.int64)
+    c = np.asarray(contract, np.int64)
+    n, k = len(c), talon_k(c)
+    assert (k > 0).all()
+    hand = _bits(hand_dealt(perm, declarer))
+    talon = np.zeros((n, 54, 6), np.uint8)
+    for j in range(6):
+        talon[np.arange(n), perm[:, 48 + j], j // k] = 1
+    game = np.zeros((n, 15), np.uint8)
+    game[np.arange(n), np.where(c <= 3, (c - 1) * 4 + np.asarray(king, np.int64), 12 + c - 4)] = 1
+    return [hand, talon, game]
+
+
 # ------------------------------------------------------------------ exploration (DESIGN.md section 4)
 _M0, _M1, _W0, _W1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57), 0x9E3779B9, 0xBB67AE85
 _LO = np.uint64(0xFFFFFFFF)

@@ -34,7 +34,7 @@ struct tarok_env {
     tk::RunParams* run_dev;                    // {first_gid, rc_epoch} the GRAPH kernel variants read (rewritten before every replay)
     int capturing;                             // launch the GRAPH variants (set while a rollout graph is being captured)
     cudaGraphExec_t bucket_graph;              // tarok_obs_buckets_host: hist + scan + scatter + counts copy as one launch
-    const void* bucket_key[5];                 // the arguments that graph was captured with
+    const void* bucket_key[6];                 // the arguments that graph was captured with, and first_gid & 3
     int lazy_mask;                             // chains of random steps write legal masks in their last launch only (default on)
     int materialise;                           // tarok_score writes the materialised piles / talon back (default on)
     int chunks;                                // upload/compute/download pipeline depth of the host-buffer entries
@@ -878,7 +878,10 @@ int tarok_obs_buckets(tarok_t* h, int players, int32_t* sel_dev, uint32_t* count
 
 // The same + the 1.5 KB of counts copied to (pinned) host memory.  This runs once per self-play step right after a
 // synchronisation, i.e. on an empty stream, where every launch costs its full latency: the three kernels and the copy are
-// replayed as ONE graph launch (captured per argument set on first use; dropped when an option changes).
+// replayed as ONE graph launch (captured per argument set on first use; dropped when an option changes).  The graph holds
+// the Env by value, and the bucket kernels read first_gid through the player rotation (first_gid + g) & 3: first_gid & 3
+// is part of the key, so a rollout at a first game id of another residue mod 4 re-captures instead of routing every
+// decision by the previous rollout's rotation.
 int tarok_obs_buckets_host(tarok_t* h, int players, int32_t* sel_dev, uint32_t* counts_dev, uint8_t* selkey_dev,
                            uint32_t* counts_host, void* stream) {
     TK_CHECK_HANDLE(h);
@@ -890,7 +893,8 @@ int tarok_obs_buckets_host(tarok_t* h, int players, int32_t* sel_dev, uint32_t* 
     if (!h->cta_hist) TK_CUDA(h, cudaMalloc((void**)&h->cta_hist, (size_t)n_cta * tk::BUCKETS * sizeof(u32)));
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     if (h->use_graph && cudaStreamIsCapturing(s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusNone) {
-        const void* key[5] = {sel_dev, counts_dev, selkey_dev, counts_host, (const void*)(intptr_t)players};
+        const void* key[6] = {sel_dev, counts_dev, selkey_dev, counts_host, (const void*)(intptr_t)players,
+                              (const void*)(intptr_t)(h->e.first_gid & 3u)};
         if (!h->bucket_graph || memcmp(key, h->bucket_key, sizeof(key)) != 0) {
             if (h->bucket_graph) { cudaGraphExecDestroy(h->bucket_graph); h->bucket_graph = nullptr; }
             if (!h->s_cap) TK_CUDA(h, cudaStreamCreateWithFlags(&h->s_cap, cudaStreamNonBlocking));

@@ -146,6 +146,32 @@ def test_device_buckets_match_the_host_partition():
     env.close()
 
 
+def test_buckets_follow_the_first_game_id_of_every_deal():
+    """One handle dealt again and again at first game ids of every residue mod 4 (and above 2^32): the bucket of each game
+    is keyed by the player (mover + game id) % 4 of THAT deal.  The counting sort is replayed from a captured CUDA graph,
+    which must not keep the rotation of the deal it was captured in."""
+    import torch
+    import tarok_b200.env as E
+    n = 5000
+    env = E.TarokEnv(n, seed=99, history=True)
+    for gid0 in (0, 1, 2, 3, 6, 2 ** 32 + 1, 4):
+        env.setup_synth(E.MODE_AUCTION_UNIFORM, gid0)
+        for t in range(3):
+            vrsta, vrstice = env.obs_shape()
+            meta = env.meta[:n]
+            mover = (E.meta_field(meta, E.M_LEADER, 2) + E.meta_field(meta, E.M_POS, 2)) & 3
+            key = vrsta.to(torch.int64) * 7 + (vrstice.to(torch.int64) // 8 - 1)
+            key = key + 28 * ((mover + torch.arange(n, device=meta.device) + gid0) & 3)
+            key = torch.where(vrsta != 255, key, torch.full_like(key, 127)).cpu().numpy()
+            sel, cnt = env.obs_buckets(4)
+            want = np.bincount(key[key != 127], minlength=128)[:128]
+            assert (cnt[:128] == want).all(), (gid0, t)
+            assert (sel[: int(want.sum())].cpu().numpy() == np.argsort(key, kind="stable")[: int(want.sum())]).all()
+            del meta, mover, sel
+            env.step_random()
+    env.close()
+
+
 def test_all_bucket_launches_equal_the_per_bucket_kernels():
     """tarok_obs_expand_buckets / tarok_select_action_buckets (one launch for every bucket of a step) produce exactly what
     tarok_obs_expand / tarok_select_action produce bucket by bucket."""
