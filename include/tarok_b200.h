@@ -86,9 +86,7 @@ enum { TAROK_F_HANDS = 0,   /* uint64 [4, n_alloc]  hand bitboards (Roka, Roka.p
 int tarok_create(int device, uint64_t n_games, uint64_t seed, uint32_t flags, tarok_t** out);
 int tarok_destroy(tarok_t* h);                 /* error if exported tensors are still alive */
 const char* tarok_last_error(const tarok_t* h);/* h may be NULL: last error of a failed tarok_create */
-/* Tuning knobs.  TAROK_OPT_STEP_IMPL: 0 auto (default), 1 plain play_step kernel, 2 persistent TMA-staged kernel (general path),
-   3 persistent prefetching lock-step kernel for the interior launches of random chains (both persistent ones measure slower). */
-#define TAROK_OPT_STEP_IMPL 1
+/* Tuning knobs.  Option id 1 (the play_step implementation) is retired and will not be reused. */
 #define TAROK_OPT_PDL 2        /* 1 (default): chain play_step launches with programmatic dependent launch */
 #define TAROK_OPT_MATERIALISE 4 /* 1 (default): tarok_score writes the full piles / Klop talon back; 0: scores + stats only */
 #define TAROK_OPT_CHUNKS 5      /* 1..32 (default 8): chunks of the upload/compute/download pipeline of tarok_rollout_host/_records */
@@ -149,9 +147,8 @@ int tarok_force_contract_synth(tarok_t* h, uint32_t mode /* 0..9 | 16 */, void* 
      discards) and ignore their group / discard entries.  discard_dev 8-byte aligned.
    tarok_step_bots: tarok_step where a bot to move plays the uniform legal card tarok_step_random would play at that game's
      play index; its card byte is ignored, except TAROK_CARD_SKIP, which still holds the game for this launch.  card_dev and
-     bots_dev 2-byte aligned.  This entry always runs the plain play_step kernel (TAROK_OPT_STEP_IMPL 2 / 3 select
-     persistent variants for the other step entries only), keeps the lock-step specialisation and PDL, and neither reads
-     nor writes the draw cache of the random chains. */
+     bots_dev 2-byte aligned.  This entry keeps the lock-step specialisation and PDL, and neither reads nor writes the
+     draw cache of the random chains. */
 int tarok_auction_bots(tarok_t* h, const uint8_t* intent_dev, const uint8_t* bots_dev, void* stream);
 int tarok_exchange_bots(tarok_t* h, const uint8_t* group_dev, const uint64_t* discard_dev, const uint8_t* bots_dev,
                         void* stream);

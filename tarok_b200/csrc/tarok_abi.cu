@@ -22,8 +22,6 @@ using tk::u32;
 
 struct tarok_env {
     int device;
-    int sm_count;
-    int step_impl;                             // 0 auto, 1 plain k_step, 2 persistent TMA-staged k_step_tma
     int pdl;                                   // chain play_step launches with programmatic dependent launch
     int lockstep;                              // pass the lock-step hint to play_step (specialised per trick position)
     int lock_plays;                            // plays made by every live game since the last deal, -1 = unknown
@@ -122,17 +120,12 @@ struct DeviceGuard {
     ~DeviceGuard() { if (ok) cudaSetDevice(prev); }
 };
 
-// play_step launcher.  Default: the plain kernel, one 512-game tile per CTA, compiled per trick position for lock-step
-// batches (the hint) with programmatic dependent launch; TAROK_OPT_STEP_IMPL=2 selects the persistent TMA-staged variant
-// (one CTA per resident slot, 4 per SM), which measures slower on B200 and is kept for comparison (tools/step_ab.py).
-// BOTS (tarok_step_bots, `bots` = the per-game seat masks) always takes the plain kernel: the persistent variants do not cover it.
+// play_step launcher: one 512-game tile per CTA, compiled per trick position for lock-step batches (the hint), with
+// programmatic dependent launch.  BOTS: tarok_step_bots, `bots` = the per-game seat masks.
 template <bool RANDOM, bool MASK = true, bool GRAPH = false, bool BOTS = false>
 static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s, const uint8_t* bots = nullptr) {
-    const unsigned tiles = grid2(h->e.n_alloc);
-    const unsigned resident = (unsigned)h->sm_count * 4u;
-    const bool tma = h->step_impl == 2 && !BOTS;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(tma ? (tiles < resident ? tiles : resident) : tiles);
+    cfg.gridDim = dim3(grid2(h->e.n_alloc));
     cfg.blockDim = dim3(tk::CTA);
     cfg.dynamicSmemBytes = 0;
     cfg.stream = s;
@@ -141,31 +134,13 @@ static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s, con
     at[0].val.programmaticStreamSerializationAllowed = h->pdl ? 1 : 0;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    // TAROK_OPT_STEP_IMPL = 3: the persistent prefetching kernel for what it covers -- interior launches (no masks) of a
-    // lock-step chain of random steps with the draw cache on for all three positions; everything else takes the plain kernel
-    const bool pp = h->step_impl == 3 && RANDOM && !MASK && h->lockstep && h->lock_plays >= 0 && h->e.rc_rows == 3u;
-    if (pp) {
-        const int hint = h->lock_plays;
-        const int pos = hint & 3;
-        const unsigned per_sm = pos == 3 ? TK_PP_BLOCKS_3 : TK_PP_BLOCKS_012;
-        const unsigned slots = (unsigned)h->sm_count * per_sm;
-        cfg.gridDim = dim3(tiles < slots ? tiles : slots);
-        switch (pos) {
-            case 0: cfg.dynamicSmemBytes = 2 * sizeof(tk::LockStage<0>); cudaLaunchKernelEx(&cfg, tk::k_step_pp<0, GRAPH>, h->e, hint); break;
-            case 1: cfg.dynamicSmemBytes = 2 * sizeof(tk::LockStage<1>); cudaLaunchKernelEx(&cfg, tk::k_step_pp<1, GRAPH>, h->e, hint); break;
-            case 2: cfg.dynamicSmemBytes = 2 * sizeof(tk::LockStage<2>); cudaLaunchKernelEx(&cfg, tk::k_step_pp<2, GRAPH>, h->e, hint); break;
-            default: cfg.dynamicSmemBytes = 2 * sizeof(tk::LockStage<3>); cudaLaunchKernelEx(&cfg, tk::k_step_pp<3, GRAPH>, h->e, hint); break;
-        }
-    } else if (tma) cudaLaunchKernelEx(&cfg, tk::k_step_tma<RANDOM>, h->e, action);
-    else {
-        const int hint = h->lockstep ? h->lock_plays : -1;
-        switch (hint >= 0 ? (hint & 3) : 4) {
-            case 0: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 0, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
-            case 1: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
-            case 2: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 2, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
-            case 3: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 3, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
-            default: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, -1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
-        }
+    const int hint = h->lockstep ? h->lock_plays : -1;
+    switch (hint >= 0 ? (hint & 3) : 4) {
+        case 0: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 0, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+        case 1: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+        case 2: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 2, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+        case 3: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, 3, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
+        default: cudaLaunchKernelEx(&cfg, tk::k_step<RANDOM, -1, MASK, GRAPH, BOTS>, h->e, action, hint, bots); break;
     }
     // lock-step bookkeeping (only a hint to the kernel, which verifies it per warp): every live game has made
     // `lock_plays` plays since the last deal; one more after this launch
@@ -173,10 +148,10 @@ static void launch_step(tarok_env* h, const uint8_t* action, cudaStream_t s, con
 }
 
 // `count` back-to-back in-kernel random steps.  Only the last launch writes legal masks (nobody can observe the interior
-// ones); with the TMA-staged implementation or the eager-mask option every launch does.
+// ones); with the eager-mask option every launch does.
 static int random_chain(tarok_env* h, uint32_t count, cudaStream_t s) {
     for (uint32_t t = 0; t < count; t++) {
-        const bool lazy = t + 1 < count && h->lazy_mask && h->step_impl != 2;
+        const bool lazy = t + 1 < count && h->lazy_mask;
         if (h->capturing) {                                // kernels of a rollout graph: run parameters from device memory
             if (lazy) launch_step<true, false, true>(h, nullptr, s);
             else launch_step<true, true, true>(h, nullptr, s);
@@ -213,7 +188,6 @@ int tarok_set_option(tarok_t* h, int option, int64_t value) {
     TK_CHECK_HANDLE(h);
     drop_graphs(h);
     if (option == TAROK_OPT_GRAPH && value >= 0 && value <= 2) { h->use_graph = (int)value; return 0; }
-    if (option == TAROK_OPT_STEP_IMPL && value >= 0 && value <= 3) { h->step_impl = (int)value; return 0; }
     if (option == TAROK_OPT_PDL && (value == 0 || value == 1)) { h->pdl = (int)value; return 0; }
     if (option == TAROK_OPT_LOCKSTEP && (value == 0 || value == 1)) { h->lockstep = (int)value; return 0; }
     if (option == TAROK_OPT_MATERIALISE && (value == 0 || value == 1)) { h->materialise = (int)value; return 0; }
@@ -243,7 +217,7 @@ int tarok_create(int device, uint64_t n_games, uint64_t seed, uint32_t flags, ta
     tarok_env* h = new (std::nothrow) tarok_env();
     if (!h) return fail(nullptr, -4, "out of host memory");
     memset(&h->e, 0, sizeof(h->e));
-    h->device = device; h->sm_count = prop.multiProcessorCount; h->step_impl = 0; h->pdl = 1; h->lockstep = 1; h->lock_plays = -1; h->lazy_mask = 1; h->materialise = 1; h->chunks = 8; h->flags = flags; h->launches = 0; h->exports = 0; h->err[0] = 0;
+    h->device = device; h->pdl = 1; h->lockstep = 1; h->lock_plays = -1; h->lazy_mask = 1; h->materialise = 1; h->chunks = 8; h->flags = flags; h->launches = 0; h->exports = 0; h->err[0] = 0;
     h->st_perm = h->st_contract = h->st_declarer = h->st_king = nullptr;
     h->s_up = h->s_down = nullptr; h->ev_fork = h->ev_join = nullptr; h->staging_ready = 0;
     memset(h->ev_up, 0, sizeof(h->ev_up)); memset(h->ev_done, 0, sizeof(h->ev_done));
@@ -639,9 +613,9 @@ int tarok_rollout_stepwise(tarok_t* h, uint32_t mode, uint64_t first_global_game
     set_first_gid(h, first_global_game_id);
     // 50 launches cost more host time than a small batch takes on the GPU: the whole rollout is replayed as ONE graph
     // launch (+ a one-thread kernel that hands over this call's first_gid and draw-cache epoch).  Not while the caller is
-    // capturing `stream` itself (the launches below are then captured as they are), nor with the TMA-staged variant.
+    // capturing `stream` itself (the launches below are then captured as they are).
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (h->use_graph && (h->use_graph == 2 || h->e.n_alloc <= (3ull << 20)) && h->step_impl != 2 && mode < TK_GRAPH_MODES
+    if (h->use_graph && (h->use_graph == 2 || h->e.n_alloc <= (3ull << 20)) && mode < TK_GRAPH_MODES
         && cudaStreamIsCapturing(s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusNone) {
         if (!h->graphs[mode] && capture_rollout_graph(h, mode) != 0) {
             h->use_graph = 0;                              // e.g. another capture is open in this thread: plain launches from now on

@@ -857,26 +857,15 @@ __device__ __forceinline__ void step_pair_general(const Env& e, u32 g, ulonglong
     step_pair_any<RANDOM, MASK, BOTS>(e, g, m, a0, a1, s0, s1, s2, s3, act, bm2);
 }
 
-// Cold paths of the lock-step kernels, kept out of line so that their registers and code do not weigh on the hot path:
-// the warp whose vote failed, and the draw-cache miss at trick positions 1-3.
-#ifndef TK_SEL8_LATE
-#define TK_SEL8_LATE 1    // table stored + barrier behind the state loads (A/B, profiles/r02/step_ab_run7.txt: 8.03 vs 8.14 us at 1 M, 71.9 vs 72.5 at 8 M)
-#endif
-#ifndef TK_COLD_NOINLINE
-#define TK_COLD_NOINLINE 0   // out of line measured slower (profiles/r02/step_ab_run6.txt): 8.78 vs 7.98 us per launch at 1 M deals
-#endif
-#if TK_COLD_NOINLINE
-#define TK_COLD __noinline__
-#else
-#define TK_COLD __forceinline__
-#endif
+// Cold paths of the lock-step kernels: the warp whose vote failed, and the draw-cache miss at trick positions 1-3.
+// Inlined: out of line measured slower (profiles/r02/step_ab_run6.txt): 8.78 vs 7.98 us per launch at 1 M deals.
 template <bool RANDOM, int HAVE, bool MASK, bool BOTS = false>
-__device__ TK_COLD void step_pair_general_cold(const Env& e, u32 g, ulonglong2 m, bool a0, bool a1, u32 act,
+__device__ __forceinline__ void step_pair_general_cold(const Env& e, u32 g, ulonglong2 m, bool a0, bool a1, u32 act,
                                                     ulonglong2 hm, ulonglong2 n0, ulonglong2 n1, ulonglong2 n2, u32 bm2 = 0u) {
     step_pair_general<RANDOM, HAVE, MASK, BOTS>(e, g, m, a0, a1, act, hm, n0, n1, n2, bm2);
 }
 template <int POS>
-__device__ TK_COLD u32 pair_lanes_cold(const Env& e, u32 g, u32 trick, bool a1) {
+__device__ __forceinline__ u32 pair_lanes_cold(const Env& e, u32 g, u32 trick, bool a1) {
     Words4 r0, r1;
     pair_blocks(e, g, trick, trick, a1, r0, r1);
     const u64 gid = e.first_gid + g;
@@ -998,9 +987,6 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
     // the run parameters: launch parameters, overwritten from the device record first thing in the GRAPH kernel variants
     const u64 fgid = (RANDOM || BOTS) ? e.first_gid : 0ull;
     const u32 tag = (RANDOM ? e.rc_epoch : 0u) | ((u32)hint >> 2);
-#if !TK_SEL8_LATE
-    if (RANDOM) { select8_store(sel8, sel8_mine); __syncthreads(); }
-#endif
     pdl_wait();                                    // the previous step's writes are visible from here on
     // every load is issued before the first use: one memory round trip per step
     ulonglong2 m = ld2(e.meta + g);
@@ -1021,12 +1007,12 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
     const bool cached = in_rows && !((u32)fgid & 1u);
     uint2 rc = {0u, 0u};
     if (in_rows && POS > 0) rc = e.rcache[(UPOS > 0u ? UPOS - 1u : 0u) * (na >> 1) + (g >> 1)];
-#if TK_SEL8_LATE
-    if (RANDOM) {                                  // behind the state loads in program order: all of them are in flight together
+    // the table is stored behind the state loads in program order, so all of them are in flight together (A/B against a store
+    // before pdl_wait, profiles/r02/step_ab_run7.txt: 8.03 vs 8.14 us at 1 M, 71.9 vs 72.5 at 8 M)
+    if (RANDOM) {
         select8_store(sel8, sel8_mine);
         __syncthreads();
     }
-#endif
     step_lock_body<RANDOM, POS, MASK, BOTS>(e, g, hint, fgid, tag, cached, m, hm, n0, n1, n2, rc, act, sel8, bm2);
 }
 
@@ -1055,168 +1041,6 @@ k_step(Env e, const uint8_t* __restrict__ action, int hint, const uint8_t* __res
         const bool a0 = (((u32)m.x >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act & 0xFFu) != CARD_SKIP),
                    a1 = (((u32)m.y >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act >> 8) != CARD_SKIP);
         if (a0 || a1) step_pair_general<RANDOM, -1, MASK, BOTS>(e, g, m, a0, a1, act, z, z, z, z, bm2);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// play_step, persistent + TMA-staged variant (the one the library launches for large batches).
-// One CTA per resident slot (4 per SM) loops over 512-game tiles.  The five read-only streams of a tile
-// (meta + 4 hands = 5 x 4 KB) are fetched by ONE elected lane with 1-D bulk async copies
-// (cp.async.bulk.shared.global -> UBLKCP) that complete on an mbarrier; two stages are in flight, so the
-// copy of tile i+1 overlaps the integer work on tile i and the global-load latency leaves the critical
-// path.  Lanes read their game pair from shared memory with conflict-free 128-bit LDS.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ u32 smem_addr(const void* p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(u64* bar, u32 count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive_expect_tx(u64* bar, u32 bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* dst_smem, const void* src_gmem, u32 bytes, u64* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_addr(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_addr(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(u64* bar, u32 parity) {
-    u32 done;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done)
-                     : "r"(smem_addr(bar)), "r"(parity)
-                     : "memory");
-    } while (!done);
-}
-
-struct __align__(128) StepStage { u64 meta[TILE]; u64 hands[4][TILE]; };
-constexpr u32 STEP_STAGE_BYTES = 5u * TILE * 8u;
-
-template <bool RANDOM>
-__global__ void __launch_bounds__(CTA, 4) k_step_tma(Env e, const uint8_t* __restrict__ action) {
-    __shared__ StepStage stage[2];
-    __shared__ __align__(8) u64 full[2];
-    pdl_launch_dependents();
-    const u64 na = e.n_alloc;
-    const u32 tiles = (u32)(na / TILE);
-    if (threadIdx.x == 0) {
-        mbar_init(&full[0], 1);
-        mbar_init(&full[1], 1);
-        mbar_fence_init();
-    }
-    __syncthreads();
-    pdl_wait();
-    auto fetch = [&](u32 tile, u32 s) {               // elected lane: arm the barrier, issue the 5 bulk copies
-        const u64 g0 = (u64)tile * TILE;
-        mbar_arrive_expect_tx(&full[s], STEP_STAGE_BYTES);
-        bulk_load(stage[s].meta, e.meta + g0, TILE * 8, &full[s]);
-#pragma unroll
-        for (int k = 0; k < 4; k++) bulk_load(stage[s].hands[k], e.hands + k * na + g0, TILE * 8, &full[s]);
-    };
-    u32 tile = blockIdx.x;
-    if (threadIdx.x == 0 && tile < tiles) fetch(tile, 0);
-    const u32 l = threadIdx.x * 2;
-    for (u32 it = 0; tile < tiles; it++, tile += gridDim.x) {
-        const u32 s = it & 1u;
-        if (threadIdx.x == 0 && tile + gridDim.x < tiles) fetch(tile + gridDim.x, s ^ 1u);
-        const u32 g = tile * TILE + l;
-        u32 act = 0;
-        if (!RANDOM) act = load_actions(action, g, e.n);
-        mbar_wait(&full[s], (it >> 1) & 1u);
-        ulonglong2 m = *reinterpret_cast<const ulonglong2*>(&stage[s].meta[l]);
-        const bool a0 = (((u32)m.x >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act & 0xFFu) != CARD_SKIP),
-                   a1 = (((u32)m.y >> M_PHASE) & 3u) == PH_PLAY && (RANDOM || (act >> 8) != CARD_SKIP);
-        if (a0 || a1) {
-            const ulonglong2 s0 = *reinterpret_cast<const ulonglong2*>(&stage[s].hands[0][l]),
-                             s1 = *reinterpret_cast<const ulonglong2*>(&stage[s].hands[1][l]),
-                             s2 = *reinterpret_cast<const ulonglong2*>(&stage[s].hands[2][l]),
-                             s3 = *reinterpret_cast<const ulonglong2*>(&stage[s].hands[3][l]);
-            step_pair_any<RANDOM>(e, g, m, a0, a1, s0, s1, s2, s3, act);
-        }
-        __syncthreads();                              // stage s may be refilled from the next iteration on
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// play_step, persistent + prefetching, position-specialised (TAROK_OPT_STEP_IMPL = 3): the interior launches of a chain of
-// in-kernel random steps (lock-step hint, lazy masks, draw cache on).  After the instruction cuts of round 2 the plain kernel
-// stalls on its initial loads (long scoreboard) -- every CTA waits a full L2 round trip before it has anything to do.  Here
-// one CTA per resident slot loops over 512-game tiles; ONE elected lane fetches the next tile's streams -- meta, the mover's
-// slot (all four at the trick-closing position) and the draw-cache row -- with 1-D bulk async copies
-// (cp.async.bulk -> UBLKCP) that complete on an mbarrier while the CTA works on the current tile, which it reads from shared
-// memory with conflict-free 128-bit LDS.  Same step_lock_body as the plain kernel, same results.
-// ------------------------------------------------------------------------------------------------
-template <int POS> struct __align__(128) LockStage {
-    u64 meta[TILE];
-    u64 slot[POS == 3 ? 4 : 1][TILE];
-    uint2 rc[POS > 0 ? TILE / 2 : 2];
-};
-template <int POS> __host__ __device__ constexpr u32 lock_stage_bytes() {
-    return TILE * 8u * (POS == 3 ? 5u : 2u) + (POS > 0 ? TILE * 4u : 0u);
-}
-#ifndef TK_PP_BLOCKS_012
-#define TK_PP_BLOCKS_012 5
-#endif
-#ifndef TK_PP_BLOCKS_3
-#define TK_PP_BLOCKS_3 4
-#endif
-
-template <int POS, bool GRAPH = false>
-__global__ void __launch_bounds__(CTA, POS == 3 ? TK_PP_BLOCKS_3 : TK_PP_BLOCKS_012) k_step_pp(Env e, int hint) {
-    extern __shared__ __align__(128) uint8_t pp_smem[];
-    LockStage<POS>* stage = reinterpret_cast<LockStage<POS>*>(pp_smem);
-    __shared__ __align__(8) u64 full[2];
-    __shared__ __align__(16) uint8_t sel8[SELECT8_SMEM];
-    pdl_launch_dependents();
-    if constexpr (GRAPH) load_run_params(e);
-    select8_to_shared(sel8);
-    const u32 na = (u32)e.n_alloc;
-    const u32 tiles = na / TILE;
-    if (threadIdx.x == 0) {
-        mbar_init(&full[0], 1);
-        mbar_init(&full[1], 1);
-        mbar_fence_init();
-    }
-    __syncthreads();
-    const u64 fgid = e.first_gid;
-    const u32 tag = e.rc_epoch | ((u32)hint >> 2);
-    const bool cached = !((u32)fgid & 1u);             // the host launches this variant with the draw cache on (rows 1-3)
-    pdl_wait();                                        // the previous step's writes are visible from here on
-    auto fetch = [&](u32 tile, u32 s) {                // elected lane: arm the barrier, issue the bulk copies of one tile
-        const u32 g0 = tile * TILE;
-        mbar_arrive_expect_tx(&full[s], lock_stage_bytes<POS>());
-        bulk_load(stage[s].meta, e.meta + g0, TILE * 8, &full[s]);
-        if (POS == 3) {
-#pragma unroll
-            for (int k = 0; k < 4; k++) bulk_load(stage[s].slot[k], e.hands + (u64)k * na + g0, TILE * 8, &full[s]);
-        } else {
-            bulk_load(stage[s].slot[0], e.hands + (u64)POS * na + g0, TILE * 8, &full[s]);
-        }
-        if (POS > 0) bulk_load(stage[s].rc, e.rcache + (u64)(POS > 0 ? POS - 1 : 0) * (na >> 1) + (g0 >> 1), TILE * 4, &full[s]);
-    };
-    u32 tile = blockIdx.x;
-    if (threadIdx.x == 0 && tile < tiles) fetch(tile, 0);
-    const u32 l = threadIdx.x * 2;
-    for (u32 it = 0; tile < tiles; it++, tile += gridDim.x) {
-        const u32 s = it & 1u;
-        if (threadIdx.x == 0 && tile + gridDim.x < tiles) fetch(tile + gridDim.x, s ^ 1u);
-        const u32 g = tile * TILE + l;
-        mbar_wait(&full[s], (it >> 1) & 1u);
-        const ulonglong2 m = *reinterpret_cast<const ulonglong2*>(&stage[s].meta[l]);
-        ulonglong2 hm, n0 = {0, 0}, n1 = {0, 0}, n2 = {0, 0};
-        if (POS == 3) {
-            hm = *reinterpret_cast<const ulonglong2*>(&stage[s].slot[POS == 3 ? 3 : 0][l]);
-            n0 = *reinterpret_cast<const ulonglong2*>(&stage[s].slot[0][l]);
-            n1 = *reinterpret_cast<const ulonglong2*>(&stage[s].slot[POS == 3 ? 1 : 0][l]);
-            n2 = *reinterpret_cast<const ulonglong2*>(&stage[s].slot[POS == 3 ? 2 : 0][l]);
-        } else {
-            hm = *reinterpret_cast<const ulonglong2*>(&stage[s].slot[0][l]);
-        }
-        uint2 rc = {0u, 0u};
-        if (POS > 0) rc = stage[s].rc[threadIdx.x];
-        step_lock_body<true, POS, false>(e, g, hint, fgid, tag, cached, m, hm, n0, n1, n2, rc, 0u, sel8);
-        __syncthreads();                               // stage s may be refilled from the next iteration on
     }
 }
 

@@ -177,11 +177,6 @@ class TarokEnv:
     discard = property(lambda self: self.view(F_DISCARD))
     qmax_hist = property(lambda self: self.view(F_QMAX_HIST))    # float32 [48, n_alloc]
 
-    def set_step_impl(self, impl: int):
-        """0 auto, 1 plain play_step kernel, 2 persistent TMA-staged kernel (general path), 3 persistent prefetching lock-step
-        kernel for the interior launches of random chains (A/B measurements)."""
-        self._check(self._lib.tarok_set_option(self._h, 1, int(impl)))
-
     def set_chunks(self, chunks: int):
         """Pipeline depth (1..32, default 8) of the host-buffer entries ``rollout_host(fused=True)`` / ``rollout_records``."""
         self._check(self._lib.tarok_set_option(self._h, 5, int(chunks)))

@@ -434,9 +434,8 @@ def test_exchange_decisions_against_oracle(oracle):
 # ---- E. cards ------------------------------------------------------------------------------------------------------------
 
 ILLEGAL = ("follow suit", "must trump", "pagat", "other seat", "already played", "talon", "no card")
-STEP_CONFIGS = [  # (name, TAROK_OPT_STEP_IMPL, lock-step, PDL)
-    ("impl1", 1, True, True), ("impl1-general", 1, False, True), ("impl1-nopdl", 1, True, False),
-    ("impl2", 2, True, True), ("impl3", 3, True, True), ("impl3-nopdl", 3, True, False)]
+STEP_CONFIGS = [  # (name, lock-step, PDL)
+    ("impl1", True, True), ("impl1-general", False, True), ("impl1-nopdl", True, False)]
 N_CARDS = 300_001
 
 
@@ -643,16 +642,14 @@ def test_illegal_cards_against_oracle(oracle, mode):
     suit, a held suit card when the player must trump, the pagat in Klop/Berac while other cards are legal, another
     seat's card, a card already played, a talon card, ids 54..253 and 0xFF -- at all four trick positions, on both games
     of a lane pair and on each alone, on whole warps, next to a TAROK_CARD_SKIP at the trick-closing position, mixed with
-    skips and with tarok_steps_random chains.  Every play_step configuration: impl 1 lock-step on / off, impl 2, impl 3,
-    PDL on / off."""
+    skips and with tarok_steps_random chains.  Every play_step configuration: lock-step on / off, PDL on / off."""
     from tarok_b200.env import TarokEnv
     env = TarokEnv(N_CARDS, seed=SEED, history=True)
     try:
         for gid in (2 ** 33 + 2, 777):
             ref, rep0, start = card_reference(oracle, mode, gid)
-            for ci, (name, impl, lock, pdl) in enumerate(STEP_CONFIGS):
+            for ci, (name, lock, pdl) in enumerate(STEP_CONFIGS):
                 what = "mode %d gid %d %s" % (mode, gid, name)
-                env.set_step_impl(impl)
                 env.set_lockstep(lock)
                 env.set_pdl(pdl)
                 env.reset_stats()
@@ -670,5 +667,24 @@ def test_illegal_cards_against_oracle(oracle, mode):
                 for name_ in ("pair both", "pair even alone", "pair odd alone", "whole warp"):
                     assert sum(run.count.get((name_, p), 0) for p in range(4)) > 0, (what, name_)
                 assert run.count.get(("error beside a skip", 3), 0) > 0, what
+    finally:
+        env.close()
+
+
+def test_retired_option_id_is_refused(oracle):
+    """Option id 1, which once selected the play_step implementation, is refused like any unknown id and changes nothing:
+    a stepwise rollout that follows still plays the oracle's games."""
+    from tarok_b200.env import TarokEnv
+    n, gid = 20_001, 41
+    env = TarokEnv(n, seed=SEED, history=True)
+    try:
+        for value in (0, 1):
+            assert env._lib.tarok_set_option(env._h, 1, value) < 0
+            assert b"unknown option" in env._lib.tarok_last_error(env._h)
+        ref = oracle.rollout(SEED, gid, n, 17)
+        env.rollout(17, first_game_id=gid)
+        same(env.scores[:n].cpu().numpy(), ref["scores"], "scores")
+        played = ref["cards"] != 0xFF
+        same(np.where(played, env.hist[:, :n].cpu().numpy().T & 63, 0xFF), ref["cards"], "cards")
     finally:
         env.close()

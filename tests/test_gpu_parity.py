@@ -701,18 +701,15 @@ def test_scores_only_path_matches_oracle(oracle, mode):
     env.close()
 
 
-@pytest.mark.parametrize("impl,pdl,lock", [(1, False, False), (1, True, False), (1, False, True), (2, True, False), (2, False, False),
-                                           (3, True, True), (3, False, True)])
-def test_every_play_step_variant_matches_oracle(oracle, impl, pdl, lock):
-    """The selectable play_step implementations (plain / TMA-staged general path / persistent prefetching lock-step kernel, PDL
-    on/off, lock-step specialisation on/off) all produce the oracle's games through the stepwise rollout (graph-backed, except
-    with impl 2) and external cards (impl 3 takes the plain kernel for those).  70,001 deals are 137 tiles, less than one
-    wave of the persistent grids, so each of their CTAs handles one tile: tests/test_gpu_step_variants.py covers the loops."""
+@pytest.mark.parametrize("pdl,lock", [(False, False), (True, False), (False, True)])
+def test_every_play_step_variant_matches_oracle(oracle, pdl, lock):
+    """The play_step launch options (PDL on/off, lock-step specialisation on/off) all produce the oracle's games through the
+    graph-backed stepwise rollout and through external cards."""
     n, seed = 70001, 31
     for mode in (17, 0):
         ref = oracle.rollout(seed, 10, n, mode)
         env = _env(n, seed=seed, history=True)
-        env.set_step_impl(impl); env.set_pdl(pdl); env.set_lockstep(lock)
+        env.set_pdl(pdl); env.set_lockstep(lock)
         env.rollout(mode, first_game_id=10)
         assert (env.scores[:n].cpu().numpy() == ref["scores"]).all()
         hist = env.hist[:, :n].cpu().numpy().T

@@ -28,9 +28,6 @@ def main():
     rec.close()
     env = TarokEnv(n, seed=1)
     env.set_materialise(False)
-    if os.environ.get("TAROK_STEP_IMPL"):
-        env.set_step_impl(int(os.environ["TAROK_STEP_IMPL"]))
-        out["step_impl"] = int(os.environ["TAROK_STEP_IMPL"])
     if os.environ.get("TAROK_DRAW_CACHE"):
         env.set_draw_cache(int(os.environ["TAROK_DRAW_CACHE"]))
         out["draw_cache"] = int(os.environ["TAROK_DRAW_CACHE"])

@@ -12,7 +12,6 @@ for mode in (16, 17, 0):
     env.rollout(mode, first_game_id=11)            # odd id: no draw cache
     env.set_graph(False); env.rollout(mode, first_game_id=12); env.set_graph(True)
     env.rollout(mode, first_game_id=12, fused=True)
-env.set_step_impl(3); env.rollout(16, first_game_id=20); env.set_step_impl(2); env.rollout(16, first_game_id=20); env.set_step_impl(0)
 env.deal(0)
 perm = env.export_perm().cpu().numpy()
 c = np.full(n, 3, np.uint8); d = (np.arange(n) & 3).astype(np.uint8); k = (np.arange(n) % 4).astype(np.uint8)
