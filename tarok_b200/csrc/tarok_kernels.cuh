@@ -27,11 +27,14 @@ constexpr int TILE = 2 * CTA;          // games per CTA in the 2-games-per-lane 
 // Resident CTAs per SM the register allocation is bounded for (A/B-measured on B200, profiles/r02/occupancy_ab.md; the
 // macros exist so that a variant library can be built with other bounds: python -m tarok_b200.build --variant ...).
 #ifndef TK_STEP_BLOCKS_RANDOM
-#define TK_STEP_BLOCKS_RANDOM 5   // 48 registers (a few spilled words at the trick-closing position): 69.2 -> 66.1 us at 8 M deals, = at 1 M
+#define TK_STEP_BLOCKS_RANDOM 5   // 48 registers, trick positions 0-2 and the general path: 69.2 -> 66.1 us at 8 M deals, = at 1 M
 #endif
 #ifndef TK_STEP_BLOCKS_RANDOM_012
 #define TK_STEP_BLOCKS_RANDOM_012 TK_STEP_BLOCKS_RANDOM   // trick positions 0-2 (lighter than the trick-closing one)
 #endif
+#ifndef TK_STEP_BLOCKS_RANDOM_3
+#define TK_STEP_BLOCKS_RANDOM_3 4 // the trick-closing position: 64 registers, no spills; at 5 blocks (48 registers) it spilled
+#endif                            // 32 / 64 B: headline 0.4575 -> 0.4434 ms per rollout at 1 M deals (profiles/r03)
 #ifndef TK_STEP_BLOCKS_FORCED
 #define TK_STEP_BLOCKS_FORCED 5   // 46-48 registers: 8.63 -> 8.22 us per launch at 1 M deals (6 blocks = 40 registers spills and loses)
 #endif
@@ -162,26 +165,42 @@ __device__ __forceinline__ void slots_to_seats(u64& a, u64& b, u64& c, u64& d, u
 __device__ __forceinline__ u32 slot_of(u32 seat, u32 leader) { return (seat - leader) & 3u; }
 __device__ __forceinline__ u32 leader_of(u64 meta) { return ((u32)meta >> M_LEADER) & 3u; }
 
+// Talon order = the L-th permutation (L < 720, Lehmer code, digits 120 / 24 / 6 / 2 / 1) of the six talon ids ascending:
+// order field i = the d_i-th smallest id not taken yet.  All on 32-bit words: the permutation is decoded on the RANKS 0..5 kept
+// as 4-bit fields of one register (a pick = one field extract + one masked merge), the ids are laid out one per byte in two
+// registers, and one byte permute per output word maps ranks to ids (the rank nibbles are the permute's selectors).
+// Equal to the 64-bit restatement (six ffs, Lehmer decode on a 36-bit packed list) for every L and talon
+// (tests/test_setup_and_closer_exact.py).
 __device__ __forceinline__ u64 order_from_lehmer(u64 talon, u32 L) {
-    u64 rem = 0;                                   // the six talon ids ascending, 6 bits each
+    // Lehmer digits by constant multiplies, exact on the ranges they see (L < 720, r1 < 120, r2 < 24)
+    const u32 d0 = (L * 1093u) >> 17, r1 = L - 120u * d0;
+    const u32 d1 = (r1 * 2731u) >> 16, r2 = r1 - 24u * d1;
+    const u32 d2 = (r2 * 43u) >> 8, r3 = r2 - 6u * d2;
+    const u32 d3 = r3 >> 1, d4 = r3 & 1u;
+    u32 rank = 0x543210u, perm = 0;                // ranks not taken yet, 4 bits each, ascending
+    auto pick = [&](u32 d, int i) {
+        const u32 sh = 4u * d;
+        perm |= ((rank >> sh) & 15u) << (4 * i);
+        const u32 high = 0xFFFFFFFFu << sh;        // fields d.. move down by one, fields below d stay
+        rank = (rank & ~high) | ((rank >> 4) & high);
+    };
+    pick(d0, 0); pick(d1, 1); pick(d2, 2); pick(d3, 3); pick(d4, 4);
+    perm |= rank << 20;                            // the one left
+    // the six ids ascending, one per byte: bytes 0-3 in a, 4-5 in b (lowest set bit, then clear it, on the 32-bit halves)
+    u32 lo = (u32)talon, hi = (u32)(talon >> 32), a = 0, b = 0;
 #pragma unroll
     for (int i = 0; i < 6; i++) {
-        u32 c = (u32)__ffsll((long long)talon) - 1u;
-        talon &= talon - 1;
-        rem |= (u64)c << (6 * i);
+        const bool inlo = lo != 0u;
+        const u32 w = inlo ? lo : hi;
+        const u32 c = (u32)__ffs(w) - 1u + (inlo ? 0u : 32u);
+        if (i < 4) a |= c << (8 * i); else b |= c << (8 * (i - 4));
+        if (inlo) lo &= lo - 1u; else hi &= hi - 1u;
     }
-    u64 order = 0;
-    const u32 fact[6] = {120, 24, 6, 2, 1, 1};
-#pragma unroll
-    for (int i = 0; i < 6; i++) {
-        u32 d = L / fact[i];
-        L -= d * fact[i];
-        u32 sh = 6 * d;
-        order |= ((rem >> sh) & 63ull) << (6 * i);
-        u64 low = rem & ((1ull << sh) - 1ull);
-        rem = low | ((rem >> (sh + 6)) << sh);
-    }
-    return order;
+    const u32 x = __byte_perm(a, b, perm & 0xFFFFu), y = __byte_perm(a, b, perm >> 16);   // ids in order, one per byte
+    // bytes -> 6-bit fields
+    const u32 olo = (x & 0x3Fu) | ((x >> 2) & 0xFC0u) | ((x >> 4) & 0x3F000u) | ((x >> 6) & 0xFC0000u);
+    const u32 ohi = (y & 0x3Fu) | ((y >> 2) & 0xFC0u);
+    return (u64)olo | ((u64)ohi << 24);
 }
 
 // The 53 bounded draws of a deal (n = 54 - c for card c; card 53 has no choice left) are BATCHED: several exact draws
@@ -577,9 +596,12 @@ __device__ __forceinline__ u32 card_points(u64 s) {
                  + 4 * __popcll(s & (KINGS | TRULA)));
 }
 
+// sel8: the byte-select table in shared memory (select8_to_shared) for the discard picks, or nullptr in kernels that have none
+// (the binary descent then runs to the end); both give the same card.
 template <bool SYNTH>
 __device__ __forceinline__ bool exchange_game(const Rng& rng, u64 gid, u32 random_group, const Words4& sb, u64& meta, u64& hand,
-                                              u64& pile, u64& talon, u64 order, u32 group, u64 discard, u64& discard_out) {
+                                              u64& pile, u64& talon, u64 order, u32 group, u64 discard, u64& discard_out,
+                                              const uint8_t* __restrict__ sel8 = nullptr) {
     u32 contract = mget(meta, M_CONTRACT, 4);
     u32 k = talon_k(contract);
     u32 ngroups = 6u / k;
@@ -603,7 +625,7 @@ __device__ __forceinline__ bool exchange_game(const Rng& rng, u64 gid, u32 rando
         discard = 0;
 #pragma unroll
         for (u32 j = 0; j < 3; j++) if (j < k) {    // uniform k-subset = random.sample (Igralec.py:166)
-            u64 bit = 1ull << nth_set_bit(avail, rd[j]);
+            u64 bit = 1ull << (sel8 ? nth_set_bit_lut(avail, rd[j], sel8) : nth_set_bit(avail, rd[j]));
             avail ^= bit; discard |= bit;
         }
     }
@@ -679,7 +701,10 @@ __global__ void __launch_bounds__(CTA) k_exchange(Env e, u32 random_group, const
 // ------------------------------------------------------------------------------------------------
 template <bool GRAPH = false>
 __global__ void __launch_bounds__(CTA, TK_SETUP_BLOCKS) k_setup_synth(Env e, u32 mode) {
+    __shared__ __align__(16) uint8_t sel8[SELECT8_SMEM];  // byte-select table of the discard picks (tarok_rules.cuh)
+    select8_to_shared(sel8);
     if constexpr (GRAPH) load_run_params(e);
+    __syncthreads();                                      // every lane reaches this: the grid covers n_alloc exactly
     const u64 g = (u64)blockIdx.x * CTA + threadIdx.x;
     const u64 na = e.n_alloc;
     if (g >= na) return;
@@ -699,7 +724,8 @@ __global__ void __launch_bounds__(CTA, TK_SETUP_BLOCKS) k_setup_synth(Env e, u32
         if (mget(meta, M_PHASE, 2) == PH_EXCHANGE) {
             u64 pile = 0;
             hand = sel4(d.h0, d.h1, d.h2, d.h3, decl);
-            exchanged = exchange_game<true>(e.rng, gid, mode == 17u, sb, meta, hand, pile, d.talon, d.order, 0u, 0ull, dout);
+            exchanged = exchange_game<true>(e.rng, gid, mode == 17u, sb, meta, hand, pile, d.talon, d.order, 0u, 0ull, dout,
+                                        sel8);
             if (!exchanged) meta = mset(meta, M_PHASE, 2, PH_DONE) | (1ull << M_ERR);
         }
         if ((meta >> M_ERR) & 1ull) atomicAdd((unsigned long long*)&e.stats[S_ERR_EVENTS], 1ull);
@@ -1024,7 +1050,8 @@ __device__ __forceinline__ void step_lock(const Env& e, const uint8_t* __restric
 // 48 bytes a step moves at trick positions 0-2 -- and only the chain's last launch produces the masks.
 // BOTS (with RANDOM = false): the third action source, tarok_step_bots -- `bots` = the per-game seat masks.
 template <bool RANDOM, int POS, bool MASK = true, bool GRAPH = false, bool BOTS = false>
-__global__ void __launch_bounds__(CTA, RANDOM ? ((POS >= 0 && POS < 3) ? TK_STEP_BLOCKS_RANDOM_012 : TK_STEP_BLOCKS_RANDOM)
+__global__ void __launch_bounds__(CTA, RANDOM ? ((POS >= 0 && POS < 3) ? TK_STEP_BLOCKS_RANDOM_012
+                                                   : POS == 3 ? TK_STEP_BLOCKS_RANDOM_3 : TK_STEP_BLOCKS_RANDOM)
                                            : BOTS ? TK_STEP_BLOCKS_BOTS : TK_STEP_BLOCKS_FORCED)
 k_step(Env e, const uint8_t* __restrict__ action, int hint, const uint8_t* __restrict__ bots) {
     pdl_launch_dependents();
@@ -1292,7 +1319,7 @@ __global__ void __launch_bounds__(CTA) k_rollout_fused(Env e, u32 mode, const ui
         if (mget(meta, M_PHASE, 2) == PH_EXCHANGE) {
             u32 decl = mget(meta, M_DECL, 2);
             u64 hand = sel4(h0, h1, h2, h3, decl), pile = 0;
-            bool ok2 = exchange_game<true>(e.rng, gid, mode == 17u, sb, meta, hand, pile, talon, order, 0u, 0ull, dout);
+            bool ok2 = exchange_game<true>(e.rng, gid, mode == 17u, sb, meta, hand, pile, talon, order, 0u, 0ull, dout, sel8);
             if (!ok2) meta = mset(meta, M_PHASE, 2, PH_DONE) | (1ull << M_ERR);
             else {
                 h0 = decl == 0 ? hand : h0; h1 = decl == 1 ? hand : h1; h2 = decl == 2 ? hand : h2; h3 = decl == 3 ? hand : h3;
